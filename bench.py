@@ -2,6 +2,7 @@
 """Benchmark of the baseband hot path on B200 (driver contract).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+                    [--dump-outputs DIR]
 
 Workload = BASELINE.json configs[1]: synthetic VDIF, 2-bit real, 16 threads,
 8032-byte frames; one step = the hot path over `--passes` (default 32)
@@ -278,12 +279,14 @@ def run_b200(args):
             dec_events.append((e0, e1))
         kernels.encode_bitfield(out, back, uo, nset, NTHREAD, PAYLOAD, 2, 1,
                                 kernels.QUANT_OFFSET_BINARY)
+        return uo
 
     def step(record=False):
         # record one decode launch in four: 640 event pairs would do no harm,
         # but the sustained figure needs no more
         for k in range(passes):
-            one_pass(record and (k % 4 == 0))
+            uo = one_pass(record and (k % 4 == 0))
+        return uo
 
     def barrier():
         if world > 1:
@@ -309,13 +312,16 @@ def run_b200(args):
     t1 = torch.cuda.Event(enable_timing=True)
     t0.record()
     for _ in range(args.steps):
-        step(record=True)
+        uo = step(record=True)
     t1.record()
     barrier()
     elapsed_ms = t0.elapsed_time(t1)
     launches = kernels.launch_count - launches0
     clocks = sampler.stop() if rank == 0 else None
     assert int(counter.item()) == 0
+    # before measure_ceilings, which overwrites `out`
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, out, back, uo, nset)
     if world > 1:
         t = torch.tensor([elapsed_ms], device=dev)
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
@@ -389,6 +395,29 @@ def run_b200(args):
 
 
 DECODE_KERNEL = 'k_decode_bitfield<2,LEVELS,ROWGROUP4>'
+DUMP_SETS = 16          # frame sets sampled by --dump-outputs (~42 MB in all)
+
+
+def dump_outputs(folder, out, back, uo, nset):
+    """What the last timed pass hands its caller, as float32 / float64 .npy
+    files, so that two builds can be compared output for output: the unit
+    offsets of the header scan in full, and the decoded samples and
+    re-encoded frames of DUMP_SETS frame sets drawn with a fixed seed (a
+    chunk decodes to 16 GiB).  The inputs come from fixed seeds too."""
+    import torch
+    os.makedirs(folder, exist_ok=True)
+    sets = np.sort(np.random.default_rng(0).choice(
+        nset, min(DUMP_SETS, nset), replace=False))
+    rows = torch.from_numpy(sets).to(out.device)
+    arrays = {
+        'frame_sets': sets.astype(np.float64),
+        'unit_offsets': uo.cpu().numpy().astype(np.float64),
+        'decoded': out.view(nset, SPF, NTHREAD)[rows].cpu().numpy(),
+        'encoded_frames': back.view(nset, SET_BYTES)[rows].cpu().numpy()
+        .astype(np.float32),
+    }
+    for name, array in arrays.items():
+        np.save(os.path.join(folder, name + '.npy'), array)
 
 
 def _leg(fn, *a):
@@ -992,7 +1021,14 @@ def main():
                     help='packed MiB per GPU and step of the state-count '
                          'consumer leg (0 = skip)')
     ap.add_argument('--no-cpu-baseline', action='store_true')
+    ap.add_argument('--dump-outputs', metavar='DIR',
+                    help='after the timed steps, write what the last one '
+                         'computed to DIR/<name>.npy (rank 0, B200 arm)')
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
+    if args.dump_outputs and args.impl != 'b200':
+        ap.error('--dump-outputs applies to the b200 implementation')
     if args.impl == 'reference':
         run_reference(args)
     else:

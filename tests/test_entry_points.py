@@ -1,38 +1,26 @@
-"""The drop-in boundary as the reference's plug-in loader sees it.
+"""The drop-in boundary as the reference's plug-in loaders see it.
 
 ``baseband.io`` (baseband/io/__init__.py:35-94) resolves a format name
 through an ``importlib.metadata.EntryPoint`` of group 'baseband.io' that
 points to a module, loads it, and calls ``module.open(name, mode=...,
-**kwargs)`` (:236-237) and ``module.info(name, **kwargs)`` (:163-164).  Here
-the reference's own loader module is loaded by path (it imports only the
-standard library at module level), given fake entry points for the
-``baseband_b200`` format modules exactly as
-baseband/tests/test_entry_points.py:50-92 does, and files are opened and read
-through it.  /root/reference exists only in the build container, so that
-part is skipped elsewhere; the GPU variant exercises the same protocol
-(EntryPoint.load() -> module.open / module.info) without the loader file.
+**kwargs)`` (:236-237) and ``module.info(name, **kwargs)`` (:163-164);
+``baseband.tasks`` (baseband/tasks/__init__.py:25-62) does the same for
+functions of group 'baseband.tasks'.  Here the entry points pyproject.toml
+declares are installed as a distribution's metadata in a temporary
+directory, found through ``importlib.metadata.entry_points(group=...)`` as
+those loaders find them, loaded, and files are opened and read through them.
 """
-import importlib.util
 import os
-import sys
-from importlib.metadata import EntryPoint
+import tomllib
+from importlib.metadata import EntryPoint, entry_points
 
 import numpy as np
 import pytest
 
-from conftest import GOLDEN, sample_path
+from conftest import GOLDEN, ROOT, sample_path
 
-REF_IO = '/root/reference/baseband/io/__init__.py'
 OUT = np.load(os.path.join(GOLDEN, 'sample_outputs.npz'))
 FORMATS = ('vdif', 'mark5b', 'mark4', 'dada', 'guppi', 'gsb')
-
-
-def _load_reference_io():
-    spec = importlib.util.spec_from_file_location('ref_baseband_io', REF_IO)
-    module = importlib.util.module_from_spec(spec)
-    sys.modules['ref_baseband_io'] = module       # its __self__ lookup
-    spec.loader.exec_module(module)
-    return module
 
 
 def _read_all_through(open_, tag=''):
@@ -54,43 +42,65 @@ def _read_all_through(open_, tag=''):
         assert fb.read_frame().shape == (20000, 1)
 
 
-@pytest.mark.skipif(not os.path.exists(REF_IO),
-                    reason='reference tree only exists in the build container')
-def test_reference_loader_resolves_b200_formats(monkeypatch):
+def _declared_entry_points(tmp_path, monkeypatch, group):
+    """The entry points of ``group`` as an installed baseband_b200 exposes
+    them: pyproject.toml's declarations written to a dist-info directory on
+    sys.path, then looked up through importlib.metadata."""
+    with open(os.path.join(ROOT, 'pyproject.toml'), 'rb') as fh:
+        project = tomllib.load(fh)['project']
+    info = tmp_path / 'baseband_b200-{}.dist-info'.format(project['version'])
+    info.mkdir()
+    (info / 'METADATA').write_text('Metadata-Version: 2.1\nName: {}\n'
+                                   'Version: {}\n'.format(project['name'],
+                                                          project['version']))
+    (info / 'entry_points.txt').write_text(''.join(
+        '[{}]\n'.format(name) + ''.join('{} = {}\n'.format(k, v)
+                                        for k, v in eps.items())
+        for name, eps in project['entry-points'].items()))
+    monkeypatch.syspath_prepend(str(tmp_path))
+    return {ep.name: ep for ep in entry_points(group=group)
+            if ep.dist is not None and ep.dist.name == project['name']}
+
+
+def test_io_entry_points_cpu(tmp_path, monkeypatch):
     import cpu_backend
     cpu_backend.install(monkeypatch)
     import baseband_b200 as bb
-    bio = _load_reference_io()
-    try:
-        dir(bio)                                  # creates FORMATS, _entries
-        for fmt in FORMATS:
-            name = fmt + '_b200'
-            bio._entries[name] = EntryPoint(name, 'baseband_b200.' + fmt, '')
-            bio.FORMATS.append(name)
-        assert 'vdif_b200' in dir(bio) and 'vdif_b200' in bio.FORMATS
-        assert bio.vdif_b200 is bb.vdif          # EntryPoint.load() -> module
-        assert 'vdif_b200' in bio.__dict__
-        for fmt in FORMATS:
-            module = getattr(bio, fmt + '_b200')
-            assert module is getattr(bb, fmt)
-            assert callable(module.open)
-        # bio.open(name, mode, format=...) -> module.open(name, mode=mode, **kw)
-        _read_all_through(
-            lambda name, mode, fmt, **kw: bio.open(name, mode, format=fmt,
-                                                   **kw), tag='_b200')
-        # what bio.file_info(name, format) does for one format (:163-164; the
-        # function itself imports baseband.base.file_info, i.e. astropy)
-        info = bio.vdif_b200.info(sample_path('sample.vdif'))
-        assert info and info.format == 'vdif'
-        assert not bio.mark5b_b200.info(sample_path('sample.vdif'))
-        # a bad entry behaves as in the reference's own test (:75-92)
-        bio._entries['bad'] = EntryPoint('bad', 'really_bad', '')
-        bio.FORMATS.append('bad')
-        with pytest.raises(AttributeError, match='not loadable'):
-            bio.bad
-        assert 'bad' not in bio.FORMATS
-    finally:
-        sys.modules.pop('ref_baseband_io', None)
+    eps = _declared_entry_points(tmp_path, monkeypatch, 'baseband.io')
+    assert sorted(eps) == sorted(fmt + '_b200' for fmt in FORMATS)
+    modules = {name: ep.load() for name, ep in eps.items()}
+    for fmt in FORMATS:
+        assert modules[fmt + '_b200'] is getattr(bb, fmt)
+    _read_all_through(lambda name, mode, fmt, **kw:
+                      modules[fmt].open(name, mode=mode, **kw), tag='_b200')
+    info = modules['vdif_b200'].info(sample_path('sample.vdif'))
+    assert info and info.format == 'vdif'
+    assert not modules['mark5b_b200'].info(sample_path('sample.vdif'))
+
+
+def test_tasks_entry_points_cpu(tmp_path, monkeypatch):
+    import cpu_backend
+    cpu_backend.install(monkeypatch)
+    import baseband_b200 as bb
+    from baseband_b200 import tasks as b200_tasks
+    eps = _declared_entry_points(tmp_path, monkeypatch, 'baseband.tasks')
+    assert sorted(eps) == ['integrated_power', 'moments', 'state_counts']
+    tasks = {name: ep.load() for name, ep in eps.items()}
+    for name, fn in tasks.items():
+        assert fn is getattr(b200_tasks, name)
+    with bb.vdif.open(sample_path('sample.vdif'), 'rs') as fh:
+        counts = tasks['state_counts'](fh, 20000)
+        data = OUT['sample_vdif_data'][:, :, 0]
+        lv = b200_tasks.state_levels(fh)
+        want = np.stack([np.stack([(data[b * 20000:(b + 1) * 20000] == v
+                                    ).sum(0) for v in lv], -1)
+                         for b in range(2)])
+        assert np.array_equal(counts, want)
+        fh.seek(0)
+        power = tasks['integrated_power'](fh, 20000)
+        ref = np.stack([(data[b * 20000:(b + 1) * 20000].astype(np.float64)
+                         ** 2).mean(0) for b in range(2)])
+        assert np.allclose(power, ref, rtol=1e-10, atol=0)
 
 
 def test_entry_point_protocol_cpu(monkeypatch):
@@ -119,48 +129,3 @@ def _entry_point_protocol():
     assert 'baseband.io' in text
     for fmt in FORMATS:
         assert 'baseband_b200.' + fmt in text
-
-
-REF_TASKS = '/root/reference/baseband/tasks/__init__.py'
-
-
-@pytest.mark.skipif(not os.path.exists(REF_TASKS),
-                    reason='reference tree only exists in the build container')
-def test_reference_tasks_loader_finds_b200_consumers(tmp_path, monkeypatch):
-    """The analysis plug-in point (baseband/tasks/__init__.py:25-62): the
-    reference's own loader, given the entry points pyproject.toml declares
-    (written to a dist-info as baseband/tests/test_entry_points.py:103-110
-    does), exposes the GPU consumers, and they run."""
-    import cpu_backend
-    cpu_backend.install(monkeypatch)
-    import baseband_b200 as bb
-    from baseband_b200 import tasks as b200_tasks
-    info = tmp_path / 'b200_tasks-0.1.dist-info'
-    info.mkdir()
-    (info / 'entry_points.txt').write_text(
-        '[baseband.tasks]\n'
-        'state_counts = baseband_b200.tasks:state_counts\n'
-        'integrated_power = baseband_b200.tasks:integrated_power\n'
-        '_ = baseband_b200.tasks:__all__\n')
-    monkeypatch.syspath_prepend(str(tmp_path))
-    spec = importlib.util.spec_from_file_location('ref_baseband_tasks',
-                                                  REF_TASKS)
-    tasks = importlib.util.module_from_spec(spec)
-    spec.loader.exec_module(tasks)
-    assert tasks._bad_entries == []
-    assert tasks.state_counts is b200_tasks.state_counts
-    assert tasks.integrated_power is b200_tasks.integrated_power
-    assert tasks.state_levels is b200_tasks.state_levels     # via __all__
-    with bb.vdif.open(sample_path('sample.vdif'), 'rs') as fh:
-        counts = tasks.state_counts(fh, 20000)
-        data = OUT['sample_vdif_data'][:, :, 0]
-        lv = tasks.state_levels(fh)
-        want = np.stack([np.stack([(data[b * 20000:(b + 1) * 20000] == v
-                                    ).sum(0) for v in lv], -1)
-                         for b in range(2)])
-        assert np.array_equal(counts, want)
-        fh.seek(0)
-        power = tasks.integrated_power(fh, 20000)
-        ref = np.stack([(data[b * 20000:(b + 1) * 20000].astype(np.float64)
-                         ** 2).mean(0) for b in range(2)])
-        assert np.allclose(power, ref, rtol=1e-10, atol=0)
