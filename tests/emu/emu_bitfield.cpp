@@ -202,9 +202,40 @@ extern "C" {
 
 const char *bb_last_error(void) { return g_err.c_str(); }
 
-// Which decomposition the planner picks (for test coverage assertions).
-int emu_decode_mode(int32_t nelem, int32_t nthread, int aligned_rows) {
-    return pick_mode(nelem, nthread, aligned_rows != 0, true);
+// What the real planner makes of a call, without running it (no pointer is
+// dereferenced by the planner, so the data pointers are null).  info[0] =
+// mode of the first launch, info[1] = its `sel`, info[2] = the number of
+// launches, info[3] = the frame sets of the first launch, info[4] = the
+// items of the last launch.  Returns 0, or BB_ERR_ARGUMENT when the planner
+// refuses the call.
+int emu_plan_decode(int64_t nset, int32_t nthread, int64_t payload_nbytes,
+                    int32_t bps, int32_t nelem, int32_t complex_data,
+                    int64_t sample_start, int64_t nsample, int64_t *info) {
+    std::vector<DecLaunch> launches;
+    if (!plan_decode(nullptr, nullptr, nset, nthread, payload_nbytes, bps,
+                     nelem, complex_data, 0.f, sample_start, nsample, nullptr,
+                     launches, g_err))
+        return BB_ERR_ARGUMENT;
+    info[0] = launches.empty() ? -1 : launches[0].mode;
+    info[1] = launches.empty() ? 0 : launches[0].sel;
+    info[2] = (int64_t)launches.size();
+    info[3] = launches.empty() ? 0 : launches[0].g.nset;
+    info[4] = launches.empty() ? 0 : launches.back().g.nitems;
+    return 0;
+}
+
+int emu_plan_encode(int64_t nset, int32_t nthread, int64_t payload_nbytes,
+                    int32_t bps, int32_t nelem, int64_t *info) {
+    std::vector<EncLaunch> launches;
+    if (!plan_encode(nullptr, nullptr, nullptr, nset, nthread, payload_nbytes,
+                     bps, nelem, launches, g_err))
+        return BB_ERR_ARGUMENT;
+    info[0] = launches.empty() ? -1 : launches[0].mode;
+    info[1] = 0;
+    info[2] = (int64_t)launches.size();
+    info[3] = launches.empty() ? 0 : launches[0].g.nset;
+    info[4] = launches.empty() ? 0 : launches.back().g.nitems;
+    return 0;
 }
 
 int bb_decode_bitfield(const void *src, const int64_t *unit_offset,

@@ -355,6 +355,114 @@ def test_fuzz_bitfield(emu):
         test_encode_bitfield(emu, case)
 
 
+def test_matrix_bitfield(emu):
+    """The multi-CTA coverage matrix through the kernel bodies vs the
+    oracle (the GPU runs the same cases in test_gpu_bitfield)."""
+    from bitfield_cases import matrix_cases
+    dec, enc = matrix_cases()
+    for case in dec:
+        test_decode_bitfield(emu, case)
+    for case in enc:
+        test_encode_bitfield(emu, case)
+
+
+def _planner_cells(emu):
+    """Every (decode, encode) cell the default planner produces over a grid
+    of geometries: bps, thread counts, elements per sample, two payload
+    sizes (one with a number of words that is not a multiple of four), full
+    reads, reads inside frames and unaligned reads."""
+    from bitfield_cases import (DECODERS, QUANTISERS, plan_decode,
+                                plan_encode)
+    dec, enc = set(), set()
+    for bps in (1, 2, 4, 8):
+        for nthread in list(range(1, 10)) + [12, 16, 32, 64]:
+            for nelem in (1, 2, 3, 4, 6, 8, 16, 32, 2048):
+                bits = bps * nelem
+                unit = bits * 32 // np.gcd(bits, 32) // 8    # bytes
+                for payload in (unit * 8, unit * 9):
+                    spf = payload * 8 // bits
+                    total = 3 * spf
+                    for start, count in ((0, total), (spf // 2, 2 * spf),
+                                         (4, total - 8), (1, total - 2)):
+                        mode, sel = plan_decode(
+                            emu, 3, nthread, payload, bps, nelem, start,
+                            count)[:2]
+                        dec.update((mode, sel, bps, d) for d in DECODERS[bps])
+                    mode = plan_encode(emu, 3, nthread, payload, bps,
+                                       nelem)[0]
+                    enc.update((mode, bps, q, t) for q in QUANTISERS[bps]
+                               for t in ('f4', 'f8'))
+    return dec, enc
+
+
+def test_matrix_covers_every_planner_cell(emu):
+    """matrix_cases() reaches exactly the kernel instances the planner can
+    choose, and every case lands in the cell it is labelled with: a new mode
+    or instance without a case, or a case that no longer plans where it
+    says, fails here."""
+    from bitfield_cases import matrix_cases, decode_cell, encode_cell
+    want_dec, want_enc = _planner_cells(emu)
+    dec, enc = matrix_cases()
+    for c in dec:
+        assert decode_cell(emu, c) == c['cell'], c['id']
+    for c in enc:
+        assert encode_cell(emu, c) == c['cell'], c['id']
+    assert {c['cell'] for c in dec} == want_dec
+    assert {c['cell'] for c in enc} == want_enc
+    assert len({c['id'] for c in dec + enc}) == len(dec) + len(enc)
+    # the variants of every decode cell: a full read; partial reads with
+    # real fill, and complex fill where nelem is even, whose fill values
+    # cover an ordinary number, -0.0 and NaN; for the modes that need
+    # aligned reads, an unaligned read of the same bps and decoder that
+    # falls back to another mode
+    fills = {np.float32(f).view('u4').item() for f in (2.5, -0.0, np.nan)}
+    for cell in want_dec:
+        mine = [c for c in dec if c['cell'] == cell
+                and 'fallback_of' not in c]
+        assert any(c['start'] == 0 and c['count'] is None for c in mine)
+        part = [c for c in mine if c['count'] is not None]
+        assert any(not c['complex'] for c in part), cell
+        if all(c['nelem'] % 2 == 0 for c in part):
+            assert any(c['complex'] for c in part), cell
+        assert {np.float32(c['fill']).view('u4').item()
+                for c in part} >= fills, cell
+        if cell[0] in ('WORDRUN', 'RUNS'):
+            assert any(c.get('fallback_of') == cell[0]
+                       and c['cell'][2:] == cell[2:] for c in dec), cell
+    # and for every cell a case whose last CTA is partly filled down to its
+    # last unrolled round (items counted by the real planner)
+    from bitfield_cases import last_launch_items, last_round_partial
+    tail = set()
+    for c in dec + enc:
+        if last_round_partial(last_launch_items(emu, c), c['cell'][0],
+                              c['bps'], 'quant' in c):
+            tail.add(c['cell'])
+    assert tail == want_dec | want_enc
+
+
+def test_matrix_case_sizes():
+    """Each matrix case spans many CTAs and ends in a partly filled one: at
+    least 4 MiB of float32 output (decode) or of input (encode), not a
+    multiple of 64 KiB; the partial reads start and end inside frames."""
+    from bitfield_cases import matrix_cases
+    dec, enc = matrix_cases()
+    for c in dec:
+        spf = c['payload_nbytes'] * 8 // (c['bps'] * c['nelem'])
+        count = c['count'] if c['count'] is not None else \
+            c['nset'] * spf - c['start']
+        nbytes = count * c['nthread'] * c['nelem'] * 4
+        assert nbytes >= 4 << 20 and nbytes % (64 << 10), c['id']
+        if c['start']:
+            assert c['start'] % spf and (c['start'] + count) % spf, c['id']
+            assert c['invalid'], c['id']
+    for c in enc:
+        spf = c['payload_nbytes'] * 8 // (c['bps'] * c['nelem'])
+        nbytes = c['nset'] * spf * c['nthread'] * c['nelem'] * \
+            np.dtype(c['dtype']).itemsize
+        assert nbytes >= 4 << 20 and nbytes % (64 << 10), c['id']
+        assert c['invalid'], c['id']
+
+
 def test_fuzz_int8_transposed(emu):
     for case in int8_cases.fuzz_cases(60, seed=77):
         test_int8_transposed(emu, case)

@@ -8,7 +8,8 @@ import torch
 from baseband_b200 import kernels, levels
 from oracle import codec
 from bitfield_cases import (DECODE_CASES, ENCODE_CASES, make_decode_case,
-                            oracle_decode, make_encode_case, oracle_encode)
+                            oracle_decode, make_encode_case, oracle_encode,
+                            matrix_cases)
 
 pytestmark = pytest.mark.gpu
 DEV = 'cuda:0'
@@ -18,20 +19,35 @@ def _t(a):
     return torch.from_numpy(np.ascontiguousarray(a)).to(DEV)
 
 
-@pytest.mark.parametrize('case', DECODE_CASES, ids=lambda c: c['id'])
+MATRIX_DECODE, MATRIX_ENCODE = matrix_cases()
+# floats of sentinel on either side of a decode's output (64 KiB each; a
+# multiple of four floats keeps the output 16-byte aligned)
+GUARD = 16384
+SENTINEL = 0x7FBADBAD               # a NaN payload no decode produces
+
+
+@pytest.mark.parametrize('case', DECODE_CASES + MATRIX_DECODE,
+                         ids=lambda c: c['id'])
 def test_decode_bitfield(case):
+    """Decode into a view of a larger buffer: the values must equal the
+    oracle bit for bit and the sentinels around the view stay untouched."""
     c = make_decode_case(case)
     want = oracle_decode(c)
+    buf = torch.full((want.size + 2 * GUARD,), SENTINEL, dtype=torch.int32,
+                     device=DEV).view(torch.float32)
+    view = buf[GUARD:GUARD + want.size].view(want.shape)
     out = kernels.decode_bitfield(
         _t(c['raw']), _t(c['unit_offset']), c['nset'], c['nthread'],
         c['payload_nbytes'], c['bps'], c['nelem'], c['complex'], c['codec'],
-        c['levels'], c['fill'], c['sample_start'], c['nsample'])
-    got = out.cpu().numpy()
-    assert got.shape == want.shape
-    assert np.array_equal(got.view('u4'), want.view('u4'))
+        c['levels'], c['fill'], c['sample_start'], c['nsample'], out=view)
+    assert out.data_ptr() == view.data_ptr()
+    got = buf.cpu().numpy().view('u4')
+    assert np.array_equal(got[GUARD:GUARD + want.size], want.ravel().view('u4'))
+    assert (got[:GUARD] == SENTINEL).all() and (got[-GUARD:] == SENTINEL).all()
 
 
-@pytest.mark.parametrize('case', ENCODE_CASES, ids=lambda c: c['id'])
+@pytest.mark.parametrize('case', ENCODE_CASES + MATRIX_ENCODE,
+                         ids=lambda c: c['id'])
 def test_encode_bitfield(case):
     c = make_encode_case(case)
     want = oracle_encode(c)

@@ -410,3 +410,109 @@ def test_state_counts_4bit_counter_limits(payload, nset):
                           np.bincount(host & 15, minlength=16))
     assert np.array_equal(got2.cpu().numpy()[0, 0, 1],
                           np.bincount(host >> 4, minlength=16))
+
+
+# ---------------------------------------------------------------------------
+# Partial reads across a launch split.  The planner cuts a call whose item
+# count would pass 32 bits (the warp-cooperative modes: 2^26 word positions)
+# into several launches; every later one carries a shifted row base and unit
+# offset pointer.  These cases read from inside a frame of the first launch
+# to inside a frame of the last, with invalid units on both sides of the
+# split, and check the sets next to the split and the partial end frames
+# bit for bit against the oracle, the fill count of the whole range exactly,
+# and the decode -> encode round trip of the whole range.
+@pytest.fixture(scope='module')
+def emu():
+    import emu_build
+    return emu_build.load()
+
+
+def _frames(nunit, payload, seed):
+    """nunit frames of a 32-byte header and `payload` random bytes."""
+    g = torch.Generator(device=DEV).manual_seed(seed)
+    raw = torch.randint(0, 256, (nunit * (payload + 32),), dtype=torch.uint8,
+                        device=DEV, generator=g)
+    uo = torch.arange(nunit, dtype=torch.int64, device=DEV) * (payload + 32) \
+        + 32
+    return raw, uo
+
+
+@pytest.mark.parametrize('mode,nthread,align', [('WORDRUN', 1, 4),
+                                                ('WORDROW4', 4, 1)])
+def test_partial_read_across_launch_split(emu, mode, nthread, align):
+    from bitfield_cases import plan_decode
+    bps, nelem, payload, fill = 8, 1, 8000, -999.0
+    spf, frame = payload, payload + 32
+    nset = 0x3ffffff // (payload // 4) + 7      # just past one launch
+    start = (spf // 3) // align * align + align
+    end = ((nset - 1) * spf + 2 * spf // 3) // align * align
+    got_mode, _, nlaunch, split, _ = plan_decode(
+        emu, nset, nthread, payload, bps, nelem, start, end - start)
+    assert (got_mode, nlaunch) == (mode, 2) and 0 < split < nset - 1
+    raw, uo = _frames(nset * nthread, payload, 77 + nthread)
+    invalid = sorted({split * nthread - 1, split * nthread,
+                      (split + 1) * nthread - 1})
+    uo_inv = uo.clone()
+    uo_inv[invalid] = -1
+    lv = levels.offset_binary(8)
+    out = kernels.decode_bitfield(raw, uo_inv, nset, nthread, payload, bps,
+                                  nelem, False, kernels.CODEC_LEVELS, lv,
+                                  fill, start, end - start)
+    frames = raw.view(nset * nthread, frame)
+
+    def want_set(s):
+        rows = np.empty((spf, nthread), np.float32)
+        for t in range(nthread):
+            u = s * nthread + t
+            rows[:, t] = fill if u in invalid else codec.vdif_decode(
+                frames[u, 32:].cpu().numpy().view('<u4'), bps)
+        return rows
+
+    for s in (0, split - 1, split, nset - 1):
+        lo, hi = max(s * spf, start), min((s + 1) * spf, end)
+        want = want_set(s)[lo - s * spf:hi - s * spf]
+        got = out[lo - start:hi - start, :, 0].cpu().numpy()
+        assert np.array_equal(got.view('u4'), want.view('u4')), s
+    nfill = sum(min((u // nthread + 1) * spf, end)
+                - max(u // nthread * spf, start) for u in invalid)
+    assert int((out == fill).sum().item()) == nfill
+    del out
+    # the whole range decoded and encoded back: the valid units' payloads
+    full = kernels.decode_bitfield(raw, uo_inv, nset, nthread, payload, bps,
+                                   nelem, False, kernels.CODEC_LEVELS, lv,
+                                   fill)
+    back = torch.zeros_like(raw)
+    kernels.encode_bitfield(full, back, uo_inv, nset, nthread, payload, bps,
+                            nelem, kernels.QUANT_OFFSET_BINARY)
+    want = raw.clone()
+    want.view(-1, frame)[:, :32] = 0
+    want.view(-1, frame)[invalid] = 0
+    assert torch.equal(back, want)
+
+
+def test_rowword_encode_across_launch_split(emu):
+    """2-bit, two complex threads (ROWWORD2): just over 2^26 word positions,
+    invalid units on both sides of the split stay untouched, the valid ones
+    re-encode to the payload they were decoded from."""
+    from bitfield_cases import plan_encode
+    bps, nelem, nthread, payload = 2, 2, 2, 8000
+    frame = payload + 32
+    nset = 0x3ffffff // (payload // 4) + 5
+    mode, _, nlaunch, split, _ = plan_encode(emu, nset, nthread, payload,
+                                             bps, nelem)
+    assert (mode, nlaunch) == ('ROWWORD2', 2) and 0 < split < nset - 1
+    raw, uo = _frames(nset * nthread, payload, 91)
+    data = kernels.decode_bitfield(raw, uo, nset, nthread, payload, bps,
+                                   nelem, True, kernels.CODEC_LEVELS,
+                                   levels.offset_binary(2))
+    invalid = [split * nthread - 2, split * nthread - 1, split * nthread + 1,
+               nset * nthread - 1]
+    uo_inv = uo.clone()
+    uo_inv[invalid] = -1
+    back = torch.full_like(raw, 0xEE)
+    kernels.encode_bitfield(data, back, uo_inv, nset, nthread, payload, bps,
+                            nelem, kernels.QUANT_OFFSET_BINARY)
+    want = raw.clone()
+    want.view(-1, frame)[:, :32] = 0xEE
+    want.view(-1, frame)[invalid] = 0xEE
+    assert torch.equal(back, want)
