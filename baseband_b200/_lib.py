@@ -16,7 +16,7 @@ BB_OK, BB_ERR_ARGUMENT, BB_ERR_ALIGNMENT, BB_ERR_UNSUPPORTED, BB_ERR_CUDA = (
     0, -1, -2, -3, -4)
 CODEC_LEVELS, CODEC_SINT = 0, 1
 QUANT_OFFSET_BINARY, QUANT_MARK5B, QUANT_SINT = 0, 1, 2
-F32, F64 = 0, 1
+F32, F64, F16, BF16 = 0, 1, 2, 3
 
 _pf = POINTER(c_float)
 _pi64 = c_void_p      # device int64*
@@ -43,12 +43,18 @@ SIGNATURES = {
     'bb_decode_bitfield': (c_int, [
         _pv, _pi64, c_int64, c_int32, c_int64, c_int32, c_int32, c_int32,
         c_int32, _pf, c_float, c_int64, c_int64, _pv, c_void_p]),
+    'bb_decode_bitfield_typed': (c_int, [
+        _pv, _pi64, c_int64, c_int32, c_int64, c_int32, c_int32, c_int32,
+        c_int32, _pf, c_float, c_int64, c_int64, c_int32, _pv, c_void_p]),
     'bb_encode_bitfield': (c_int, [
         _pv, c_int32, _pv, _pi64, c_int64, c_int32, c_int64, c_int32,
         c_int32, c_int32, c_void_p]),
     'bb_mark4_decode': (c_int, [
         _pv, _pi64, c_int64, c_int32, c_int32, c_int32, _pf, c_float,
         c_int64, c_int64, _pv, c_void_p]),
+    'bb_mark4_decode_typed': (c_int, [
+        _pv, _pi64, c_int64, c_int32, c_int32, c_int32, _pf, c_float,
+        c_int64, c_int64, c_int32, _pv, c_void_p]),
     'bb_mark4_encode': (c_int, [
         _pv, c_int32, _pv, _pi64, c_int64, c_int32, c_int32, c_int32,
         c_void_p]),
@@ -59,12 +65,18 @@ SIGNATURES = {
     'bb_decode_int8_transposed': (c_int, [
         _pv, _pi64, c_int64, c_int64, c_int64, c_int32, _pi64, _pi64, _pi64,
         _pv, c_void_p]),
+    'bb_decode_int8_transposed_typed': (c_int, [
+        _pv, _pi64, c_int64, c_int64, c_int64, c_int32, _pi64, _pi64, _pi64,
+        c_int32, _pv, c_void_p]),
     'bb_encode_int8_transposed': (c_int, [
         _pv, c_int32, _pv, _pi64, c_int64, c_int64, c_int64, c_int32,
         c_void_p]),
     'bb_decode_int8_timefirst': (c_int, [
         _pv, _pi64, c_int64, c_int64, c_int32, c_int32, c_int32, _pi64,
         _pi64, _pi64, _pv, c_void_p]),
+    'bb_decode_int8_timefirst_typed': (c_int, [
+        _pv, _pi64, c_int64, c_int64, c_int32, c_int32, c_int32, _pi64,
+        _pi64, _pi64, c_int32, _pv, c_void_p]),
     'bb_encode_int8_timefirst': (c_int, [
         _pv, c_int32, _pv, _pi64, c_int64, c_int64, c_int32, c_int32,
         c_int32, c_void_p]),
@@ -119,6 +131,11 @@ SIGNATURES = {
 
 # every symbol include/baseband_b200.h declares
 EXPORTS = tuple(SIGNATURES)
+# the reduced-precision decoders: bound when present, asked for by name when
+# a float16 / bfloat16 result is wanted (`kernels._typed`)
+OPTIONAL = ('bb_decode_bitfield_typed', 'bb_mark4_decode_typed',
+            'bb_decode_int8_transposed_typed',
+            'bb_decode_int8_timefirst_typed')
 
 
 def bind(cdll, required=EXPORTS):
@@ -153,7 +170,8 @@ def load():
         # Every symbol of include/baseband_b200.h must be there; a partial
         # library is a build error, not something to work around.
         _lib = bind(ctypes.CDLL(LIB_PATH),
-                    required=() if os.environ.get('BB_ALLOW_PARTIAL') else EXPORTS)
+                    required=() if os.environ.get('BB_ALLOW_PARTIAL') else
+                    tuple(n for n in EXPORTS if n not in OPTIONAL))
         if _lib.bb_abi_version() != 2:
             raise ImportError('baseband_b200: ABI version mismatch')
     return _lib

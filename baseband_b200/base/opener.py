@@ -5,7 +5,7 @@ modes 'rb', 'wb', 'rs', 'ws' ('r'/'w' default to stream mode); ``name`` is a
 path or an open binary file handle; for writing, keyword arguments that are
 not reader/writer options are used to build ``header0`` through
 ``Header.fromvalues``.  The extra stream options of this implementation
-(``device``, ``chunk_nbytes``) are non-header keys, so they are never fed to
+(``device``, ``chunk_nbytes``, ``dtype``) are non-header keys, so they are never fed to
 the header (SURVEY.md section 5, "Config / flag system").
 """
 import io
@@ -14,7 +14,7 @@ import os
 __all__ = ['make_opener', 'make_info', 'normalize_mode']
 
 COMMON_NON_HEADER = {'squeeze', 'subset', 'fill_value', 'verify',
-                     'file_size', 'device', 'chunk_nbytes'}
+                     'file_size', 'device', 'chunk_nbytes', 'dtype'}
 
 
 def normalize_mode(mode):

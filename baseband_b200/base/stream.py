@@ -395,12 +395,13 @@ class _Stage:
         _device._threaded_copy(dst.reshape(-1).view(np.uint8),
                                src.numpy().reshape(-1).view(np.uint8))
 
-    def buffers(self, nbytes, nfloat, dev, need_dec):
+    def buffers(self, nbytes, nfloat, dev, need_dec, dtype=torch.float32):
         if self.pin is None or self.pin.numel() < nbytes:
             self.pin = _device.pinned_empty(nbytes, torch.uint8)
             self.raw = torch.empty(nbytes, dtype=torch.uint8, device=dev)
-        if need_dec and (self.dec is None or self.dec.numel() < nfloat):
-            self.dec = torch.empty(nfloat, dtype=torch.float32, device=dev)
+        if need_dec and (self.dec is None or self.dec.numel() < nfloat
+                         or self.dec.dtype != dtype):
+            self.dec = torch.empty(nfloat, dtype=dtype, device=dev)
         return self.pin[:nbytes], self.raw[:nbytes]
 
 
@@ -411,15 +412,26 @@ class StreamReaderBase(StreamBase):
     ``_file_offset0``) and ``_decode_chunk``; everything else is here.
 
     Parameters beyond the reference's: ``device`` (CUDA device to decode on;
-    when given, ``read`` returns a ``torch.Tensor`` on that device) and
-    ``chunk_nbytes`` (packed bytes per pipeline stage).
+    when given, ``read`` returns a ``torch.Tensor`` on that device),
+    ``chunk_nbytes`` (packed bytes per pipeline stage) and ``dtype``
+    (``None`` / ``'float32'``: float32 / complex64 samples as the reference
+    returns them; ``'float16'``: float16 / complex32; ``'bfloat16'``:
+    bfloat16, complex samples with a trailing axis of 2 (re, im); torch dtypes
+    are accepted too).  The kernels write the reduced types directly: every
+    value is the float32 result rounded to nearest even, as ``.to(dtype)``
+    rounds it.  With a reduced ``dtype``, ``read`` always returns a torch
+    tensor (numpy has neither bfloat16 nor complex half): on ``device``, or
+    in pinned host memory that the device-to-host copy lands in (small reads,
+    sliced from the decoded window, in ordinary host memory).
     """
 
     def __init__(self, fh_raw, header0, *, squeeze=True, subset=(),
                  fill_value=0., verify=True, device=None,
-                 chunk_nbytes=None, **kwargs):
+                 chunk_nbytes=None, dtype=None, **kwargs):
         super().__init__(fh_raw, header0, squeeze=squeeze, device=device,
                          **kwargs)
+        # the torch dtype the kernels write: float32, float16 or bfloat16
+        self._dec_dtype = _decode_dtype_arg(dtype)
         if subset is None:
             subset = ()
         elif not isinstance(subset, tuple):
@@ -436,6 +448,42 @@ class StreamReaderBase(StreamBase):
 
     subset = property(lambda self: self._subset)
     fill_value = property(lambda self: self._fill_value)
+
+    @property
+    def dtype(self):
+        """Element type of what ``read`` returns: the numpy float32 /
+        complex64 of the reference by default, else the torch dtype
+        (float16, complex32 or bfloat16)."""
+        if self._dec_dtype == torch.float32:
+            return StreamBase.dtype.fget(self)
+        return self._result_dtype(self._dec_dtype)
+
+    def _result_dtype(self, dec):
+        """torch dtype of the samples decoded as ``dec`` elements."""
+        if not self._complex_data:
+            return dec
+        return {torch.float32: torch.complex64,
+                torch.float16: torch.complex32}.get(dec, dec)
+
+    def _pair_axis(self, dec):
+        """(2,) where complex samples keep a (re, im) axis (bfloat16)."""
+        return (2,) if self._complex_data and dec == torch.bfloat16 else ()
+
+    def _read_decode_dtype(self, out):
+        """Element type the kernels write for a read into ``out``: the
+        reader's, except that a float32 reader handed a float16 / complex32 /
+        (real) bfloat16 torch tensor decodes straight to it."""
+        if self._dec_dtype == torch.float32 and isinstance(out, torch.Tensor):
+            for dec in (torch.float16, torch.bfloat16):
+                if (out.dtype == self._result_dtype(dec)
+                        and not self._pair_axis(dec)):
+                    return dec
+        return self._dec_dtype
+
+    def _complex_view(self, t):
+        """Decoded (..., 2) elements -> complex samples (bfloat16: kept
+        as they are)."""
+        return t if t.dtype == torch.bfloat16 else torch.view_as_complex(t)
 
     # --------------------------------------------------------------- shapes
     @property
@@ -544,7 +592,10 @@ class StreamReaderBase(StreamBase):
         Returns an array ``(count,) + sample_shape`` of float32/complex64:
         a `numpy.ndarray`, or a CUDA `torch.Tensor` if the stream was opened
         with ``device=`` or ``out`` is a CUDA tensor.  ``out`` may be a numpy
-        array or a torch tensor whose leading dimension sets ``count``.
+        array or a torch tensor whose leading dimension sets ``count``.  With
+        a reduced ``dtype`` (see the class) the result is a torch tensor of
+        that type; ``out`` is then a torch tensor of it, or, for real float16
+        streams, also a numpy float16 array.
 
         ``on_device`` (extension): a callable that is handed every decoded
         chunk as a CUDA tensor ``(n,) + sample_shape``, in order, on the
@@ -558,9 +609,17 @@ class StreamReaderBase(StreamBase):
             if count is None or count < 0:
                 count = max(0, self._nsample - self.offset)
         else:
-            assert tuple(out.shape[1:]) == tuple(self.sample_shape), (
-                "'out' must have trailing shape {}".format(
-                    tuple(self.sample_shape)))
+            trailing = tuple(self.sample_shape) + self._pair_axis(
+                self._dec_dtype)
+            assert tuple(out.shape[1:]) == trailing, (
+                "'out' must have trailing shape {}".format(trailing))
+            if (isinstance(out, np.ndarray)
+                    and self._dec_dtype != torch.float32
+                    and (self.dtype != torch.float16
+                         or out.dtype != np.float16)):
+                raise TypeError('out must be a torch tensor of {}{}'.format(
+                    self.dtype, ' or a numpy float16 array'
+                    if self.dtype == torch.float16 else ''))
             count = out.shape[0]
         if count > 0 and (self.offset < 0
                           or self.offset + count > self._nsample):
@@ -570,7 +629,7 @@ class StreamReaderBase(StreamBase):
         if (not to_device and on_device is None and count > 0
                 and self._small_read_cache_ok
                 and (out is None or isinstance(out, np.ndarray))
-                and count * self._floats_per_sample * 4
+                and count * self._floats_per_sample * self._dec_dtype.itemsize
                 <= self.SMALL_READ_NBYTES):
             result = self._read_small_cached(self.offset, count, out)
             self.offset += count
@@ -601,7 +660,7 @@ class StreamReaderBase(StreamBase):
     _small_read_cache_ok = True
 
     def _read_small_cached(self, start, count, out):
-        nb = self._floats_per_sample * 4
+        nb = self._floats_per_sample * self._dec_dtype.itemsize
         block = max(1, min(self._samples_per_frame,
                            self.SMALL_READ_WINDOW_NBYTES // nb))
         cache = self._small_cache
@@ -613,7 +672,8 @@ class StreamReaderBase(StreamBase):
             cache = self._small_cache = (w0, w1, data, self._fill_value)
         piece = cache[2][start - cache[0]:start - cache[0] + count]
         if out is None:
-            return piece.copy()
+            return piece.clone() if isinstance(piece, torch.Tensor) \
+                else piece.copy()
         out[...] = piece
         return out
 
@@ -852,7 +912,8 @@ class StreamReaderBase(StreamBase):
     def _decode_chunk(self, raw, frame0, nframe, sample_start, nsample, out):
         """Decode ``nsample`` samples starting ``sample_start`` samples into
         the first frame of ``raw`` (device bytes of ``nframe`` frames) into
-        the float32 device tensor ``out`` (flat, unsliced sample layout)."""
+        the float32, float16 or bfloat16 device tensor ``out`` (flat,
+        unsliced sample layout)."""
         raise NotImplementedError
 
     # -- helpers ---------------------------------------------------------
@@ -864,10 +925,10 @@ class StreamReaderBase(StreamBase):
         return n
 
     def _finish(self, flat, nsample):
-        """float32 device buffer -> (nsample, *sample_shape) tensor."""
+        """Decoded device buffer -> (nsample, *sample_shape) tensor."""
         shape = tuple(self._unsliced_shape)
         if self._complex_data:
-            data = torch.view_as_complex(
+            data = self._complex_view(
                 flat[:nsample * self._floats_per_sample].view(
                     (nsample,) + shape + (2,)))
         else:
@@ -995,14 +1056,14 @@ class StreamReaderBase(StreamBase):
     def _read_to_device(self, start, count, out):
         dev = out.device if out is not None else self.device
         fps = self._floats_per_sample
+        dec = self._read_decode_dtype(out)
         direct = (out is not None and not self._subset and out.is_contiguous()
-                  and out.dtype == (torch.complex64 if self._complex_data
-                                    else torch.float32))
+                  and out.dtype == self._result_dtype(dec))
         if direct:
-            flat = (torch.view_as_real(out) if self._complex_data
+            flat = (torch.view_as_real(out) if out.is_complex()
                     else out).reshape(-1)
         else:
-            flat = torch.empty(count * fps, dtype=torch.float32, device=dev)
+            flat = torch.empty(count * fps, dtype=dec, device=dev)
         stages, ss = self._pipeline(dev)
         ss.after_caller(1)
         chunks = list(self._chunks(start, count))
@@ -1051,8 +1112,9 @@ class StreamReaderBase(StreamBase):
         with ss.use(1):
             ss.wait_event(1, st.done)
             piece = flat[row * fps:(row + ns) * fps]
-            if piece.data_ptr() % 16:
-                tmp = torch.empty(ns * fps, dtype=torch.float32, device=dev)
+            # the kernels store 4 elements at a time (16 / 8 bytes)
+            if piece.data_ptr() % (4 * piece.element_size()):
+                tmp = torch.empty(ns * fps, dtype=piece.dtype, device=dev)
                 self._decode_chunk(raw, f0, nf, s0, ns, tmp)
                 piece.copy_(tmp)
             else:
@@ -1065,21 +1127,23 @@ class StreamReaderBase(StreamBase):
     def _read_to_host(self, start, count, out):
         dev = self.device
         fps = self._floats_per_sample
-        shape = (count,) + tuple(self.sample_shape)
-        np_dtype = self.dtype
-        t_dtype = torch.complex64 if self._complex_data else torch.float32
+        dec = self._read_decode_dtype(out)
+        shape = (count,) + tuple(self.sample_shape) + self._pair_axis(dec)
+        t_dtype = self._result_dtype(dec)
+        reduced = dec != torch.float32
         staged = False
         if out is None:
             # The result itself is pinned memory: D2H lands in it directly.
             holder = (_device.pinned_empty(shape, t_dtype) if count > 0
                       else torch.empty(shape, dtype=t_dtype))
             target = holder
-            result = holder.numpy()
+            result = holder if reduced else holder.numpy()
         elif isinstance(out, torch.Tensor):
             target, result = out, out
         else:
             result = out
-            target = _as_host_tensor(out, np_dtype)
+            target = _as_host_tensor(out, np.dtype(np.float16) if reduced
+                                     else self.dtype)
             # A large pageable destination: page-locking it in place costs
             # more than it saves (cudaHostRegister pins ~10 GB/s), so each
             # chunk lands in the stage's pinned buffer and is copied on by a
@@ -1097,7 +1161,7 @@ class StreamReaderBase(StreamBase):
                 st.flush()
                 if st.done is not None:
                     st.done.synchronize()
-                pin, raw = st.buffers(nbytes, ns * fps, dev, True)
+                pin, raw = st.buffers(nbytes, ns * fps, dev, True, dec)
                 got = self._read_raw(f0, nf, pin, s0, ns)
                 pin = pin if got is None else got
                 with ss.use(0):
@@ -1178,6 +1242,22 @@ class StreamReaderBase(StreamBase):
         self.__dict__.update(state)
         if '_slots_host' in state:
             self._slots_dev = None
+
+
+_DECODE_DTYPES = {None: torch.float32, 'float32': torch.float32,
+                  torch.float32: torch.float32, 'float16': torch.float16,
+                  torch.float16: torch.float16, 'bfloat16': torch.bfloat16,
+                  torch.bfloat16: torch.bfloat16}
+
+
+def _decode_dtype_arg(dtype):
+    """The reader's ``dtype`` argument -> torch dtype the kernels write."""
+    try:
+        return _DECODE_DTYPES[dtype]
+    except (KeyError, TypeError):
+        raise ValueError("dtype must be None, 'float32', 'float16' or "
+                         "'bfloat16' (or the torch dtype), not {!r}"
+                         .format(dtype)) from None
 
 
 def _torch_index(subset, dev):

@@ -62,7 +62,7 @@ inline unsigned tile_grid(uint32_t nitems, int unroll) {
 
 // The decode table lives in shared memory (see DecodeLut): built per CTA from
 // the per-code levels in the kernel parameters (at most 256 floats).
-template <int BPS, int CODEC, int MODE, bool SEL = false>
+template <int BPS, int CODEC, int MODE, bool SEL, typename OT>
 __global__ void __launch_bounds__(kBlock)
 k_decode_bitfield(const DecGeom p, const LevelTable<BPS> lv) {
     using Lut = DecodeLut<BPS>;
@@ -97,8 +97,8 @@ k_decode_bitfield(const DecGeom p, const LevelTable<BPS> lv) {
                 for (int j = 0; j < F; ++j) {
                     const uint32_t src = wr_src_lane<BPS>(lane, j);
                     const uint32_t ws = __shfl_sync(0xffffffffu, w[b], src);
-                    wr_emit<BPS, CODEC>(p, lut, item >> 5, lane, j, ws,
-                                        (okmask >> src) & 1u);
+                    wr_emit<BPS, CODEC, OT>(p, lut, item >> 5, lane, j, ws,
+                                            (okmask >> src) & 1u);
                 }
             }
         }
@@ -143,8 +143,8 @@ k_decode_bitfield(const DecGeom p, const LevelTable<BPS> lv) {
                 // two separate loops: the interior one stays free of the
                 // edge path's bounds arithmetic
                 if (wrow_interior<BPS, G>(p, item >> 5)) {   // warp uniform
-                    float *chunk_out = wrow_chunk_out<BPS, G, NG>(p,
-                                                                  item >> 5);
+                    OT *chunk_out = wrow_chunk_out<BPS, G, NG, OT>(p,
+                                                                   item >> 5);
 #pragma unroll
                     for (int j = 0; j < NST; ++j) {
                         const uint32_t q = lane + 32u * j;
@@ -171,7 +171,7 @@ k_decode_bitfield(const DecGeom p, const LevelTable<BPS> lv) {
 #pragma unroll
                     for (int g = 0; g < G; ++g)
                         ws[g] = wbuf[warp][b][src][grp * G + g];
-                    wrow_emit<BPS, CODEC, G, NG>(
+                    wrow_emit<BPS, CODEC, G, NG, OT>(
                         p, lut, item >> 5, lane, j, ws,
                         (okbuf[warp][b][src] >> (grp * G))
                         & ((1u << G) - 1u));
@@ -200,7 +200,7 @@ k_decode_bitfield(const DecGeom p, const LevelTable<BPS> lv) {
             }
 #pragma unroll
             for (int b = 0; b < RB; ++b)
-                rowgroup_emit<BPS, CODEC, G, SEL>(p, lut, it[b], lv);
+                rowgroup_emit<BPS, CODEC, G, SEL, OT>(p, lut, it[b], lv);
         }
         return;
     }
@@ -215,7 +215,8 @@ k_decode_bitfield(const DecGeom p, const LevelTable<BPS> lv) {
                 if (item < p.nitems) runs_fetch<BPS>(p, item, it[b]);
             }
 #pragma unroll
-            for (int b = 0; b < B; ++b) runs_emit<BPS, CODEC>(p, lut, it[b]);
+            for (int b = 0; b < B; ++b)
+                runs_emit<BPS, CODEC, OT>(p, lut, it[b]);
         }
         return;
     }
@@ -230,7 +231,7 @@ k_decode_bitfield(const DecGeom p, const LevelTable<BPS> lv) {
                 if (item < p.nitems) run_fetch<BPS>(p, item, it[b]);
             }
 #pragma unroll
-            for (int b = 0; b < B; ++b) run_emit<BPS, CODEC>(p, lut, it[b]);
+            for (int b = 0; b < B; ++b) run_emit<BPS, CODEC, OT>(p, lut, it[b]);
         }
         return;
     }
@@ -238,13 +239,13 @@ k_decode_bitfield(const DecGeom p, const LevelTable<BPS> lv) {
     for (int u = 0; u < U; ++u) {
         const uint32_t item = item0 + u * kBlock;
         if (item >= p.nitems) break;
-        dec_scalar<BPS, CODEC>(p, lut, item);
+        dec_scalar<BPS, CODEC, OT>(p, lut, item);
     }
 }
 
 // TILE (rows of four float4, see bb_bitfield.cuh): warp-cooperative, words
 // staged in shared memory, every store instruction 512 contiguous bytes.
-template <int BPS, int CODEC, int G, int P, bool SEL, int U>
+template <int BPS, int CODEC, int G, int P, bool SEL, int U, typename OT>
 __global__ void __launch_bounds__(kBlock)
 k_decode_tile(const DecGeom p, const LevelTable<BPS> lv) {
     using Lut = DecodeLut<BPS>;
@@ -286,7 +287,7 @@ k_decode_tile(const DecGeom p, const LevelTable<BPS> lv) {
             if (item >= p.nitems) break;          // warp uniform
             const uint32_t chunk = item >> 5;
             if (full[b] && tile_interior<BPS, G, P>(p, chunk)) {
-                float *chunk_out = tile_chunk_out<BPS, G, P>(p, chunk);
+                OT *chunk_out = tile_chunk_out<BPS, G, P, OT>(p, chunk);
 #pragma unroll
                 for (int j = 0; j < T::kStores; ++j) {
                     const uint32_t q = lane + 32u * j;
@@ -295,8 +296,8 @@ k_decode_tile(const DecGeom p, const LevelTable<BPS> lv) {
                     uint32_t ws[G];
 #pragma unroll
                     for (int g = 0; g < G; ++g) ws[g] = wbuf[warp][b][at + g];
-                    *reinterpret_cast<F4 *>(chunk_out + 4u * q) =
-                        tile_decode<BPS, CODEC, G, P, SEL>(q, ws, lut, lv);
+                    store4(chunk_out + 4u * q,
+                           tile_decode<BPS, CODEC, G, P, SEL>(q, ws, lut, lv));
                 }
                 continue;
             }
@@ -310,7 +311,8 @@ k_decode_tile(const DecGeom p, const LevelTable<BPS> lv) {
                 for (int g = 0; g < G; ++g) ws[g] = wbuf[warp][b][at + g];
                 const uint32_t okm = full[b] ? (1u << G) - 1u
                     : tile_group_ok<BPS, G, P>(okbuf[warp][b], q);
-                tile_emit<BPS, CODEC, G, P, SEL>(p, lut, lv, chunk, q, ws, okm);
+                tile_emit<BPS, CODEC, G, P, SEL, OT>(p, lut, lv, chunk, q, ws,
+                                                     okm);
             }
         }
     }
@@ -394,51 +396,51 @@ k_encode_bitfield(const EncGeom p, const QuantConsts<T> c) {
 
 // The 2-bit level-table variants under evaluation (register select, TILE).
 // Returns false if the launch is not one of them.
-template <int BPS, int CODEC, int G, int P, bool SEL>
+template <int BPS, int CODEC, int G, int P, bool SEL, typename OT>
 static void launch_tile(const DecLaunch &l, const LevelTable<BPS> &lv,
                         cudaStream_t stream) {
     if (l.tile_u >= 2)
-        k_decode_tile<BPS, CODEC, G, P, SEL, 2>
+        k_decode_tile<BPS, CODEC, G, P, SEL, 2, OT>
             <<<tile_grid(l.g.nitems, 2), kBlock, 0, stream>>>(l.g, lv);
     else
-        k_decode_tile<BPS, CODEC, G, P, SEL, 1>
+        k_decode_tile<BPS, CODEC, G, P, SEL, 1, OT>
             <<<tile_grid(l.g.nitems, 1), kBlock, 0, stream>>>(l.g, lv);
 }
 
-template <int BPS, int CODEC>
+template <int BPS, int CODEC, typename OT>
 static bool launch_c2(const DecLaunch &l, const LevelTable<BPS> &lv,
                       cudaStream_t stream) {
     const uint32_t n = l.g.nitems;
     if (l.mode == MODE_ROWGROUP4 && l.sel) {
-        k_decode_bitfield<BPS, CODEC, MODE_ROWGROUP4, true>
+        k_decode_bitfield<BPS, CODEC, MODE_ROWGROUP4, true, OT>
             <<<tile_grid(n, Unroll<BPS, MODE_ROWGROUP4>::value), kBlock, 0,
                stream>>>(l.g, lv);
         return true;
     }
     if (l.mode == MODE_ROWGROUP2 && l.sel) {
-        k_decode_bitfield<BPS, CODEC, MODE_ROWGROUP2, true>
+        k_decode_bitfield<BPS, CODEC, MODE_ROWGROUP2, true, OT>
             <<<tile_grid(n, Unroll<BPS, MODE_ROWGROUP2>::value), kBlock, 0,
                stream>>>(l.g, lv);
         return true;
     }
     if (l.mode == MODE_TILE4) {
-        if (l.tile_p == 8 && l.sel) launch_tile<BPS, CODEC, 4, 8, true>(l, lv, stream);
-        else if (l.tile_p == 8) launch_tile<BPS, CODEC, 4, 8, false>(l, lv, stream);
-        else if (l.sel) launch_tile<BPS, CODEC, 4, 4, true>(l, lv, stream);
-        else launch_tile<BPS, CODEC, 4, 4, false>(l, lv, stream);
+        if (l.tile_p == 8 && l.sel) launch_tile<BPS, CODEC, 4, 8, true, OT>(l, lv, stream);
+        else if (l.tile_p == 8) launch_tile<BPS, CODEC, 4, 8, false, OT>(l, lv, stream);
+        else if (l.sel) launch_tile<BPS, CODEC, 4, 4, true, OT>(l, lv, stream);
+        else launch_tile<BPS, CODEC, 4, 4, false, OT>(l, lv, stream);
         return true;
     }
     if (l.mode == MODE_TILE2) {
-        if (l.tile_p == 8 && l.sel) launch_tile<BPS, CODEC, 2, 8, true>(l, lv, stream);
-        else if (l.tile_p == 8) launch_tile<BPS, CODEC, 2, 8, false>(l, lv, stream);
-        else if (l.sel) launch_tile<BPS, CODEC, 2, 4, true>(l, lv, stream);
-        else launch_tile<BPS, CODEC, 2, 4, false>(l, lv, stream);
+        if (l.tile_p == 8 && l.sel) launch_tile<BPS, CODEC, 2, 8, true, OT>(l, lv, stream);
+        else if (l.tile_p == 8) launch_tile<BPS, CODEC, 2, 8, false, OT>(l, lv, stream);
+        else if (l.sel) launch_tile<BPS, CODEC, 2, 4, true, OT>(l, lv, stream);
+        else launch_tile<BPS, CODEC, 2, 4, false, OT>(l, lv, stream);
         return true;
     }
     return false;
 }
 
-template <int BPS, int CODEC>
+template <int BPS, int CODEC, typename OT>
 static int launch_decode(const std::vector<DecLaunch> &launches,
                          const float *levels_host, cudaStream_t stream) {
     LevelTable<BPS> lv;
@@ -447,59 +449,59 @@ static int launch_decode(const std::vector<DecLaunch> &launches,
     for (const DecLaunch &l : launches) {
         const uint32_t n = l.g.nitems;
         if constexpr (BPS == 2 && CODEC == CODEC_LEVELS) {
-            if (launch_c2<BPS, CODEC>(l, lv, stream)) {
+            if (launch_c2<BPS, CODEC, OT>(l, lv, stream)) {
                 BB_CHECK_LAUNCH("bb_decode_bitfield launch");
                 continue;
             }
         }
         switch (l.mode) {
         case MODE_ROWGROUP4:
-            k_decode_bitfield<BPS, CODEC, MODE_ROWGROUP4>
+            k_decode_bitfield<BPS, CODEC, MODE_ROWGROUP4, false, OT>
                 <<<tile_grid(n, Unroll<BPS, MODE_ROWGROUP4>::value), kBlock, 0,
                    stream>>>(l.g, lv);
             break;
         case MODE_ROWGROUP2:
-            k_decode_bitfield<BPS, CODEC, MODE_ROWGROUP2>
+            k_decode_bitfield<BPS, CODEC, MODE_ROWGROUP2, false, OT>
                 <<<tile_grid(n, Unroll<BPS, MODE_ROWGROUP2>::value), kBlock, 0,
                    stream>>>(l.g, lv);
             break;
         case MODE_RUN:
-            k_decode_bitfield<BPS, CODEC, MODE_RUN>
+            k_decode_bitfield<BPS, CODEC, MODE_RUN, false, OT>
                 <<<tile_grid(n, Unroll<BPS, MODE_RUN>::value), kBlock, 0,
                    stream>>>(l.g, lv);
             break;
         case MODE_RUNS:
-            k_decode_bitfield<BPS, CODEC, MODE_RUNS>
+            k_decode_bitfield<BPS, CODEC, MODE_RUNS, false, OT>
                 <<<tile_grid(n, Unroll<BPS, MODE_RUNS>::value), kBlock, 0,
                    stream>>>(l.g, lv);
             break;
         case MODE_WORDRUN:
-            k_decode_bitfield<BPS, CODEC, MODE_WORDRUN>
+            k_decode_bitfield<BPS, CODEC, MODE_WORDRUN, false, OT>
                 <<<tile_grid(n, Unroll<BPS, MODE_WORDRUN>::value), kBlock, 0,
                    stream>>>(l.g, lv);
             break;
         case MODE_WORDROW4:
-            k_decode_bitfield<BPS, CODEC, MODE_WORDROW4>
+            k_decode_bitfield<BPS, CODEC, MODE_WORDROW4, false, OT>
                 <<<tile_grid(n, Unroll<BPS, MODE_WORDROW4>::value), kBlock, 0,
                    stream>>>(l.g, lv);
             break;
         case MODE_WORDROW2:
-            k_decode_bitfield<BPS, CODEC, MODE_WORDROW2>
+            k_decode_bitfield<BPS, CODEC, MODE_WORDROW2, false, OT>
                 <<<tile_grid(n, Unroll<BPS, MODE_WORDROW2>::value), kBlock, 0,
                    stream>>>(l.g, lv);
             break;
         case MODE_WORDROW4X2:
-            k_decode_bitfield<BPS, CODEC, MODE_WORDROW4X2>
+            k_decode_bitfield<BPS, CODEC, MODE_WORDROW4X2, false, OT>
                 <<<tile_grid(n, Unroll<BPS, MODE_WORDROW4X2>::value), kBlock,
                    0, stream>>>(l.g, lv);
             break;
         case MODE_WORDROW2X2:
-            k_decode_bitfield<BPS, CODEC, MODE_WORDROW2X2>
+            k_decode_bitfield<BPS, CODEC, MODE_WORDROW2X2, false, OT>
                 <<<tile_grid(n, Unroll<BPS, MODE_WORDROW2X2>::value), kBlock,
                    0, stream>>>(l.g, lv);
             break;
         default:
-            k_decode_bitfield<BPS, CODEC, MODE_SCALAR>
+            k_decode_bitfield<BPS, CODEC, MODE_SCALAR, false, OT>
                 <<<tile_grid(n, Unroll<BPS, MODE_SCALAR>::value), kBlock, 0,
                    stream>>>(l.g, lv);
         }
@@ -579,20 +581,50 @@ static int dispatch_encode(int bps, int quantiser,
                      quantiser);
 }
 
+template <typename OT>
+static int dispatch_decode(int bps, int codec, const float *levels_host,
+                           const std::vector<DecLaunch> &l, cudaStream_t s) {
+    if (codec == BB_CODEC_LEVELS) {
+        switch (bps) {
+        case 1: return launch_decode<1, CODEC_LEVELS, OT>(l, levels_host, s);
+        case 2: return launch_decode<2, CODEC_LEVELS, OT>(l, levels_host, s);
+        case 4: return launch_decode<4, CODEC_LEVELS, OT>(l, levels_host, s);
+        case 8:
+            if (affine8_matches(levels_host))       // the standard 8-bit table
+                return launch_decode<8, CODEC_AFFINE8, OT>(l, nullptr, s);
+            return launch_decode<8, CODEC_LEVELS, OT>(l, levels_host, s);
+        }
+    } else if (codec == BB_CODEC_SINT) {
+        switch (bps) {
+        case 4: return launch_decode<4, CODEC_SINT, OT>(l, nullptr, s);
+        case 8: return launch_decode<8, CODEC_SINT, OT>(l, nullptr, s);
+        }
+    }
+    return set_error(BB_ERR_UNSUPPORTED, "no decoder for bps=%d codec=%d", bps,
+                     codec);
+}
+
 }  // namespace bb
 
 using namespace bb;
 
-extern "C" int bb_decode_bitfield(
+extern "C" int bb_decode_bitfield_typed(
     const void *src, const int64_t *unit_offset, int64_t nset, int32_t nthread,
     int64_t payload_nbytes, int32_t bps, int32_t nelem, int32_t complex_data,
     int32_t codec, const float *levels_host, float fill_value,
-    int64_t sample_start, int64_t nsample, float *out, void *stream) {
+    int64_t sample_start, int64_t nsample, int32_t out_dtype, void *out,
+    void *stream) {
     if (!src || !unit_offset || !out)
         return set_error(BB_ERR_ARGUMENT, "null pointer argument");
-    if (!aligned(out, 16) || !aligned(src, 4))
+    const int esize = out_elem_nbytes(out_dtype);
+    if (esize == 0)
+        return set_error(BB_ERR_ARGUMENT,
+                         "out_dtype must be BB_F32, BB_F16 or BB_BF16");
+    const int out_align = 4 * esize;             // one float4-equivalent
+    if (!aligned(out, out_align) || !aligned(src, 4))
         return set_error(BB_ERR_ALIGNMENT,
-                         "out must be 16-byte and src 4-byte aligned");
+                         "out must be %d-byte and src 4-byte aligned",
+                         out_align);
     if (codec == BB_CODEC_LEVELS && !levels_host)
         return set_error(BB_ERR_ARGUMENT, "levels_host required");
     std::vector<DecLaunch> launches;
@@ -602,24 +634,23 @@ extern "C" int bb_decode_bitfield(
                      out, launches, err))
         return set_error(BB_ERR_ARGUMENT, "%s", err.c_str());
     cudaStream_t s = as_stream(stream);
-    if (codec == BB_CODEC_LEVELS) {
-        switch (bps) {
-        case 1: return launch_decode<1, CODEC_LEVELS>(launches, levels_host, s);
-        case 2: return launch_decode<2, CODEC_LEVELS>(launches, levels_host, s);
-        case 4: return launch_decode<4, CODEC_LEVELS>(launches, levels_host, s);
-        case 8:
-            if (affine8_matches(levels_host))       // the standard 8-bit table
-                return launch_decode<8, CODEC_AFFINE8>(launches, nullptr, s);
-            return launch_decode<8, CODEC_LEVELS>(launches, levels_host, s);
-        }
-    } else if (codec == BB_CODEC_SINT) {
-        switch (bps) {
-        case 4: return launch_decode<4, CODEC_SINT>(launches, nullptr, s);
-        case 8: return launch_decode<8, CODEC_SINT>(launches, nullptr, s);
-        }
-    }
-    return set_error(BB_ERR_UNSUPPORTED, "no decoder for bps=%d codec=%d", bps,
-                     codec);
+    if (out_dtype == BB_F16)
+        return dispatch_decode<F16>(bps, codec, levels_host, launches, s);
+    if (out_dtype == BB_BF16)
+        return dispatch_decode<BF16>(bps, codec, levels_host, launches, s);
+    return dispatch_decode<float>(bps, codec, levels_host, launches, s);
+}
+
+extern "C" int bb_decode_bitfield(
+    const void *src, const int64_t *unit_offset, int64_t nset, int32_t nthread,
+    int64_t payload_nbytes, int32_t bps, int32_t nelem, int32_t complex_data,
+    int32_t codec, const float *levels_host, float fill_value,
+    int64_t sample_start, int64_t nsample, float *out, void *stream) {
+    return bb_decode_bitfield_typed(src, unit_offset, nset, nthread,
+                                    payload_nbytes, bps, nelem, complex_data,
+                                    codec, levels_host, fill_value,
+                                    sample_start, nsample, BB_F32, out,
+                                    stream);
 }
 
 extern "C" int bb_encode_bitfield(

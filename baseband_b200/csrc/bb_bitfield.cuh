@@ -3,7 +3,10 @@
 // Logical layout (see include/baseband_b200.h, bb_decode_bitfield):
 //   unit (set, slot): nword 32-bit words = codes of BPS bits, LSB first, in
 //                     order [time][E]   (E = nelem)
-//   out:              [row][slot][E] float32, row = set*spf + t - sample_start
+//   out:              [row][slot][E] float32 (or F16 / BF16: the emit steps
+//                     are templated on the output type OT; a "float4" below
+//                     is then four 16-bit values, 8 bytes),
+//                     row = set*spf + t - sample_start
 //
 // Three work decompositions, chosen by the launcher:
 //   ROWGROUP<G>  E*G == 4, nthread % G == 0.  A thread takes word k of G
@@ -62,7 +65,8 @@ struct DecodeLut {
 struct DecGeom {
     const uint8_t *src;
     const long long *unit_offset;   // [nset * nthread] for this launch
-    float *out;                     // row 0 of the whole call
+    void *out;                      // row 0 of the whole call (float32,
+                                    // F16 or BF16 elements)
     long long row_base;             // row of (set 0, t 0) of this launch
     long long nsample;              // valid rows are [0, nsample)
     uint32_t nset, nthread, nelem, nword;
@@ -234,7 +238,7 @@ BB_HD void rowgroup_fetch(const DecGeom &p, uint32_t item, RowItem<G> &it) {
     }
 }
 
-template <int BPS, int CODEC, int G, bool SEL = false>
+template <int BPS, int CODEC, int G, bool SEL = false, typename OT = float>
 BB_HD void rowgroup_emit(const DecGeom &p, const float *lut,
                          const RowItem<G> &it,
                          const LevelTable<BPS> &lv = LevelTable<BPS>()) {
@@ -245,7 +249,7 @@ BB_HD void rowgroup_emit(const DecGeom &p, const float *lut,
     const uint32_t *w = it.w;
     const long long row0 = it.row0;
     const size_t rowlen = (size_t)p.nthread * E;
-    float *dst = p.out + row0 * (long long)rowlen + it.g * 4;
+    OT *dst = out_as<OT>(p) + row0 * (long long)rowlen + it.g * 4;
     if (it.okmask == (1u << G) - 1u && row0 >= 0
         && row0 + TPW <= p.nsample) {
         // Fast path: all rows inside the requested range, every slot valid.
@@ -257,9 +261,9 @@ BB_HD void rowgroup_emit(const DecGeom &p, const float *lut,
                 F2 b = decode_pair_v<BPS, CODEC, SEL>(w[1 % G], m, lut, lv);
                 F2 c = decode_pair_v<BPS, CODEC, SEL>(w[2 % G], m, lut, lv);
                 F2 d = decode_pair_v<BPS, CODEC, SEL>(w[3 % G], m, lut, lv);
-                *reinterpret_cast<F4 *>(dst) = F4{a.x, b.x, c.x, d.x};
+                store4(dst, F4{a.x, b.x, c.x, d.x});
                 dst += rowlen;
-                *reinterpret_cast<F4 *>(dst) = F4{a.y, b.y, c.y, d.y};
+                store4(dst, F4{a.y, b.y, c.y, d.y});
                 dst += rowlen;
             }
         } else {
@@ -268,7 +272,7 @@ BB_HD void rowgroup_emit(const DecGeom &p, const float *lut,
                 const uint32_t i = c0 + ii;
                 F2 a = decode_pair_v<BPS, CODEC, SEL>(w[0], i, lut, lv);
                 F2 b = decode_pair_v<BPS, CODEC, SEL>(w[1 % G], i, lut, lv);
-                *reinterpret_cast<F4 *>(dst) = F4{a.x, a.y, b.x, b.y};
+                store4(dst, F4{a.x, a.y, b.x, b.y});
                 dst += rowlen;
             }
         }
@@ -301,15 +305,15 @@ BB_HD void rowgroup_emit(const DecGeom &p, const float *lut,
             v.z = ok1 ? b.x : p.fill;
             v.w = ok1 ? b.y : fill_im;
         }
-        *reinterpret_cast<F4 *>(dst) = v;
+        store4(dst, v);
     }
 }
 
-template <int BPS, int CODEC, int G>
+template <int BPS, int CODEC, int G, typename OT = float>
 BB_HD void dec_rowgroup(const DecGeom &p, const float *lut, uint32_t item) {
     RowItem<G> it;
     rowgroup_fetch<BPS, G>(p, item, it);
-    rowgroup_emit<BPS, CODEC, G>(p, lut, it);
+    rowgroup_emit<BPS, CODEC, G, false, OT>(p, lut, it);
 }
 
 // RUN: item = float4 index within the launch's block of rows; again split
@@ -353,7 +357,7 @@ BB_HD void run_fetch(const DecGeom &p, uint32_t item, RunItem &it) {
     }
 }
 
-template <int BPS, int CODEC>
+template <int BPS, int CODEC, typename OT = float>
 BB_HD void run_emit(const DecGeom &p, const float *lut, const RunItem &it) {
     if (it.gidx < 0) return;
     F4 v;
@@ -365,14 +369,14 @@ BB_HD void run_emit(const DecGeom &p, const float *lut, const RunItem &it) {
         const float fill_im = p.complex_fill ? 0.f : p.fill;
         v = F4{p.fill, fill_im, p.fill, fill_im};
     }
-    *reinterpret_cast<F4 *>(p.out + it.gidx) = v;
+    store4(out_as<OT>(p) + it.gidx, v);
 }
 
-template <int BPS, int CODEC>
+template <int BPS, int CODEC, typename OT = float>
 BB_HD void dec_run(const DecGeom &p, const float *lut, uint32_t item) {
     RunItem it;
     run_fetch<BPS>(p, item, it);
-    run_emit<BPS, CODEC>(p, lut, it);
+    run_emit<BPS, CODEC, OT>(p, lut, it);
 }
 
 // RUNS: RUN for words that hold S = tpw >= 1 complete samples of a thread slot
@@ -418,17 +422,16 @@ BB_HD void runs_fetch(const DecGeom &p, uint32_t item, RunsItem &it) {
     }
 }
 
-template <int BPS, int CODEC>
+template <int BPS, int CODEC, typename OT = float>
 BB_HD void runs_emit(const DecGeom &p, const float *lut, const RunsItem &it) {
     if (it.gidx < 0) return;
     const uint32_t S = p.tpw, R = p.runs_rows;
     const size_t rowlen = (size_t)p.nthread * p.nelem;
-    float *dst = p.out + it.gidx;
+    OT *dst = out_as<OT>(p) + it.gidx;
     const float fill_im = p.complex_fill ? 0.f : p.fill;
     if (!it.valid) {
         for (uint32_t r = 0; r < R; ++r, dst += rowlen)
-            *reinterpret_cast<F4 *>(dst) = F4{p.fill, fill_im, p.fill,
-                                              fill_im};
+            store4(dst, F4{p.fill, fill_im, p.fill, fill_im});
         return;
     }
 #pragma unroll
@@ -439,16 +442,16 @@ BB_HD void runs_emit(const DecGeom &p, const float *lut, const RunsItem &it) {
             const uint32_t pair = ((s << p.log2_nelem) + it.e) >> 1;
             F2 a = decode_pair<BPS, CODEC>(w, pair, lut);
             F2 b = decode_pair<BPS, CODEC>(w, pair + 1, lut);
-            *reinterpret_cast<F4 *>(dst) = F4{a.x, a.y, b.x, b.y};
+            store4(dst, F4{a.x, a.y, b.x, b.y});
         }
     }
 }
 
-template <int BPS, int CODEC>
+template <int BPS, int CODEC, typename OT = float>
 BB_HD void dec_runs(const DecGeom &p, const float *lut, uint32_t item) {
     RunsItem it;
     runs_fetch<BPS>(p, item, it);
-    runs_emit<BPS, CODEC>(p, lut, it);
+    runs_emit<BPS, CODEC, OT>(p, lut, it);
 }
 
 // WORDRUN: a warp owns chunk = 32 consecutive words of the launch (nthread
@@ -475,7 +478,7 @@ BB_HD bool wr_load(const DecGeom &p, uint32_t chunk, uint32_t lane,
     return true;
 }
 
-template <int BPS, int CODEC>
+template <int BPS, int CODEC, typename OT = float>
 BB_HD void wr_emit(const DecGeom &p, const float *lut, uint32_t chunk,
                    uint32_t lane, int j, uint32_t w, bool valid) {
     constexpr int F = 8 / BPS;
@@ -494,7 +497,7 @@ BB_HD void wr_emit(const DecGeom &p, const float *lut, uint32_t chunk,
         const float fill_im = p.complex_fill ? 0.f : p.fill;
         v = F4{p.fill, fill_im, p.fill, fill_im};
     }
-    *reinterpret_cast<F4 *>(p.out + gidx) = v;
+    store4(out_as<OT>(p) + gidx, v);
 }
 
 // WORDROW<G, NG>: nthread * E == 4 * NG (G = 4 single-channel threads or G = 2
@@ -566,7 +569,7 @@ BB_HD F4 wrow_decode(const DecGeom &p, const float *lut, uint32_t c,
 
 // Checked store (edges of the read / of the launch).  ``w`` and ``okmask``
 // are those of the float4's group.
-template <int BPS, int CODEC, int G, int NG>
+template <int BPS, int CODEC, int G, int NG, typename OT = float>
 BB_HD void wrow_emit(const DecGeom &p, const float *lut, uint32_t chunk,
                      uint32_t lane, int j, const uint32_t w[G],
                      uint32_t okmask) {
@@ -576,8 +579,8 @@ BB_HD void wrow_emit(const DecGeom &p, const float *lut, uint32_t chunk,
     if (chunk * 32u + r / TPW >= p.nwords_total) return;
     const long long row = p.row_base + ((long long)chunk * 32 * TPW + r);
     if (row < 0 || row >= p.nsample) return;
-    *reinterpret_cast<F4 *>(p.out + (row * NG + q % NG) * 4) =
-        wrow_decode<BPS, CODEC, G>(p, lut, r % TPW, w, okmask);
+    store4(out_as<OT>(p) + (row * NG + q % NG) * 4,
+           wrow_decode<BPS, CODEC, G>(p, lut, r % TPW, w, okmask));
 }
 
 // Interior chunks (all 32 word positions inside the launch, all 32 * TPW rows
@@ -592,18 +595,18 @@ BB_HD bool wrow_interior(const DecGeom &p, uint32_t chunk) {
     return row0 >= 0 && row0 + 32 * TPW <= p.nsample;
 }
 
-template <int BPS, int G, int NG>
-BB_HD float *wrow_chunk_out(const DecGeom &p, uint32_t chunk) {
+template <int BPS, int G, int NG, typename OT = float>
+BB_HD OT *wrow_chunk_out(const DecGeom &p, uint32_t chunk) {
     constexpr int TPW = (32 / BPS) / (4 / G);
-    return p.out + (p.row_base + (long long)chunk * (32 * TPW)) * (4 * NG);
+    return out_as<OT>(p) + (p.row_base + (long long)chunk * (32 * TPW)) * (4 * NG);
 }
 
-template <int BPS, int CODEC, int G, int NG>
-BB_HD void wrow_emit_fast(const DecGeom &p, const float *lut, float *chunk_out,
+template <int BPS, int CODEC, int G, int NG, typename OT>
+BB_HD void wrow_emit_fast(const DecGeom &p, const float *lut, OT *chunk_out,
                           uint32_t q, const uint32_t w[G], uint32_t okmask) {
     constexpr int TPW = (32 / BPS) / (4 / G);
-    *reinterpret_cast<F4 *>(chunk_out + 4u * q) =
-        wrow_decode<BPS, CODEC, G>(p, lut, (q / NG) % TPW, w, okmask);
+    store4(chunk_out + 4u * q,
+           wrow_decode<BPS, CODEC, G>(p, lut, (q / NG) % TPW, w, okmask));
 }
 
 // TILE<G, P>: rows of exactly four float4 (16 single-channel threads with
@@ -662,10 +665,10 @@ BB_HD bool tile_interior(const DecGeom &p, uint32_t chunk) {
     return row0 >= 0 && row0 + P * T::kTpw <= p.nsample;
 }
 
-template <int BPS, int G, int P>
-BB_HD float *tile_chunk_out(const DecGeom &p, uint32_t chunk) {
+template <int BPS, int G, int P, typename OT = float>
+BB_HD OT *tile_chunk_out(const DecGeom &p, uint32_t chunk) {
     using T = Tile<BPS, G, P>;
-    return p.out + (p.row_base + (long long)chunk * (P * T::kTpw)) * 16;
+    return out_as<OT>(p) + (p.row_base + (long long)chunk * (P * T::kTpw)) * 16;
 }
 
 // float4 q of a chunk from the G words `w` of its group (all slots valid).
@@ -686,7 +689,7 @@ BB_HD F4 tile_decode(uint32_t q, const uint32_t w[G], const float *lut,
 
 // Checked store for edge chunks / chunks with invalid units.  okmask: bit s =
 // slot s of the float4's group valid.
-template <int BPS, int CODEC, int G, int P, bool SEL>
+template <int BPS, int CODEC, int G, int P, bool SEL, typename OT = float>
 BB_HD void tile_emit(const DecGeom &p, const float *lut,
                      const LevelTable<BPS> &lv, uint32_t chunk, uint32_t q,
                      const uint32_t w[G], uint32_t okmask) {
@@ -708,7 +711,7 @@ BB_HD void tile_emit(const DecGeom &p, const float *lut,
             if (!(okmask & 2u)) { v.z = p.fill; v.w = fill_im; }
         }
     }
-    *reinterpret_cast<F4 *>(p.out + (row * 4 + (q & 3u)) * 4) = v;
+    store4(out_as<OT>(p) + (row * 4 + (q & 3u)) * 4, v);
 }
 
 // Valid bits of group g = q & 3 of the row of float4 q, from the per-lane
@@ -728,7 +731,7 @@ BB_HD uint32_t tile_group_ok(const uint32_t *oks, uint32_t q) {
 }
 
 // SCALAR: item = element index within the launch's block of rows.
-template <int BPS, int CODEC>
+template <int BPS, int CODEC, typename OT = float>
 BB_HD void dec_scalar(const DecGeom &p, const float *lut, uint32_t item) {
     constexpr int CPW = 32 / BPS;
     const uint32_t rowlen = p.nthread * p.nelem;
@@ -747,7 +750,7 @@ BB_HD void dec_scalar(const DecGeom &p, const float *lut, uint32_t item) {
     } else {
         v = (p.complex_fill && (e & 1u)) ? 0.f : p.fill;
     }
-    p.out[gidx] = v;
+    store1(out_as<OT>(p) + gidx, v);
 }
 
 // ------------------------------------------------------------------ encode

@@ -85,7 +85,7 @@ inline int pick_mode(int nelem, int nthread, bool aligned_rows,
 inline bool plan_decode(const void *src, const int64_t *unit_offset,
                         int64_t nset, int nthread, int64_t payload_nbytes,
                         int bps, int nelem, int complex_data, float fill,
-                        int64_t sample_start, int64_t nsample, float *out,
+                        int64_t sample_start, int64_t nsample, void *out,
                         std::vector<DecLaunch> &launches, std::string &err) {
     uint32_t nword, spf;
     if (!plan_geometry(payload_nbytes, bps, nelem, nthread, nset, nword, spf,

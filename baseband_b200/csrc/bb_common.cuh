@@ -114,6 +114,93 @@ BB_HD float uint_as_float(uint32_t u) {
 BB_HD float small_int_to_float(int32_t i) {
     return add_rn(uint_as_float(0x4B400000u + (uint32_t)i), -12582912.0f);
 }
+// ------------------------------------------------- decoder output element types
+// A decoder writes float32 (`float`) or the 16-bit patterns of IEEE half
+// (F16) or bfloat16 (BF16).  The kernels compute every value in float32 and
+// round it to the output type once, when it is stored (round to nearest even,
+// overflow to +-inf: torch's `.to(dtype)`), so a reduced-precision result is
+// the float32 result converted elementwise.
+struct alignas(2) F16 { uint16_t bits; static constexpr bool kBrain = false; };
+struct alignas(2) BF16 { uint16_t bits; static constexpr bool kBrain = true; };
+struct alignas(8) H4 { uint32_t lo, hi; };
+
+BB_HD uint32_t float_as_uint(float f) {
+#if defined(__CUDA_ARCH__)
+    return __float_as_uint(f);
+#else
+    uint32_t u;
+    __builtin_memcpy(&u, &f, 4);
+    return u;
+#endif
+}
+
+// Host rounding of a float32 bit pattern (the CPU emulation and the tests).
+// NaN keeps its sign and becomes a quiet NaN; its payload is not specified.
+inline uint16_t f32_to_f16_bits(uint32_t x) {
+    const uint32_t sign = (x >> 16) & 0x8000u, ax = x & 0x7fffffffu;
+    if (ax > 0x7f800000u) return (uint16_t)(sign | 0x7e00u);
+    if (ax >= 0x477ff000u) return (uint16_t)(sign | 0x7c00u);  // >= 65520
+    if (ax >= 0x38800000u) {                                 // normal half
+        const uint32_t r = ax + 0xfffu + ((ax >> 13) & 1u);
+        return (uint16_t)(sign | ((r >> 13) - 0x1c000u));
+    }
+    const uint32_t e = ax >> 23;                             // subnormal half
+    if (e < 102) return (uint16_t)sign;                      // < 2^-25
+    const uint32_t m = (ax & 0x7fffffu) | 0x800000u, s = 126 - e;
+    uint32_t q = m >> s;
+    const uint32_t rem = m & ((1u << s) - 1u), half = 1u << (s - 1);
+    if (rem > half || (rem == half && (q & 1u))) ++q;
+    return (uint16_t)(sign | q);
+}
+
+inline uint16_t f32_to_bf16_bits(uint32_t x) {
+    if ((x & 0x7fffffffu) > 0x7f800000u)
+        return (uint16_t)(((x >> 16) & 0x8000u) | 0x7fc0u);
+    return (uint16_t)((x + 0x7fffu + ((x >> 16) & 1u)) >> 16);
+}
+
+// Two float32 -> two values of OT (F16 / BF16) in one word, `lo` in the low
+// half: one cvt.rn.{f16,bf16}x2.f32 on the device.
+template <typename OT>
+BB_HD uint32_t pack_half2(float lo, float hi) {
+#if defined(__CUDA_ARCH__)
+    uint32_t r;
+    if (OT::kBrain)
+        asm("cvt.rn.bf16x2.f32 %0, %1, %2;" : "=r"(r) : "f"(hi), "f"(lo));
+    else
+        asm("cvt.rn.f16x2.f32 %0, %1, %2;" : "=r"(r) : "f"(hi), "f"(lo));
+    return r;
+#else
+    const uint32_t a = float_as_uint(lo), b = float_as_uint(hi);
+    if (OT::kBrain)
+        return f32_to_bf16_bits(a) | ((uint32_t)f32_to_bf16_bits(b) << 16);
+    return f32_to_f16_bits(a) | ((uint32_t)f32_to_f16_bits(b) << 16);
+#endif
+}
+
+// Stores of 4, 2 and 1 decoded values at an element pointer of the output
+// type: 16/8/4 bytes for float32, 8/4/2 for the 16-bit types.
+BB_HD void store4(float *p, const F4 &v) { *reinterpret_cast<F4 *>(p) = v; }
+BB_HD void store2(float *p, const F2 &v) { *reinterpret_cast<F2 *>(p) = v; }
+BB_HD void store1(float *p, float v) { *p = v; }
+template <typename OT>
+BB_HD void store4(OT *p, const F4 &v) {
+    *reinterpret_cast<H4 *>(p) = H4{pack_half2<OT>(v.x, v.y),
+                                    pack_half2<OT>(v.z, v.w)};
+}
+template <typename OT>
+BB_HD void store2(OT *p, const F2 &v) {
+    *reinterpret_cast<uint32_t *>(p) = pack_half2<OT>(v.x, v.y);
+}
+template <typename OT>
+BB_HD void store1(OT *p, float v) {
+    p->bits = (uint16_t)pack_half2<OT>(v, 0.f);
+}
+
+// The output of a geometry struct (`void *out`) as elements of OT.
+template <typename OT, typename Geom>
+BB_HD OT *out_as(const Geom &p) { return static_cast<OT *>(p.out); }
+
 BB_HD double add_rn(double a, double b) {
 #if defined(__CUDA_ARCH__)
     return __dadd_rn(a, b);

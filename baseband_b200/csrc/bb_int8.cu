@@ -5,20 +5,22 @@
 
 namespace bb {
 
+template <typename OT>
 __global__ void __launch_bounds__(kI8Threads) k_int8_decode_t(const I8Geom p) {
     __shared__ __align__(16) uint8_t tile[kI8SmemBytes];
     i8_dec_load(p, tile, blockIdx.x, threadIdx.x);
     __syncthreads();
-    i8_dec_store(p, tile, blockIdx.x, threadIdx.x);
+    i8_dec_store<OT>(p, tile, blockIdx.x, threadIdx.x);
 }
 
+template <typename OT>
 __global__ void __launch_bounds__(kF8Threads) k_int8_decode_t64(const I8Geom p) {
     __shared__ __align__(16) uint32_t tile[kF8SmemWords];
     // knock-outs (BB_TUNE_KNOCK_I8, tools/sweep_guppi.py): which half of the
     // kernel costs what
     if (!(p.knock & 1u)) f8_dec_load(p, tile, blockIdx.x, threadIdx.x);
     __syncthreads();
-    if (!(p.knock & 2u)) f8_dec_store(p, tile, blockIdx.x, threadIdx.x);
+    if (!(p.knock & 2u)) f8_dec_store<OT>(p, tile, blockIdx.x, threadIdx.x);
 }
 
 // Min-blocks hint of 4: lets ptxas keep eight float4 loads in flight (64
@@ -41,12 +43,13 @@ __global__ void __launch_bounds__(kI8Threads) k_int8_encode_t(const I8Geom p) {
 
 constexpr int kTFThreads = 256, kTFUnroll = 4;
 
+template <typename OT>
 __global__ void __launch_bounds__(kTFThreads) k_int8_decode_timefirst(
     const TFGeom p) {
     const uint32_t item0 = blockIdx.x * (kTFThreads * kTFUnroll) + threadIdx.x;
 #pragma unroll
     for (int u = 0; u < kTFUnroll; ++u)
-        tf_decode(p, blockIdx.y, item0 + u * kTFThreads);
+        tf_decode<OT>(p, blockIdx.y, item0 + u * kTFThreads);
 }
 
 template <typename T>
@@ -85,23 +88,51 @@ static int fill_geom(I8Geom &g, int64_t nunit, int64_t nrow, int64_t ncol,
     return BB_OK;
 }
 
+template <typename OT>
+static void launch_int8_decode_t(const I8Geom &g, uint64_t nblocks, bool fast,
+                                 cudaStream_t s) {
+    if (fast)
+        k_int8_decode_t64<OT><<<(unsigned)nblocks, kF8Threads, 0, s>>>(g);
+    else
+        k_int8_decode_t<OT><<<(unsigned)nblocks, kI8Threads, 0, s>>>(g);
+}
+
+template <typename OT>
+static void launch_int8_decode_tf(const TFGeom &g, dim3 grid, cudaStream_t s) {
+    k_int8_decode_timefirst<OT><<<grid, kTFThreads, 0, s>>>(g);
+}
+
+// Alignment the int8 decoders require of `out`: float32 keeps its 8 / 4
+// bytes; the 16-bit types need 8.  0: not a decoder output type.
+static int int8_out_align(int32_t out_dtype, int f32_align) {
+    const int esize = out_elem_nbytes(out_dtype);
+    return esize == 4 ? f32_align : esize == 2 ? 8 : 0;
+}
+
 }  // namespace bb
 
 using namespace bb;
 
-extern "C" int bb_decode_int8_transposed(
+extern "C" int bb_decode_int8_transposed_typed(
     const void *src, const int64_t *unit_offset, int64_t nunit, int64_t nrow,
     int64_t ncol, int32_t item_nbytes, const int64_t *col_begin,
-    const int64_t *col_end, const int64_t *out_col0, float *out,
-    void *stream) {
+    const int64_t *col_end, const int64_t *out_col0, int32_t out_dtype,
+    void *out, void *stream) {
     if (!src || !unit_offset || !col_begin || !col_end || !out_col0 || !out)
         return set_error(BB_ERR_ARGUMENT, "null pointer argument");
-    if (!aligned(out, 8))
-        return set_error(BB_ERR_ALIGNMENT, "out must be 8-byte aligned");
+    const int align = int8_out_align(out_dtype, 8);
+    if (align == 0)
+        return set_error(BB_ERR_ARGUMENT,
+                         "out_dtype must be BB_F32, BB_F16 or BB_BF16");
+    if (!aligned(out, align))
+        return set_error(BB_ERR_ALIGNMENT, "out must be %d-byte aligned",
+                         align);
     I8Geom g;
     uint64_t nblocks;
-    // Fast tile kernel: rows paired into 16-byte (complex) / 8-byte stores.
-    const bool fast = nrow % 2 == 0 && aligned(out, 16);
+    // Fast tile kernel: rows paired into float4-equivalent (complex) /
+    // float2-equivalent stores.
+    const bool fast = nrow % 2 == 0
+        && aligned(out, 4 * out_elem_nbytes(out_dtype));
     int rc = fill_geom(g, nunit, nrow, ncol, item_nbytes, nblocks, fast);
     if (rc != BB_OK) return rc;
     if (nblocks == 0) return BB_OK;
@@ -112,14 +143,22 @@ extern "C" int bb_decode_int8_transposed(
     g.out_col0 = (const long long *)out_col0;
     g.out = out;
     g.in = nullptr;
-    if (fast)
-        k_int8_decode_t64<<<(unsigned)nblocks, kF8Threads, 0,
-                            as_stream(stream)>>>(g);
-    else
-        k_int8_decode_t<<<(unsigned)nblocks, kI8Threads, 0,
-                          as_stream(stream)>>>(g);
+    cudaStream_t s = as_stream(stream);
+    if (out_dtype == BB_F16) launch_int8_decode_t<F16>(g, nblocks, fast, s);
+    else if (out_dtype == BB_BF16) launch_int8_decode_t<BF16>(g, nblocks, fast, s);
+    else launch_int8_decode_t<float>(g, nblocks, fast, s);
     BB_CHECK_LAUNCH("bb_decode_int8_transposed launch");
     return BB_OK;
+}
+
+extern "C" int bb_decode_int8_transposed(
+    const void *src, const int64_t *unit_offset, int64_t nunit, int64_t nrow,
+    int64_t ncol, int32_t item_nbytes, const int64_t *col_begin,
+    const int64_t *col_end, const int64_t *out_col0, float *out,
+    void *stream) {
+    return bb_decode_int8_transposed_typed(src, unit_offset, nunit, nrow, ncol,
+                                           item_nbytes, col_begin, col_end,
+                                           out_col0, BB_F32, out, stream);
 }
 
 extern "C" int bb_encode_int8_transposed(
@@ -154,18 +193,24 @@ extern "C" int bb_encode_int8_transposed(
     return BB_OK;
 }
 
-extern "C" int bb_decode_int8_timefirst(
+extern "C" int bb_decode_int8_timefirst_typed(
     const void *src, const int64_t *unit_offset, int64_t nunit,
     int64_t nsample, int32_t nchan, int32_t npol, int32_t item_nbytes,
     const int64_t *t_begin, const int64_t *t_end, const int64_t *out_t0,
-    float *out, void *stream) {
+    int32_t out_dtype, void *out, void *stream) {
     if (!src || !unit_offset || !t_begin || !t_end || !out_t0 || !out)
         return set_error(BB_ERR_ARGUMENT, "null pointer argument");
-    if (!aligned(out, 4))
-        return set_error(BB_ERR_ALIGNMENT, "out must be 4-byte aligned");
+    const int align = int8_out_align(out_dtype, 4);
+    if (align == 0)
+        return set_error(BB_ERR_ARGUMENT,
+                         "out_dtype must be BB_F32, BB_F16 or BB_BF16");
+    if (!aligned(out, align))
+        return set_error(BB_ERR_ALIGNMENT, "out must be %d-byte aligned",
+                         align);
     TFGeom g;
-    if (const char *msg = tf_fill_geom(g, nunit, nsample, nchan, npol,
-                                       item_nbytes, aligned(out, 16)))
+    if (const char *msg = tf_fill_geom(
+            g, nunit, nsample, nchan, npol, item_nbytes,
+            aligned(out, 4 * out_elem_nbytes(out_dtype))))
         return set_error(BB_ERR_ARGUMENT, "%s", msg);
     if (nunit == 0) return BB_OK;
     g.src = (const uint8_t *)src;
@@ -177,9 +222,22 @@ extern "C" int bb_decode_int8_timefirst(
     g.in = nullptr;
     const uint32_t per = kTFThreads * kTFUnroll;
     dim3 grid((g.items_per_unit + per - 1) / per, (unsigned)nunit);
-    k_int8_decode_timefirst<<<grid, kTFThreads, 0, as_stream(stream)>>>(g);
+    cudaStream_t s = as_stream(stream);
+    if (out_dtype == BB_F16) launch_int8_decode_tf<F16>(g, grid, s);
+    else if (out_dtype == BB_BF16) launch_int8_decode_tf<BF16>(g, grid, s);
+    else launch_int8_decode_tf<float>(g, grid, s);
     BB_CHECK_LAUNCH("bb_decode_int8_timefirst launch");
     return BB_OK;
+}
+
+extern "C" int bb_decode_int8_timefirst(
+    const void *src, const int64_t *unit_offset, int64_t nunit,
+    int64_t nsample, int32_t nchan, int32_t npol, int32_t item_nbytes,
+    const int64_t *t_begin, const int64_t *t_end, const int64_t *out_t0,
+    float *out, void *stream) {
+    return bb_decode_int8_timefirst_typed(src, unit_offset, nunit, nsample,
+                                          nchan, npol, item_nbytes, t_begin,
+                                          t_end, out_t0, BB_F32, out, stream);
 }
 
 extern "C" int bb_encode_int8_timefirst(

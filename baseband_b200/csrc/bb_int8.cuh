@@ -29,7 +29,7 @@ struct I8Geom {
     const uint8_t *src;              // decode: packed input; encode: output
     const long long *unit_offset;    // [nunit]
     const long long *col_begin, *col_end, *out_col0;   // decode only
-    float *out;
+    void *out;                       // float32, F16 or BF16 elements
     const void *in;                  // encode input (float or double)
     uint32_t nunit, nrow, ncol, ib;  // ib = item bytes (1 or 2)
     uint32_t tiles_r, tiles_c;       // tiles per unit
@@ -77,6 +77,7 @@ BB_HD void i8_dec_load(const I8Geom &p, uint8_t *smem, uint32_t block,
 }
 
 // Phase 2 of decode: shared tile -> transposed float output.
+template <typename OT = float>
 BB_HD void i8_dec_store(const I8Geom &p, const uint8_t *smem, uint32_t block,
                         uint32_t tid) {
     I8Tile t = i8_tile(p, block);
@@ -96,11 +97,10 @@ BB_HD void i8_dec_store(const I8Geom &p, const uint8_t *smem, uint32_t block,
         size_t o = (size_t)(oc0 + j - cb) * p.nrow + t.r0 + r;
         const int8_t *s = reinterpret_cast<const int8_t *>(
             smem + r * kI8Pitch + c * p.ib);
-        if (p.ib == 2) {
-            *reinterpret_cast<F2 *>(p.out + 2 * o) = F2{(float)s[0], (float)s[1]};
-        } else {
-            p.out[o] = (float)s[0];
-        }
+        if (p.ib == 2)
+            store2(out_as<OT>(p) + 2 * o, F2{(float)s[0], (float)s[1]});
+        else
+            store1(out_as<OT>(p) + o, (float)s[0]);
     }
 }
 
@@ -261,6 +261,7 @@ BB_HD float f8_byte(uint32_t w, int k) {
     return small_int_to_float((int32_t)(int8_t)(w >> (8 * k)));
 }
 
+template <typename OT = float>
 BB_HD void f8_dec_store(const I8Geom &p, const uint32_t *smem, uint32_t block,
                         uint32_t tid) {
     const F8Tile t = f8_tile(p, block);
@@ -284,9 +285,9 @@ BB_HD void f8_dec_store(const I8Geom &p, const uint32_t *smem, uint32_t block,
                 const long long jk = j + k;
                 if (jk < cb || jk >= lim) continue;
                 const size_t o = (size_t)(oc0 + jk - cb) * p.nrow + row;
-                *reinterpret_cast<F4 *>(p.out + 2 * o) = F4{
+                store4(out_as<OT>(p) + 2 * o, F4{
                     f8_byte(a, 2 * k), f8_byte(a, 2 * k + 1),
-                    f8_byte(b, 2 * k), f8_byte(b, 2 * k + 1)};
+                    f8_byte(b, 2 * k), f8_byte(b, 2 * k + 1)});
             }
         } else {
             const long long j = ((long long)t.w0 + wc) * 4;
@@ -295,8 +296,7 @@ BB_HD void f8_dec_store(const I8Geom &p, const uint32_t *smem, uint32_t block,
                 const long long jk = j + k;
                 if (jk < cb || jk >= lim) continue;
                 const size_t o = (size_t)(oc0 + jk - cb) * p.nrow + row;
-                *reinterpret_cast<F2 *>(p.out + o) = F2{f8_byte(a, k),
-                                                        f8_byte(b, k)};
+                store2(out_as<OT>(p) + o, F2{f8_byte(a, k), f8_byte(b, k)});
             }
         }
     }
@@ -444,7 +444,7 @@ struct TFGeom {
     const uint8_t *src;              // decode input / encode output
     const long long *unit_offset;    // [nunit]
     const long long *t_begin, *t_end, *out_t0;      // decode only
-    float *out;
+    void *out;                       // float32, F16 or BF16 elements
     const void *in;                  // encode input
     uint32_t nunit, nsample, nchan, npol, ib, vec;
     uint32_t sample_floats;          // npol * nchan * ib
@@ -510,7 +510,7 @@ BB_HD float tf_f(uint32_t b) {
     return small_int_to_float((int32_t)(int8_t)b);
 }
 
-template <int NPOL>
+template <int NPOL, typename OT>
 BB_HD void tf_decode_group(const TFGeom &p, uint32_t unit, uint32_t item,
                            long long off) {
     uint32_t t_rel, cg;
@@ -520,8 +520,8 @@ BB_HD void tf_decode_group(const TFGeom &p, uint32_t unit, uint32_t item,
     uint32_t w[NPOL];
     tf_load_group<NPOL>(p.src + off
                         + ((size_t)t * (p.row_floats / 4) + cg) * (4 * NPOL), w);
-    float *dst = p.out + ((size_t)(p.out_t0[unit] + t_rel) * p.sample_floats
-                          + 4 * cg);
+    OT *dst = out_as<OT>(p) + ((size_t)(p.out_t0[unit] + t_rel)
+                               * p.sample_floats + 4 * cg);
 #pragma unroll
     for (int pol = 0; pol < NPOL; ++pol) {
         F4 v;
@@ -534,18 +534,19 @@ BB_HD void tf_decode_group(const TFGeom &p, uint32_t unit, uint32_t item,
                    tf_f(tf_get_byte(w, 2 * NPOL + pol)),
                    tf_f(tf_get_byte(w, 3 * NPOL + pol))};
         }
-        *reinterpret_cast<F4 *>(dst + (size_t)pol * p.row_floats) = v;
+        store4(dst + (size_t)pol * p.row_floats, v);
     }
 }
 
+template <typename OT = float>
 BB_HD void tf_decode(const TFGeom &p, uint32_t unit, uint32_t item) {
     if (item >= p.items_per_unit) return;
     const long long off = p.unit_offset[unit];
     if (off < 0) return;
     if (p.vec == 4) {
-        if (p.npol == 2) tf_decode_group<2>(p, unit, item, off);
-        else if (p.npol == 4) tf_decode_group<4>(p, unit, item, off);
-        else tf_decode_group<1>(p, unit, item, off);
+        if (p.npol == 2) tf_decode_group<2, OT>(p, unit, item, off);
+        else if (p.npol == 4) tf_decode_group<4, OT>(p, unit, item, off);
+        else tf_decode_group<1, OT>(p, unit, item, off);
         return;
     }
     // one float per item: (sample, pol, chan, component)
@@ -556,8 +557,9 @@ BB_HD void tf_decode(const TFGeom &p, uint32_t unit, uint32_t item) {
     if (t >= p.t_end[unit] || t >= (long long)p.nsample) return;
     const uint32_t chan = p.ib == 2 ? f >> 1 : f, k = p.ib == 2 ? (f & 1u) : 0u;
     const int8_t *s = reinterpret_cast<const int8_t *>(p.src + off);
-    p.out[(size_t)(p.out_t0[unit] + t_rel) * p.sample_floats + r] =
-        (float)s[(((size_t)t * p.nchan + chan) * p.npol + pol) * p.ib + k];
+    store1(out_as<OT>(p) + (size_t)(p.out_t0[unit] + t_rel) * p.sample_floats
+           + r,
+           (float)s[(((size_t)t * p.nchan + chan) * p.npol + pol) * p.ib + k]);
 }
 
 template <typename T, int NPOL>

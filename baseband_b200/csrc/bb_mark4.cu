@@ -21,7 +21,7 @@ static inline unsigned m4_grid(uint32_t nitems, int unroll) {
     return (unsigned)((nitems + per - 1) / per);
 }
 
-template <int MODE>
+template <int MODE, typename OT>
 __global__ void __launch_bounds__(kM4Block) k_mark4_decode(const M4Geom p) {
     // pair LUT over the raw code (sign | magnitude << 1), see DecodeLut<2>
     __shared__ __align__(16) float lut[DecodeLut<2>::kFloats];
@@ -60,7 +60,7 @@ __global__ void __launch_bounds__(kM4Block) k_mark4_decode(const M4Geom p) {
                 if (item >= p.nitems) break;       // warp uniform
                 const unsigned okmask = __ballot_sync(0xffffffffu, ok[u]);
                 if (m4w_interior(p, item >> 5)) {
-                    float *chunk_out = m4w_chunk_out(p, item >> 5);
+                    OT *chunk_out = m4w_chunk_out<OT>(p, item >> 5);
                     const uint32_t r = m4_reorder32(w[u]);
 #pragma unroll
                     for (int j = 0; j < 4; ++j) {
@@ -75,7 +75,7 @@ __global__ void __launch_bounds__(kM4Block) k_mark4_decode(const M4Geom p) {
                     const uint32_t q = lane + 32u * j;
                     const uint32_t src = m4w_src_lane(p, lc, q);
                     const uint32_t ws = __shfl_sync(0xffffffffu, w[u], src);
-                    m4w_emit(p, lc, lv, item >> 5, q, ws, (okmask >> src) & 1u);
+                    m4w_emit<OT>(p, lc, lv, item >> 5, q, ws, (okmask >> src) & 1u);
                 }
             }
             return;
@@ -89,7 +89,7 @@ __global__ void __launch_bounds__(kM4Block) k_mark4_decode(const M4Geom p) {
             if (item >= p.nitems) break;           // warp uniform
             const unsigned okmask = __ballot_sync(0xffffffffu, ok[u]);
             if (m4w_interior(p, item >> 5)) {      // warp uniform
-                float *chunk_out = m4w_chunk_out(p, item >> 5);
+                OT *chunk_out = m4w_chunk_out<OT>(p, item >> 5);
 #pragma unroll
                 for (int j = 0; j < 4; ++j) {
                     const uint32_t ws = __shfl_sync(0xffffffffu, w[u], srcl[j]);
@@ -103,7 +103,7 @@ __global__ void __launch_bounds__(kM4Block) k_mark4_decode(const M4Geom p) {
                 const uint32_t q = lane + 32u * j;
                 const uint32_t src = m4w_src_lane(p, lc, q);
                 const uint32_t ws = __shfl_sync(0xffffffffu, w[u], src);
-                m4w_emit(p, lc, lv, item >> 5, q, ws, (okmask >> src) & 1u);
+                m4w_emit<OT>(p, lc, lv, item >> 5, q, ws, (okmask >> src) & 1u);
             }
         }
         return;
@@ -112,9 +112,9 @@ __global__ void __launch_bounds__(kM4Block) k_mark4_decode(const M4Geom p) {
     for (int u = 0; u < U; ++u) {
         const uint32_t item = item0 + u * kM4Block;
         if (item >= p.nitems) break;
-        if (MODE == M4_FAST) m4_dec_fast(p, lut, item);
-        else if (MODE == M4_GENERIC_VEC) m4_dec_generic<true>(p, item);
-        else m4_dec_generic<false>(p, item);
+        if (MODE == M4_FAST) m4_dec_fast<OT>(p, lut, item);
+        else if (MODE == M4_GENERIC_VEC) m4_dec_generic<true, OT>(p, item);
+        else m4_dec_generic<false, OT>(p, item);
     }
 }
 
@@ -149,20 +149,21 @@ k_mark4_encode_half(const M4Geom p, const QuantConsts<T> c) {
     }
 }
 
+template <typename OT>
 static int run_decode(const std::vector<M4Launch> &launches, cudaStream_t s) {
     for (const M4Launch &l : launches) {
         const uint32_t n = l.g.nitems;
         if (l.mode == M4_FAST)
-            k_mark4_decode<M4_FAST>
+            k_mark4_decode<M4_FAST, OT>
                 <<<m4_grid(n, kM4UnrollFast), kM4Block, 0, s>>>(l.g);
         else if (l.mode == M4_WARP)
-            k_mark4_decode<M4_WARP>
+            k_mark4_decode<M4_WARP, OT>
                 <<<m4_grid(n, kM4UnrollWarp), kM4Block, 0, s>>>(l.g);
         else if (l.mode == M4_GENERIC_VEC)
-            k_mark4_decode<M4_GENERIC_VEC>
+            k_mark4_decode<M4_GENERIC_VEC, OT>
                 <<<m4_grid(n, kM4UnrollVec), kM4Block, 0, s>>>(l.g);
         else
-            k_mark4_decode<M4_GENERIC_SCALAR>
+            k_mark4_decode<M4_GENERIC_SCALAR, OT>
                 <<<m4_grid(n, kM4UnrollScalar), kM4Block, 0, s>>>(l.g);
         BB_CHECK_LAUNCH("bb_mark4_decode launch");
     }
@@ -195,15 +196,21 @@ static int run_encode(const std::vector<M4Launch> &launches, cudaStream_t s) {
 
 using namespace bb;
 
-extern "C" int bb_mark4_decode(
+extern "C" int bb_mark4_decode_typed(
     const void *src, const int64_t *unit_offset, int64_t nframe, int32_t nchan,
     int32_t fanout, int32_t ft, const float *levels_host, float fill_value,
-    int64_t sample_start, int64_t nsample, float *out, void *stream) {
+    int64_t sample_start, int64_t nsample, int32_t out_dtype, void *out,
+    void *stream) {
     if (!src || !unit_offset || !out || !levels_host)
         return set_error(BB_ERR_ARGUMENT, "null pointer argument");
-    if (!aligned(out, 16) || !aligned(src, 8))
+    const int esize = out_elem_nbytes(out_dtype);
+    if (esize == 0)
+        return set_error(BB_ERR_ARGUMENT,
+                         "out_dtype must be BB_F32, BB_F16 or BB_BF16");
+    if (!aligned(out, 4 * esize) || !aligned(src, 8))
         return set_error(BB_ERR_ALIGNMENT,
-                         "out must be 16-byte and src 8-byte aligned");
+                         "out must be %d-byte and src 8-byte aligned",
+                         4 * esize);
     std::vector<M4Launch> launches;
     std::string err;
     if (!plan_m4_frames(false, src, unit_offset, nframe, nchan, fanout, ft,
@@ -212,7 +219,19 @@ extern "C" int bb_mark4_decode(
         return set_error(err.rfind("no Mark 4 codec", 0) == 0
                          ? BB_ERR_UNSUPPORTED : BB_ERR_ARGUMENT, "%s",
                          err.c_str());
-    return run_decode(launches, as_stream(stream));
+    cudaStream_t s = as_stream(stream);
+    if (out_dtype == BB_F16) return run_decode<F16>(launches, s);
+    if (out_dtype == BB_BF16) return run_decode<BF16>(launches, s);
+    return run_decode<float>(launches, s);
+}
+
+extern "C" int bb_mark4_decode(
+    const void *src, const int64_t *unit_offset, int64_t nframe, int32_t nchan,
+    int32_t fanout, int32_t ft, const float *levels_host, float fill_value,
+    int64_t sample_start, int64_t nsample, float *out, void *stream) {
+    return bb_mark4_decode_typed(src, unit_offset, nframe, nchan, fanout, ft,
+                                 levels_host, fill_value, sample_start,
+                                 nsample, BB_F32, out, stream);
 }
 
 extern "C" int bb_mark4_encode(
@@ -251,7 +270,7 @@ extern "C" int bb_mark4_decode_words(
         return set_error(err.rfind("no Mark 4 codec", 0) == 0
                          ? BB_ERR_UNSUPPORTED : BB_ERR_ARGUMENT, "%s",
                          err.c_str());
-    return run_decode(launches, as_stream(stream));
+    return run_decode<float>(launches, as_stream(stream));
 }
 
 extern "C" int bb_mark4_encode_words(

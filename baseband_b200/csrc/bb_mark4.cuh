@@ -25,7 +25,8 @@ namespace bb {
 struct M4Geom {
     const uint8_t *src;              // decode input / encode output base
     const long long *unit_offset;    // per frame payload offset; null => 0
-    float *out;                      // decode output (row 0 of the call)
+    void *out;                       // decode output (row 0 of the call;
+                                     // float32, F16 or BF16 elements)
     const void *in;                  // encode input
     unsigned long long in_elem_offset;
     long long row_base, nsample;
@@ -57,6 +58,7 @@ BB_HD F2 m4_pair(uint32_t byte_, uint32_t fp, const float *lut) {
 }
 
 // FAST decode.  item = (frame, step, half).
+template <typename OT = float>
 BB_HD void m4_dec_fast(const M4Geom &p, const float *lut, uint32_t item) {
     const uint32_t nhalf = p.wordbytes >> 2;           // 1 or 2
     const uint32_t h = item & (nhalf - 1u);
@@ -68,7 +70,7 @@ BB_HD void m4_dec_fast(const M4Geom &p, const float *lut, uint32_t item) {
     if (row0 + 4 <= 0 || row0 >= p.nsample) return;
     const long long off = p.unit_offset ? p.unit_offset[frame] : 0;
     const bool data = off >= 0 && step >= p.header_steps;
-    float *dst = p.out + row0 * (long long)p.nchan + 4 * h;
+    OT *dst = out_as<OT>(p) + row0 * (long long)p.nchan + 4 * h;
     F4 rows[4];
     if (data) {
         uint32_t w = *reinterpret_cast<const uint32_t *>(
@@ -91,12 +93,12 @@ BB_HD void m4_dec_fast(const M4Geom &p, const float *lut, uint32_t item) {
     if (row0 >= 0 && row0 + 4 <= p.nsample) {
 #pragma unroll
         for (int i = 0; i < 4; ++i)
-            *reinterpret_cast<F4 *>(dst + (size_t)i * p.nchan) = rows[i];
+            store4(dst + (size_t)i * p.nchan, rows[i]);
     } else {
 #pragma unroll
         for (int i = 0; i < 4; ++i)
             if (row0 + i >= 0 && row0 + i < p.nsample)
-                *reinterpret_cast<F4 *>(dst + (long long)i * p.nchan) = rows[i];
+                store4(dst + (long long)i * p.nchan, rows[i]);
     }
 }
 
@@ -128,7 +130,7 @@ BB_HD float m4_dec_element(const M4Geom &p, uint32_t row_local, uint32_t c) {
     return m4_value(p, w, f, c);
 }
 
-template <bool VEC>
+template <bool VEC, typename OT = float>
 BB_HD void m4_dec_generic(const M4Geom &p, uint32_t item) {
     const uint32_t n = VEC ? item * 4u : item;
     long long gidx = p.row_base * (long long)p.nchan + n;
@@ -140,9 +142,10 @@ BB_HD void m4_dec_generic(const M4Geom &p, uint32_t item) {
             uint32_t e = n + i;
             v[i] = m4_dec_element(p, e >> p.log2_nchan, e & (p.nchan - 1u));
         }
-        *reinterpret_cast<F4 *>(p.out + gidx) = F4{v[0], v[1], v[2], v[3]};
+        store4(out_as<OT>(p) + gidx, F4{v[0], v[1], v[2], v[3]});
     } else {
-        p.out[gidx] = m4_dec_element(p, n >> p.log2_nchan, n & (p.nchan - 1u));
+        store1(out_as<OT>(p) + gidx,
+               m4_dec_element(p, n >> p.log2_nchan, n & (p.nchan - 1u)));
     }
 }
 
@@ -200,6 +203,7 @@ BB_HD uint32_t m4w_src_lane(const M4Geom &p, const M4Lane &c, uint32_t q) {
     return ((n << p.log2_wordbytes) >> 2) + c.half;
 }
 
+template <typename OT = float>
 BB_HD void m4w_emit(const M4Geom &p, const M4Lane &c, const float lv[4],
                     uint32_t chunk, uint32_t q, uint32_t w, bool valid) {
     if (chunk * 32u + m4w_src_lane(p, c, q) >= p.total32) return;
@@ -218,7 +222,7 @@ BB_HD void m4w_emit(const M4Geom &p, const M4Lane &c, const float lv[4],
     } else {
         v = F4{p.fill, p.fill, p.fill, p.fill};
     }
-    *reinterpret_cast<F4 *>(p.out + gidx) = v;
+    store4(out_as<OT>(p) + gidx, v);
 }
 
 // Interior chunks (all 32 values inside the launch, all 128 float4 inside the
@@ -232,8 +236,9 @@ BB_HD bool m4w_interior(const M4Geom &p, uint32_t chunk) {
     return g0 >= 0 && g0 + 512 <= p.nsample * (long long)p.nchan;
 }
 
-BB_HD float *m4w_chunk_out(const M4Geom &p, uint32_t chunk) {
-    return p.out + (p.row_base * (long long)p.nchan + (long long)chunk * 512);
+template <typename OT = float>
+BB_HD OT *m4w_chunk_out(const M4Geom &p, uint32_t chunk) {
+    return out_as<OT>(p) + (p.row_base * (long long)p.nchan + (long long)chunk * 512);
 }
 
 BB_HD uint32_t m4w_pair_index(const M4Lane &c, uint32_t w, int k) {
@@ -242,8 +247,9 @@ BB_HD uint32_t m4w_pair_index(const M4Lane &c, uint32_t w, int k) {
         | (((w >> c.mbit[k + 1]) & 1u) << 3);
 }
 
+template <typename OT>
 BB_HD void m4w_emit_fast(const M4Geom &p, const M4Lane &c, const float *lut,
-                         float *chunk_out, uint32_t q, uint32_t w, bool valid) {
+                         OT *chunk_out, uint32_t q, uint32_t w, bool valid) {
     F4 v;
     if (valid) {
         const F2 a = reinterpret_cast<const F2 *>(lut)[m4w_pair_index(c, w, 0)];
@@ -252,7 +258,7 @@ BB_HD void m4w_emit_fast(const M4Geom &p, const M4Lane &c, const float *lut,
     } else {
         v = F4{p.fill, p.fill, p.fill, p.fill};
     }
-    *reinterpret_cast<F4 *>(chunk_out + 4u * q) = v;
+    store4(chunk_out + 4u * q, v);
 }
 
 // WARP decode specialised for the standard fan-out 4 layouts (32 and 64
@@ -282,10 +288,11 @@ BB_HD F4 m4s_decode(uint32_t r, uint32_t i, const float *lut) {
     return F4{a.x, a.y, b.x, b.y};
 }
 
-BB_HD void m4s_emit_fast(const M4Geom &p, const float *lut, float *chunk_out,
+template <typename OT>
+BB_HD void m4s_emit_fast(const M4Geom &p, const float *lut, OT *chunk_out,
                          uint32_t q, uint32_t i, uint32_t r, bool valid) {
-    *reinterpret_cast<F4 *>(chunk_out + 4u * q) = valid
-        ? m4s_decode(r, i, lut) : F4{p.fill, p.fill, p.fill, p.fill};
+    store4(chunk_out + 4u * q, valid
+           ? m4s_decode(r, i, lut) : F4{p.fill, p.fill, p.fill, p.fill});
 }
 
 // ------------------------------------------------------------------ encode

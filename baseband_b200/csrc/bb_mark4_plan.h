@@ -146,7 +146,7 @@ inline bool plan_m4_frames(bool encode, const void *src_or_dst,
                            const int64_t *unit_offset, int64_t nframe,
                            int nchan, int fanout, int ft, const float *levels,
                            float fill, int64_t sample_start, int64_t nsample,
-                           float *out, const void *in,
+                           void *out, const void *in,
                            std::vector<M4Launch> &launches, std::string &err) {
     M4Geom base;
     if (!m4_base_geom(nchan, fanout, ft, levels, base, err)) return false;

@@ -30,6 +30,13 @@ inline bool aligned(const void *p, uintptr_t a) {
     return (reinterpret_cast<uintptr_t>(p) & (a - 1)) == 0;
 }
 
+// Bytes per element of a decoder output type (bb_dtype), 0 if a decoder
+// cannot write it.
+inline int out_elem_nbytes(int32_t out_dtype) {
+    return out_dtype == BB_F32 ? 4
+        : (out_dtype == BB_F16 || out_dtype == BB_BF16) ? 2 : 0;
+}
+
 #define BB_CHECK_LAUNCH(what)                                            \
     do {                                                                 \
         cudaError_t e__ = cudaGetLastError();                            \

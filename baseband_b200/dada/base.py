@@ -68,7 +68,7 @@ class DADAStreamReader(_DADAStreamBase, StreamReaderBase):
     """DADA stream reader (GPU decode)."""
 
     def __init__(self, fh_raw, squeeze=True, subset=(), verify=True,
-                 device=None, chunk_nbytes=None):
+                 device=None, chunk_nbytes=None, dtype=None):
         fh_raw = DADAFileReader(fh_raw)
         header0 = fh_raw.read_header()
         size = fh_raw.seek(0, 2)
@@ -91,7 +91,7 @@ class DADAStreamReader(_DADAStreamBase, StreamReaderBase):
         self._mkbf = header0.get('INSTRUMENT') == 'MKBF'
         super().__init__(fh_raw, header0, squeeze=squeeze, subset=subset,
                          verify=verify, samples_per_frame=spf, device=device,
-                         chunk_nbytes=chunk_nbytes)
+                         chunk_nbytes=chunk_nbytes, dtype=dtype)
         self._sample_nbytes = header0._bits_per_sample // 8
         self._last_nsample = self._last_nbytes // self._sample_nbytes
 

@@ -131,7 +131,7 @@ class GSBStreamReader(_GSBStreamBase, StreamReaderBase):
     def __init__(self, fh_ts, fh_raw, sample_rate=None,
                  samples_per_frame=None, payload_nbytes=None, nchan=None,
                  bps=None, complex_data=None, squeeze=True, subset=(),
-                 verify=True, device=None, chunk_nbytes=None):
+                 verify=True, device=None, chunk_nbytes=None, dtype=None):
         self.fh_ts = GSBTimeStampIO(fh_ts)
         header0 = self.fh_ts.read_timestamp()
         g = _geometry(header0, fh_raw, sample_rate, samples_per_frame,
@@ -143,7 +143,8 @@ class GSBStreamReader(_GSBStreamBase, StreamReaderBase):
             samples_per_frame=g['samples_per_frame'],
             sample_shape=g['sample_shape'], bps=g['bps'],
             complex_data=g['complex_data'], squeeze=squeeze, subset=subset,
-            verify=verify, device=device, chunk_nbytes=chunk_nbytes)
+            verify=verify, device=device, chunk_nbytes=chunk_nbytes,
+            dtype=dtype)
         # frames = complete timestamp lines that also have payload bytes
         self.fh_ts.seek(0)
         text = self.fh_ts.read()
@@ -232,6 +233,10 @@ class GSBStreamWriter(_GSBStreamBase, StreamWriterBase):
                  samples_per_frame=None, payload_nbytes=None, nchan=None,
                  bps=None, complex_data=None, squeeze=True, device=None,
                  **kwargs):
+        if 'dtype' in kwargs:
+            # as for the other formats' writers: `dtype` is a reader option
+            raise TypeError("GSBStreamWriter got an unexpected keyword "
+                            "argument 'dtype'")
         self.fh_ts = GSBTimeStampIO(fh_ts)
         if header0 is None:
             header0 = GSBHeader.fromvalues(**kwargs)

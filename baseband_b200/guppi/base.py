@@ -76,7 +76,7 @@ class GUPPIStreamReader(_GUPPIStreamBase, StreamReaderBase):
     overlap."""
 
     def __init__(self, fh_raw, squeeze=True, subset=(), verify=True,
-                 device=None, chunk_nbytes=None):
+                 device=None, chunk_nbytes=None, dtype=None):
         fh_raw = GUPPIFileReader(fh_raw)
         header0 = fh_raw.read_header()
         self._full_spf = header0.samples_per_frame
@@ -88,7 +88,7 @@ class GUPPIStreamReader(_GUPPIStreamBase, StreamReaderBase):
         super().__init__(
             fh_raw, header0, squeeze=squeeze, subset=subset, verify=verify,
             samples_per_frame=self._full_spf - self._overlap,
-            device=device, chunk_nbytes=chunk_nbytes)
+            device=device, chunk_nbytes=chunk_nbytes, dtype=dtype)
 
     @property
     def _nsample(self):

@@ -12,7 +12,7 @@ import torch
 
 from . import _lib
 from ._lib import (CODEC_LEVELS, CODEC_SINT, QUANT_OFFSET_BINARY,  # noqa
-                   QUANT_MARK5B, QUANT_SINT, F32, F64)
+                   QUANT_MARK5B, QUANT_SINT, F32, F64, F16, BF16)
 
 _FLOATP = ctypes.POINTER(ctypes.c_float)
 
@@ -83,6 +83,29 @@ def _float_code(data):
         data.dtype))
 
 
+# Element types the decoders can write (bb_dtype codes).
+OUT_DTYPES = {torch.float32: F32, torch.float16: F16, torch.bfloat16: BF16}
+
+
+def _typed(lib, name, out):
+    """The decode entry point for ``out``'s element type and the arguments
+    that select it: ``(fn, extra)``, where float32 uses the plain function
+    (no extra argument) and float16 / bfloat16 its ``_typed`` variant, which
+    takes the bb_dtype code before ``out``."""
+    if out.dtype == torch.float32:
+        return getattr(lib, name), ()
+    code = OUT_DTYPES.get(out.dtype)
+    if code is None:
+        raise TypeError('out must be float32, float16 or bfloat16, not {}'
+                        .format(out.dtype))
+    try:
+        fn = getattr(lib, name + '_typed')
+    except AttributeError:
+        raise ImportError('libbaseband_b200.so has no {}_typed: rebuild it '
+                          'for float16 / bfloat16 output'.format(name))
+    return fn, (code,)
+
+
 def _levels_arg(levels):
     if levels is None:
         return None, None
@@ -106,28 +129,30 @@ def to_device_bytes(raw, device, pinned=None):
 def decode_bitfield(src, unit_offset, nset, nthread, payload_nbytes, bps,
                     nelem, complex_data=False, codec=CODEC_LEVELS,
                     levels=None, fill_value=0.0, sample_start=0,
-                    nsample=None, out=None):
-    """bb_decode_bitfield -> float32 tensor (nsample, nthread, nelem)."""
+                    nsample=None, out=None, dtype=torch.float32):
+    """bb_decode_bitfield -> tensor (nsample, nthread, nelem) of ``dtype``
+    (float32, float16 or bfloat16) or of ``out``'s dtype."""
     lib = _lib.load()
     _require_cuda(src, unit_offset, out)
     spf = payload_nbytes * 8 // (bps * nelem)
     if nsample is None:
         nsample = nset * spf - sample_start
     if out is None:
-        out = torch.empty((nsample, nthread, nelem), dtype=torch.float32,
+        out = torch.empty((nsample, nthread, nelem), dtype=dtype,
                           device=src.device)
     elif out.numel() != nsample * nthread * nelem:
         raise ValueError('out has the wrong number of elements')
     if out.numel() == 0:
         return out                       # an empty tensor has no storage
+    fn, typed = _typed(lib, 'bb_decode_bitfield', out)
     keep, lv = _levels_arg(levels)
     with _on(src.device):
-        rc = lib.bb_decode_bitfield(
+        rc = fn(
             _dev(src, 'src', torch.uint8), _dev(unit_offset, 'unit_offset',
                                                 torch.int64),
             nset, nthread, payload_nbytes, bps, nelem, int(bool(complex_data)),
-            codec, lv, float(fill_value), sample_start, nsample,
-            _dev(out, 'out', torch.float32), _stream_ptr(src.device))
+            codec, lv, float(fill_value), sample_start, nsample, *typed,
+            _dev(out, 'out'), _stream_ptr(src.device))
     _lib.check(rc, lib)
     _count()
     return out
@@ -155,24 +180,25 @@ def encode_bitfield(data, dst, unit_offset, nset, nthread, payload_nbytes,
 
 def mark4_decode(src, unit_offset, nframe, nchan, fanout, ft=False,
                  levels=None, fill_value=0.0, sample_start=0, nsample=None,
-                 out=None):
+                 out=None, dtype=torch.float32):
+    """bb_mark4_decode -> tensor (nsample, nchan) of ``dtype`` (float32,
+    float16 or bfloat16) or of ``out``'s dtype."""
     lib = _lib.load()
     spf = 20000 * fanout
     if nsample is None:
         nsample = nframe * spf - sample_start
     if out is None:
-        out = torch.empty((nsample, nchan), dtype=torch.float32,
-                          device=src.device)
+        out = torch.empty((nsample, nchan), dtype=dtype, device=src.device)
     if out.numel() == 0:
         return out
+    fn, typed = _typed(lib, 'bb_mark4_decode', out)
     keep, lv = _levels_arg(levels)
     with _on(src.device):
-        rc = lib.bb_mark4_decode(
+        rc = fn(
             _dev(src, 'src', torch.uint8),
             _dev(unit_offset, 'unit_offset', torch.int64), nframe, nchan,
             fanout, int(bool(ft)), lv, float(fill_value), sample_start,
-            nsample, _dev(out, 'out', torch.float32),
-            _stream_ptr(src.device))
+            nsample, *typed, _dev(out, 'out'), _stream_ptr(src.device))
     _lib.check(rc, lib)
     _count()
     return out
@@ -225,17 +251,20 @@ def mark4_encode_words(data, words, nword, nchan, fanout, ft=False):
 
 def decode_int8_transposed(src, unit_offset, nunit, nrow, ncol, item_nbytes,
                            col_begin, col_end, out_col0, out):
+    """bb_decode_int8_transposed into ``out`` (float32, float16 or
+    bfloat16)."""
     lib = _lib.load()
     if out.numel() == 0:
         return out
+    fn, typed = _typed(lib, 'bb_decode_int8_transposed', out)
     with _on(src.device):
-        rc = lib.bb_decode_int8_transposed(
+        rc = fn(
             _dev(src, 'src', torch.uint8),
             _dev(unit_offset, 'unit_offset', torch.int64), nunit, nrow, ncol,
             item_nbytes, _dev(col_begin, 'col_begin', torch.int64),
             _dev(col_end, 'col_end', torch.int64),
-            _dev(out_col0, 'out_col0', torch.int64),
-            _dev(out, 'out', torch.float32), _stream_ptr(src.device))
+            _dev(out_col0, 'out_col0', torch.int64), *typed,
+            _dev(out, 'out'), _stream_ptr(src.device))
     _lib.check(rc, lib)
     _count()
     return out
@@ -260,18 +289,19 @@ def encode_int8_transposed(data, dst, unit_offset, nunit, nrow, ncol,
 def decode_int8_timefirst(src, unit_offset, nunit, nsample, nchan, npol,
                           item_nbytes, t_begin, t_end, out_t0, out):
     """bb_decode_int8_timefirst: [time][chan][pol] int8 -> (time, pol, chan)
-    float32 rows of ``out``."""
+    rows of ``out`` (float32, float16 or bfloat16)."""
     lib = _lib.load()
     if out.numel() == 0:
         return out
+    fn, typed = _typed(lib, 'bb_decode_int8_timefirst', out)
     with _on(src.device):
-        rc = lib.bb_decode_int8_timefirst(
+        rc = fn(
             _dev(src, 'src', torch.uint8),
             _dev(unit_offset, 'unit_offset', torch.int64), nunit, nsample,
             nchan, npol, item_nbytes, _dev(t_begin, 't_begin', torch.int64),
             _dev(t_end, 't_end', torch.int64),
-            _dev(out_t0, 'out_t0', torch.int64),
-            _dev(out, 'out', torch.float32), _stream_ptr(src.device))
+            _dev(out_t0, 'out_t0', torch.int64), *typed,
+            _dev(out, 'out'), _stream_ptr(src.device))
     _lib.check(rc, lib)
     _count()
     return out

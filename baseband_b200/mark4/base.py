@@ -131,7 +131,7 @@ class Mark4StreamReader(StreamReaderBase):
 
     def __init__(self, fh_raw, sample_rate=None, ntrack=None, decade=None,
                  ref_time=None, squeeze=True, subset=(), fill_value=0.,
-                 verify=True, device=None, chunk_nbytes=None):
+                 verify=True, device=None, chunk_nbytes=None, dtype=None):
         if decade is None and ref_time is None:
             raise TypeError('Mark 4 stream reader requires either decade or '
                             'ref_time to be passed in.')
@@ -155,7 +155,7 @@ class Mark4StreamReader(StreamReaderBase):
         super().__init__(
             fh_raw, header0, sample_rate=sample_rate, squeeze=squeeze,
             subset=subset, fill_value=fill_value, verify=verify,
-            device=device, chunk_nbytes=chunk_nbytes)
+            device=device, chunk_nbytes=chunk_nbytes, dtype=dtype)
         coder = Mark4Payload(np.zeros(
             header0.payload_nbytes // header0.stream_dtype.itemsize,
             header0.stream_dtype), header0)._coder

@@ -120,7 +120,7 @@ class Mark5BStreamReader(_Mark5BStreamBase, StreamReaderBase):
 
     def __init__(self, fh_raw, sample_rate=None, kday=None, ref_time=None,
                  nchan=None, bps=2, squeeze=True, subset=(), fill_value=0.,
-                 verify=True, device=None, chunk_nbytes=None):
+                 verify=True, device=None, chunk_nbytes=None, dtype=None):
         if nchan is None:
             raise TypeError('Mark 5B stream reader requires nchan to be '
                             'passed in explicitly.')
@@ -146,7 +146,8 @@ class Mark5BStreamReader(_Mark5BStreamBase, StreamReaderBase):
             fh_raw, header0, sample_rate=sample_rate, samples_per_frame=spf,
             sample_shape=(nchan,), bps=bps, complex_data=False,
             squeeze=squeeze, subset=subset, fill_value=fill_value,
-            verify=verify, device=device, chunk_nbytes=chunk_nbytes)
+            verify=verify, device=device, chunk_nbytes=chunk_nbytes,
+            dtype=dtype)
         self._levels = levels.mark5b(bps)
         self._checks = []
         if self.verify and self._nframe > 1:

@@ -96,8 +96,12 @@ def read_sharded(fh, rank=None, world=None, gather=False, group=None):
         raise TypeError('gather=True over NCCL needs a reader with device '
                         'output (open(..., device=...)): NCCL moves device '
                         'tensors only.')
-    t_dtype = torch.complex64 if fh.complex_data else torch.float32
-    shape = (world * block,) + tuple(fh.sample_shape)
+    # the reader's result type: float16 / bfloat16 readers gather half the
+    # bytes of float32 ones
+    dec = fh._dec_dtype
+    t_dtype = fh._result_dtype(dec)
+    reduced = dec != torch.float32
+    shape = (world * block,) + tuple(fh.sample_shape) + fh._pair_axis(dec)
     if on_device:
         whole = torch.empty(shape, dtype=t_dtype, device=fh.device)
     else:
@@ -105,7 +109,7 @@ def read_sharded(fh, rank=None, world=None, gather=False, group=None):
     mine = whole[rank * block:(rank + 1) * block]
     if stop > start:
         fh.seek(start)
-        fh.read(out=mine[:stop - start] if on_device
+        fh.read(out=mine[:stop - start] if on_device or reduced
                 else mine[:stop - start].numpy())
     # rows past the end of the stream (short last blocks) are never looked at
     if on_device or backend != 'gloo':
@@ -116,7 +120,7 @@ def read_sharded(fh, rank=None, world=None, gather=False, group=None):
         dist.all_gather([whole[r * block:(r + 1) * block]
                          for r in range(world)], mine.clone(), group=group)
     whole = whole[:total]
-    if not on_device:
+    if not on_device and not reduced:
         whole = whole.numpy()
     return whole, (0, total)
 

@@ -167,7 +167,7 @@ class VDIFStreamReader(_VDIFStreamBase, StreamReaderBase):
     """
     def __init__(self, fh_raw, sample_rate=None, squeeze=True, subset=(),
                  fill_value=0., verify='fix', device=None,
-                 chunk_nbytes=None):
+                 chunk_nbytes=None, dtype=None):
         fh_raw = VDIFFileReader(fh_raw)
         header0 = fh_raw.read_header()
         fh_raw.seek(0)
@@ -187,7 +187,7 @@ class VDIFStreamReader(_VDIFStreamBase, StreamReaderBase):
             fh_raw, header0, sample_rate=sample_rate,
             sample_shape=(nthread, header0.nchan), squeeze=squeeze,
             subset=subset, fill_value=fill_value, verify=verify,
-            device=device, chunk_nbytes=chunk_nbytes)
+            device=device, chunk_nbytes=chunk_nbytes, dtype=dtype)
         # Split the subset into thread selection (done by the scan kernel's
         # slot table, so unwanted threads are never decoded) and the rest,
         # applied after decoding (vdif/base.py:464-490).
@@ -268,8 +268,8 @@ class VDIFStreamReader(_VDIFStreamBase, StreamReaderBase):
         nthread, nchan = len(self._decode_ids), self._sample_shape[1]
         n = nsample * self._floats_per_sample
         if self._complex_data:
-            data = torch.view_as_complex(flat[:n].view(nsample, nthread,
-                                                       nchan, 2))
+            data = self._complex_view(flat[:n].view(nsample, nthread,
+                                                    nchan, 2))
         else:
             data = flat[:n].view(nsample, nthread, nchan)
         if self._thread_expand is not None:

@@ -66,7 +66,13 @@ typedef enum bb_quantiser {
                                    (gsb/payload.py:45-53, guppi/payload.py:17) */
 } bb_quantiser;
 
-typedef enum bb_dtype { BB_F32 = 0, BB_F64 = 1 } bb_dtype;
+/* Element types.  Encoders take BB_F32 / BB_F64 input; decoders write BB_F32
+ * or, through the `_typed` entry points, BB_F16 (IEEE half) / BB_BF16
+ * (bfloat16).  A 16-bit result is the float32 result rounded elementwise to
+ * nearest even (overflow to +-inf), as torch's `.to(dtype)` converts it. */
+typedef enum bb_dtype {
+    BB_F32 = 0, BB_F64 = 1, BB_F16 = 2, BB_BF16 = 3
+} bb_dtype;
 
 /* ---------------------------------------------------------------- runtime */
 int bb_abi_version(void);
@@ -116,6 +122,18 @@ int bb_decode_bitfield(const void *src, const int64_t *unit_offset,
                        int32_t codec, const float *levels_host,
                        float fill_value, int64_t sample_start,
                        int64_t nsample, float *out, void *stream);
+/* The same with the output element type chosen by `out_dtype`: BB_F32 (the
+ * call above, out 16-byte aligned), BB_F16 or BB_BF16 (out 8-byte aligned;
+ * each value is the float32 result rounded to nearest even).  The work
+ * decomposition is the same for every output type. */
+int bb_decode_bitfield_typed(const void *src, const int64_t *unit_offset,
+                             int64_t nset, int32_t nthread,
+                             int64_t payload_nbytes, int32_t bps,
+                             int32_t nelem, int32_t complex_data,
+                             int32_t codec, const float *levels_host,
+                             float fill_value, int64_t sample_start,
+                             int64_t nsample, int32_t out_dtype, void *out,
+                             void *stream);
 
 /* Inverse: quantise + pack `in` (same logical layout as `out` above, float32
  * or float64 — arithmetic is done in the input width exactly as numpy does,
@@ -148,6 +166,14 @@ int bb_mark4_decode(const void *src, const int64_t *unit_offset,
                     const float *levels_host, float fill_value,
                     int64_t sample_start, int64_t nsample, float *out,
                     void *stream);
+/* Typed output as bb_decode_bitfield_typed (BB_F16 / BB_BF16: out 8-byte
+ * aligned). */
+int bb_mark4_decode_typed(const void *src, const int64_t *unit_offset,
+                          int64_t nframe, int32_t nchan, int32_t fanout,
+                          int32_t ft, const float *levels_host,
+                          float fill_value, int64_t sample_start,
+                          int64_t nsample, int32_t out_dtype, void *out,
+                          void *stream);
 /* Inverse for whole frames; rows falling in the header region are ignored. */
 int bb_mark4_encode(const void *in, int32_t in_dtype, void *dst,
                     const int64_t *unit_offset, int64_t nframe, int32_t nchan,
@@ -179,6 +205,16 @@ int bb_decode_int8_transposed(const void *src, const int64_t *unit_offset,
                               int32_t item_nbytes, const int64_t *col_begin,
                               const int64_t *col_end, const int64_t *out_col0,
                               float *out, void *stream);
+/* Typed output (out 8-byte aligned for every type). */
+int bb_decode_int8_transposed_typed(const void *src,
+                                    const int64_t *unit_offset, int64_t nunit,
+                                    int64_t nrow, int64_t ncol,
+                                    int32_t item_nbytes,
+                                    const int64_t *col_begin,
+                                    const int64_t *col_end,
+                                    const int64_t *out_col0,
+                                    int32_t out_dtype, void *out,
+                                    void *stream);
 int bb_encode_int8_transposed(const void *in, int32_t in_dtype, void *dst,
                               const int64_t *unit_offset, int64_t nunit,
                               int64_t nrow, int64_t ncol, int32_t item_nbytes,
@@ -196,6 +232,15 @@ int bb_decode_int8_timefirst(const void *src, const int64_t *unit_offset,
                              int32_t npol, int32_t item_nbytes,
                              const int64_t *t_begin, const int64_t *t_end,
                              const int64_t *out_t0, float *out, void *stream);
+/* Typed output (BB_F32: out 4-byte aligned; BB_F16 / BB_BF16: 8-byte). */
+int bb_decode_int8_timefirst_typed(const void *src,
+                                   const int64_t *unit_offset, int64_t nunit,
+                                   int64_t nsample, int32_t nchan,
+                                   int32_t npol, int32_t item_nbytes,
+                                   const int64_t *t_begin,
+                                   const int64_t *t_end,
+                                   const int64_t *out_t0, int32_t out_dtype,
+                                   void *out, void *stream);
 int bb_encode_int8_timefirst(const void *in, int32_t in_dtype, void *dst,
                              const int64_t *unit_offset, int64_t nunit,
                              int64_t nsample, int32_t nchan, int32_t npol,
