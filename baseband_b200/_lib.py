@@ -49,6 +49,9 @@ SIGNATURES = {
     'bb_encode_bitfield': (c_int, [
         _pv, c_int32, _pv, _pi64, c_int64, c_int32, c_int64, c_int32,
         c_int32, c_int32, c_void_p]),
+    'bb_encode_bitfield_typed': (c_int, [
+        _pv, c_int32, _pv, _pi64, c_int64, c_int32, c_int64, c_int32,
+        c_int32, c_int32, c_void_p]),
     'bb_mark4_decode': (c_int, [
         _pv, _pi64, c_int64, c_int32, c_int32, c_int32, _pf, c_float,
         c_int64, c_int64, _pv, c_void_p]),
@@ -56,6 +59,9 @@ SIGNATURES = {
         _pv, _pi64, c_int64, c_int32, c_int32, c_int32, _pf, c_float,
         c_int64, c_int64, c_int32, _pv, c_void_p]),
     'bb_mark4_encode': (c_int, [
+        _pv, c_int32, _pv, _pi64, c_int64, c_int32, c_int32, c_int32,
+        c_void_p]),
+    'bb_mark4_encode_typed': (c_int, [
         _pv, c_int32, _pv, _pi64, c_int64, c_int32, c_int32, c_int32,
         c_void_p]),
     'bb_mark4_decode_words': (c_int, [
@@ -71,6 +77,9 @@ SIGNATURES = {
     'bb_encode_int8_transposed': (c_int, [
         _pv, c_int32, _pv, _pi64, c_int64, c_int64, c_int64, c_int32,
         c_void_p]),
+    'bb_encode_int8_transposed_typed': (c_int, [
+        _pv, c_int32, _pv, _pi64, c_int64, c_int64, c_int64, c_int32,
+        c_void_p]),
     'bb_decode_int8_timefirst': (c_int, [
         _pv, _pi64, c_int64, c_int64, c_int32, c_int32, c_int32, _pi64,
         _pi64, _pi64, _pv, c_void_p]),
@@ -78,6 +87,9 @@ SIGNATURES = {
         _pv, _pi64, c_int64, c_int64, c_int32, c_int32, c_int32, _pi64,
         _pi64, _pi64, c_int32, _pv, c_void_p]),
     'bb_encode_int8_timefirst': (c_int, [
+        _pv, c_int32, _pv, _pi64, c_int64, c_int64, c_int32, c_int32,
+        c_int32, c_void_p]),
+    'bb_encode_int8_timefirst_typed': (c_int, [
         _pv, c_int32, _pv, _pi64, c_int64, c_int64, c_int32, c_int32,
         c_int32, c_void_p]),
     'bb_vdif_scan': (c_int, [
@@ -131,11 +143,14 @@ SIGNATURES = {
 
 # every symbol include/baseband_b200.h declares
 EXPORTS = tuple(SIGNATURES)
-# the reduced-precision decoders: bound when present, asked for by name when
-# a float16 / bfloat16 result is wanted (`kernels._typed`)
+# the reduced-precision decoders and encoders: bound when present, asked for
+# by name when a float16 / bfloat16 result or input is handled
+# (`kernels._typed`, `kernels._typed_encoder`)
 OPTIONAL = ('bb_decode_bitfield_typed', 'bb_mark4_decode_typed',
             'bb_decode_int8_transposed_typed',
-            'bb_decode_int8_timefirst_typed')
+            'bb_decode_int8_timefirst_typed', 'bb_encode_bitfield_typed',
+            'bb_mark4_encode_typed', 'bb_encode_int8_transposed_typed',
+            'bb_encode_int8_timefirst_typed')
 
 
 def bind(cdll, required=EXPORTS):

@@ -18,6 +18,7 @@ CUDA ``torch.Tensor`` as ``out`` keeps the decoded samples on the GPU.
 
 There is no CPU decode path: without the CUDA library every read raises.
 """
+import functools
 import mmap
 import operator
 import os
@@ -1287,6 +1288,16 @@ class StreamWriterBase(StreamBase):
     file (base/base.py:1276-1342 semantics, including the zero-padded,
     invalid last frame emitted by ``close``).
 
+    torch tensors, on the device or on the host, may also hold the
+    half-precision types a ``dtype=`` reader returns: float16 or bfloat16
+    for real streams; complex32, or bfloat16 with a trailing (re, im) axis
+    of 2, for complex streams.  They go to the device at 2 bytes per
+    component and are encoded from there: each value gives exactly the bits
+    its float32 value would.  Writes of mixed types are combined in
+    ``torch.result_type`` of all of them (float16 with float32 or bfloat16
+    gives float32, exactly; anything with float64 gives float64).  numpy
+    float16 arrays are converted to float64, like other numpy types.
+
     Subclasses implement ``_encode_frames``.
     """
 
@@ -1299,19 +1310,35 @@ class StreamWriterBase(StreamBase):
         self._npending = 0
         self._frame_index = 0
 
+    def _pair(self, t):
+        """Whether ``t`` holds complex samples as a trailing (re, im) axis."""
+        return self._complex_data and not t.is_complex()
+
     def _unsqueeze(self, data):
         shape = tuple(self._unsliced_shape)
-        if tuple(data.shape[1:]) != shape:
+        pair = (2,) if self._pair(data) else ()
+        given = tuple(data.shape[1:len(data.shape) - len(pair)])
+        if given != shape:
             try:
-                data = data.reshape((data.shape[0],) + shape)
+                data = data.reshape((data.shape[0],) + shape + pair)
             except (RuntimeError, ValueError):
                 raise ValueError('cannot reshape data with sample shape {} '
-                                 'to {}'.format(tuple(data.shape[1:]), shape))
+                                 'to {}'.format(given, shape))
         return data
 
     def _to_device(self, data):
         dev = self.device
         if isinstance(data, torch.Tensor):
+            # 16-bit complex samples are kept as (re, im) pairs
+            if self._complex_data and data.dtype == torch.complex32:
+                # its float16 view: no other ComplexHalf op is needed
+                return torch.view_as_real(data).to(dev)
+            if self._complex_data and data.dtype == torch.bfloat16:
+                if data.ndim < 2 or data.shape[-1] != 2:
+                    raise ValueError('stream holds complex data: bfloat16 '
+                                     'values need a trailing (re, im) axis '
+                                     'of length 2')
+                return data.to(dev)
             t = data.to(dev)
         else:
             arr = np.asanyarray(data)
@@ -1394,16 +1421,23 @@ class StreamWriterBase(StreamBase):
             pos += n
             if pos >= take:
                 break
-        dtypes = {t.dtype for t, _ in self._pending}
-        dtype = torch.result_type(*[t for t, _ in self._pending][:2]) \
-            if len(dtypes) > 1 else dtypes.pop()
-        data = torch.cat([t.to(dtype) for t, _ in self._pending]) \
-            if len(self._pending) > 1 else self._pending[0][0]
+        pending = [t for t, _ in self._pending]
+        if self._complex_data and any(self._pair(t) for t in pending):
+            # 16-bit complex samples are kept as (re, im) pairs: combine all
+            # in that form, so the types promote as their components do
+            pending = [torch.view_as_real(t) if t.is_complex() else t
+                       for t in pending]
+        dtypes = {t.dtype for t in pending}
+        dtype = functools.reduce(torch.promote_types, dtypes)
+        data = torch.cat([t.to(dtype) for t in pending]) \
+            if len(pending) > 1 else pending[0]
         rest = data[take:]
         rest_valid = self._pending[-1][1]
         data = data[:take].contiguous()
-        if self._complex_data:
+        if data.is_complex():
             data = torch.view_as_real(data)
+        if data.element_size() == 2 and data.data_ptr() % 8:
+            data = data.clone()          # the 16-bit loads need 8 bytes
         frames = self._encode_frames(data.reshape(-1), self._frame_index,
                                      nframe, valid)
         self._write_raw(frames)

@@ -322,9 +322,9 @@ k_decode_tile(const DecGeom p, const LevelTable<BPS> lv) {
 // its own so that it can carry a min-blocks hint of 4 (<= 64 registers): that
 // lets ptxas keep the eight float4 loads of a lane in flight instead of
 // serialising them to stay within 40 registers.
-template <typename T, int BPS, int QUANT, int G>
+template <typename S, int BPS, int QUANT, int G>
 __global__ void __launch_bounds__(kBlock, 4)
-k_encode_rowword(const EncGeom p, const QuantConsts<T> c) {
+k_encode_rowword(const EncGeom p, const QuantConsts<arith_t<S>> c) {
     constexpr int MODE = G == 4 ? MODE_ROWWORD4 : MODE_ROWWORD2;
     constexpr int U = EncUnroll<BPS, MODE>::value;
     constexpr int TPW = (32 / BPS) / (4 / G);
@@ -336,20 +336,22 @@ k_encode_rowword(const EncGeom p, const QuantConsts<T> c) {
     for (int u = 0; u < U; ++u) {
         const uint32_t item = item0 + u * kBlock;
         if (item >= p.nitems) break;
-        rw_stage<T, BPS, QUANT, G>(p, c, item >> 5, lane, cbuf[warp]);
+        rw_stage<S, BPS, QUANT, G>(p, c, item >> 5, lane, cbuf[warp]);
         __syncwarp();
         rw_emit<BPS, G>(p, item >> 5, lane, cbuf[warp]);
         __syncwarp();                             // before the buffer is reused
     }
 }
 
-template <typename T, int BPS, int QUANT, int MODE>
+template <typename S, int BPS, int QUANT, int MODE>
 __global__ void __launch_bounds__(kBlock)
-k_encode_bitfield(const EncGeom p, const QuantConsts<T> c) {
+k_encode_bitfield(const EncGeom p, const QuantConsts<arith_t<S>> c) {
+    using T = arith_t<S>;
     constexpr int U = EncUnroll<BPS, MODE>::value;
     const uint32_t item0 = blockIdx.x * (kBlock * U) + threadIdx.x;
     if (MODE == MODE_RUNQ) {
-        // four words per item: two items' (eight) loads in flight
+        // four words per item: two items' (eight) loads in flight (float
+        // arithmetic; one for float64)
         constexpr int B = sizeof(T) == 4 ? 2 : 1;
 #pragma unroll 1
         for (int u0 = 0; u0 < U; u0 += B) {
@@ -358,7 +360,7 @@ k_encode_bitfield(const EncGeom p, const QuantConsts<T> c) {
             for (int b = 0; b < B; ++b) {
                 const uint32_t item = item0 + (u0 + b) * kBlock;
                 it[b].dst = nullptr;
-                if (item < p.nitems) enc_quad_fetch<T>(p, item, it[b]);
+                if (item < p.nitems) enc_quad_fetch<S>(p, item, it[b]);
             }
 #pragma unroll
             for (int b = 0; b < B; ++b) enc_quad_emit<T, QUANT>(c, it[b]);
@@ -375,7 +377,7 @@ k_encode_bitfield(const EncGeom p, const QuantConsts<T> c) {
             for (int b = 0; b < B; ++b) {
                 const uint32_t item = item0 + (u0 + b) * kBlock;
                 it[b].dst = nullptr;
-                if (item < p.nitems) enc_word_fetch<T, BPS>(p, item, it[b]);
+                if (item < p.nitems) enc_word_fetch<S, BPS>(p, item, it[b]);
             }
 #pragma unroll
             for (int b = 0; b < B; ++b)
@@ -387,10 +389,10 @@ k_encode_bitfield(const EncGeom p, const QuantConsts<T> c) {
     for (int u = 0; u < U; ++u) {
         const uint32_t item = item0 + u * kBlock;
         if (item >= p.nitems) break;
-        if (MODE == MODE_ROWGROUP4) enc_rowgroup<T, BPS, QUANT, 4>(p, c, item);
-        else if (MODE == MODE_ROWGROUP2) enc_rowgroup<T, BPS, QUANT, 2>(p, c, item);
-        else if (MODE == MODE_RUN) enc_word<T, BPS, QUANT, true>(p, c, item);
-        else enc_word<T, BPS, QUANT, false>(p, c, item);
+        if (MODE == MODE_ROWGROUP4) enc_rowgroup<S, BPS, QUANT, 4>(p, c, item);
+        else if (MODE == MODE_ROWGROUP2) enc_rowgroup<S, BPS, QUANT, 2>(p, c, item);
+        else if (MODE == MODE_RUN) enc_word<S, BPS, QUANT, true>(p, c, item);
+        else enc_word<S, BPS, QUANT, false>(p, c, item);
     }
 }
 
@@ -510,44 +512,45 @@ static int launch_decode(const std::vector<DecLaunch> &launches,
     return BB_OK;
 }
 
-template <typename T, int BPS, int QUANT>
+template <typename S, int BPS, int QUANT>
 static int launch_encode(const std::vector<EncLaunch> &launches,
                          cudaStream_t stream) {
+    using T = arith_t<S>;
     static const QuantConsts<T> consts = make_quant_consts<T>();
     for (const EncLaunch &l : launches) {
         const uint32_t n = l.g.nitems;
         switch (l.mode) {
         case MODE_ROWGROUP4:
-            k_encode_bitfield<T, BPS, QUANT, MODE_ROWGROUP4>
+            k_encode_bitfield<S, BPS, QUANT, MODE_ROWGROUP4>
                 <<<tile_grid(n, EncUnroll<BPS, MODE_ROWGROUP4>::value), kBlock,
                    0, stream>>>(l.g, consts);
             break;
         case MODE_ROWGROUP2:
-            k_encode_bitfield<T, BPS, QUANT, MODE_ROWGROUP2>
+            k_encode_bitfield<S, BPS, QUANT, MODE_ROWGROUP2>
                 <<<tile_grid(n, EncUnroll<BPS, MODE_ROWGROUP2>::value), kBlock,
                    0, stream>>>(l.g, consts);
             break;
         case MODE_ROWWORD4:
-            k_encode_rowword<T, BPS, QUANT, 4>
+            k_encode_rowword<S, BPS, QUANT, 4>
                 <<<tile_grid(n, EncUnroll<BPS, MODE_ROWWORD4>::value), kBlock,
                    0, stream>>>(l.g, consts);
             break;
         case MODE_ROWWORD2:
-            k_encode_rowword<T, BPS, QUANT, 2>
+            k_encode_rowword<S, BPS, QUANT, 2>
                 <<<tile_grid(n, EncUnroll<BPS, MODE_ROWWORD2>::value), kBlock,
                    0, stream>>>(l.g, consts);
             break;
         case MODE_RUN:
-            k_encode_bitfield<T, BPS, QUANT, MODE_RUN>
+            k_encode_bitfield<S, BPS, QUANT, MODE_RUN>
                 <<<tile_grid(n, 4), kBlock, 0, stream>>>(l.g, consts);
             break;
         case MODE_RUNQ:
             if constexpr (BPS == 8)
-                k_encode_bitfield<T, 8, QUANT, MODE_RUNQ>
+                k_encode_bitfield<S, 8, QUANT, MODE_RUNQ>
                     <<<tile_grid(n, 4), kBlock, 0, stream>>>(l.g, consts);
             break;
         default:
-            k_encode_bitfield<T, BPS, QUANT, MODE_SCALAR>
+            k_encode_bitfield<S, BPS, QUANT, MODE_SCALAR>
                 <<<tile_grid(n, 4), kBlock, 0, stream>>>(l.g, consts);
         }
         BB_CHECK_LAUNCH("bb_encode_bitfield launch");
@@ -555,25 +558,25 @@ static int launch_encode(const std::vector<EncLaunch> &launches,
     return BB_OK;
 }
 
-template <typename T>
+template <typename S>
 static int dispatch_encode(int bps, int quantiser,
                            const std::vector<EncLaunch> &l, cudaStream_t s) {
     if (quantiser == BB_QUANT_OFFSET_BINARY) {
         switch (bps) {
-        case 1: return launch_encode<T, 1, QUANT_OFFSET>(l, s);
-        case 2: return launch_encode<T, 2, QUANT_OFFSET>(l, s);
-        case 4: return launch_encode<T, 4, QUANT_OFFSET>(l, s);
-        case 8: return launch_encode<T, 8, QUANT_OFFSET>(l, s);
+        case 1: return launch_encode<S, 1, QUANT_OFFSET>(l, s);
+        case 2: return launch_encode<S, 2, QUANT_OFFSET>(l, s);
+        case 4: return launch_encode<S, 4, QUANT_OFFSET>(l, s);
+        case 8: return launch_encode<S, 8, QUANT_OFFSET>(l, s);
         }
     } else if (quantiser == BB_QUANT_MARK5B) {
         switch (bps) {
-        case 1: return launch_encode<T, 1, QUANT_MARK5B>(l, s);
-        case 2: return launch_encode<T, 2, QUANT_MARK5B>(l, s);
+        case 1: return launch_encode<S, 1, QUANT_MARK5B>(l, s);
+        case 2: return launch_encode<S, 2, QUANT_MARK5B>(l, s);
         }
     } else if (quantiser == BB_QUANT_SINT) {
         switch (bps) {
-        case 4: return launch_encode<T, 4, QUANT_SINT>(l, s);
-        case 8: return launch_encode<T, 8, QUANT_SINT>(l, s);
+        case 4: return launch_encode<S, 4, QUANT_SINT>(l, s);
+        case 8: return launch_encode<S, 8, QUANT_SINT>(l, s);
         }
     }
     return set_error(BB_ERR_UNSUPPORTED,
@@ -653,15 +656,20 @@ extern "C" int bb_decode_bitfield(
                                     stream);
 }
 
-extern "C" int bb_encode_bitfield(
+extern "C" int bb_encode_bitfield_typed(
     const void *in, int32_t in_dtype, void *dst, const int64_t *unit_offset,
     int64_t nset, int32_t nthread, int64_t payload_nbytes, int32_t bps,
     int32_t nelem, int32_t quantiser, void *stream) {
     if (!in || !dst || !unit_offset)
         return set_error(BB_ERR_ARGUMENT, "null pointer argument");
-    if (!aligned(in, 16) || !aligned(dst, 4))
+    const int in_align = in_vec_align(in_dtype);
+    if (in_align == 0)
+        return set_error(BB_ERR_ARGUMENT,
+                         "in_dtype must be BB_F32, BB_F64, BB_F16 or BB_BF16");
+    if (!aligned(in, in_align) || !aligned(dst, 4))
         return set_error(BB_ERR_ALIGNMENT,
-                         "in must be 16-byte and dst 4-byte aligned");
+                         "in must be %d-byte and dst 4-byte aligned",
+                         in_align);
     std::vector<EncLaunch> launches;
     std::string err;
     if (!plan_encode(in, dst, unit_offset, nset, nthread, payload_nbytes, bps,
@@ -670,5 +678,17 @@ extern "C" int bb_encode_bitfield(
     cudaStream_t s = as_stream(stream);
     if (in_dtype == BB_F32) return dispatch_encode<float>(bps, quantiser, launches, s);
     if (in_dtype == BB_F64) return dispatch_encode<double>(bps, quantiser, launches, s);
-    return set_error(BB_ERR_ARGUMENT, "in_dtype must be BB_F32 or BB_F64");
+    if (in_dtype == BB_F16) return dispatch_encode<F16>(bps, quantiser, launches, s);
+    return dispatch_encode<BF16>(bps, quantiser, launches, s);
+}
+
+extern "C" int bb_encode_bitfield(
+    const void *in, int32_t in_dtype, void *dst, const int64_t *unit_offset,
+    int64_t nset, int32_t nthread, int64_t payload_nbytes, int32_t bps,
+    int32_t nelem, int32_t quantiser, void *stream) {
+    if (in_dtype != BB_F32 && in_dtype != BB_F64)
+        return set_error(BB_ERR_ARGUMENT, "in_dtype must be BB_F32 or BB_F64");
+    return bb_encode_bitfield_typed(in, in_dtype, dst, unit_offset, nset,
+                                    nthread, payload_nbytes, bps, nelem,
+                                    quantiser, stream);
 }

@@ -755,7 +755,7 @@ BB_HD void dec_scalar(const DecGeom &p, const float *lut, uint32_t item) {
 
 // ------------------------------------------------------------------ encode
 struct EncGeom {
-    const void *in;                 // [nset*spf][nthread][nelem] T (whole call)
+    const void *in;                 // [nset*spf][nthread][nelem] S (whole call)
     unsigned long long in_elem_offset;   // first element of this launch
     uint8_t *dst;
     const long long *unit_offset;
@@ -765,20 +765,14 @@ struct EncGeom {
     FastDiv div_nword, div_ngroup, div_nthread;
 };
 
-template <typename T> struct Vec4;
-template <> struct Vec4<float> {
-    float x, y, z, w;
-    static BB_HD Vec4 load(const float *p) {
-        F4 v = *reinterpret_cast<const F4 *>(p);
-        return {v.x, v.y, v.z, v.w};
-    }
-};
-template <> struct Vec4<double> {
-    double x, y, z, w;
-    static BB_HD Vec4 load(const double *p) {
-        D2 a = *reinterpret_cast<const D2 *>(p);
-        D2 b = *reinterpret_cast<const D2 *>(p + 2);
-        return {a.x, a.y, b.x, b.y};
+template <typename T> struct Vec4 {
+    T x, y, z, w;
+    // four consecutive values of storage type S (arith_t<S> == T)
+    template <typename S>
+    static BB_HD Vec4 load(const S *p) {
+        T v[4];
+        load4(p, v);
+        return {v[0], v[1], v[2], v[3]};
     }
 };
 
@@ -786,9 +780,10 @@ BB_HD void store_u32(uint8_t *p, uint32_t v) {
     *reinterpret_cast<uint32_t *>(p) = v;
 }
 
-template <typename T, int BPS, int QUANT, int G>
-BB_HD void enc_rowgroup(const EncGeom &p, const QuantConsts<T> &c,
+template <typename S, int BPS, int QUANT, int G>
+BB_HD void enc_rowgroup(const EncGeom &p, const QuantConsts<arith_t<S>> &c,
                         uint32_t item) {
+    using T = arith_t<S>;
     constexpr int E = 4 / G;
     constexpr int CPW = 32 / BPS;
     constexpr int TPW = CPW / E;
@@ -797,7 +792,7 @@ BB_HD void enc_rowgroup(const EncGeom &p, const QuantConsts<T> &c,
     uint32_t set, k;
     p.div_nword.divmod(lw, set, k);
     const size_t rowlen = (size_t)p.nthread * E;
-    const T *src = reinterpret_cast<const T *>(p.in) + p.in_elem_offset
+    const S *src = reinterpret_cast<const S *>(p.in) + p.in_elem_offset
         + (size_t)lw * TPW * rowlen + g * 4;
     uint32_t w[G];
 #pragma unroll
@@ -851,14 +846,15 @@ BB_HD uint32_t rw_pack_row(const Vec4<T> &v, const QuantConsts<T> &c) {
     return (q0 | (q1 << BPS)) | ((q2 | (q3 << BPS)) << 16);
 }
 
-template <typename T, int BPS, int QUANT, int G>
-BB_HD void rw_stage(const EncGeom &p, const QuantConsts<T> &c, uint32_t chunk,
-                    uint32_t lane, uint32_t *buf) {
+template <typename S, int BPS, int QUANT, int G>
+BB_HD void rw_stage(const EncGeom &p, const QuantConsts<arith_t<S>> &c,
+                    uint32_t chunk, uint32_t lane, uint32_t *buf) {
+    using T = arith_t<S>;
     constexpr int TPW = (32 / BPS) / (4 / G);
     constexpr int LB = TPW < 8 ? TPW : 8;         // loads in flight per lane
     const size_t nrows = (size_t)p.nwords_total * TPW;
     const size_t row0 = (size_t)chunk * (32 * TPW);
-    const T *in = reinterpret_cast<const T *>(p.in) + p.in_elem_offset;
+    const S *in = reinterpret_cast<const S *>(p.in) + p.in_elem_offset;
 #pragma unroll
     for (int j0 = 0; j0 < TPW; j0 += LB) {
         Vec4<T> v[LB];
@@ -926,9 +922,10 @@ struct EncWordItem {
     uint8_t *dst;                   // null: nothing to do
 };
 
-template <typename T, int BPS>
+template <typename S, int BPS>
 BB_HD void enc_word_fetch(const EncGeom &p, uint32_t item,
-                          EncWordItem<T, BPS> &it) {
+                          EncWordItem<arith_t<S>, BPS> &it) {
+    using T = arith_t<S>;
     constexpr int CPW = 32 / BPS;
     uint32_t rest, k, set, slot;
     p.div_nthread.divmod(item, rest, slot);
@@ -937,7 +934,7 @@ BB_HD void enc_word_fetch(const EncGeom &p, uint32_t item,
     it.dst = nullptr;
     if (off < 0) return;
     it.dst = p.dst + off + 4ull * k;
-    const T *in = reinterpret_cast<const T *>(p.in) + p.in_elem_offset;
+    const S *in = reinterpret_cast<const S *>(p.in) + p.in_elem_offset;
     const size_t rowlen = (size_t)p.nthread * p.nelem;
     const size_t set_base = (size_t)set * p.spf * rowlen;
 #pragma unroll
@@ -979,8 +976,10 @@ struct EncQuadItem {
     uint8_t *dst;                   // null: nothing to do
 };
 
-template <typename T>
-BB_HD void enc_quad_fetch(const EncGeom &p, uint32_t item, EncQuadItem<T> &it) {
+template <typename S>
+BB_HD void enc_quad_fetch(const EncGeom &p, uint32_t item,
+                          EncQuadItem<arith_t<S>> &it) {
+    using T = arith_t<S>;
     uint32_t rest, kq, set, slot;
     p.div_nthread.divmod(item, rest, slot);
     p.div_nword.divmod(rest, set, kq);
@@ -988,7 +987,7 @@ BB_HD void enc_quad_fetch(const EncGeom &p, uint32_t item, EncQuadItem<T> &it) {
     it.dst = nullptr;
     if (off < 0) return;
     it.dst = p.dst + off + 16ull * kq;
-    const T *in = reinterpret_cast<const T *>(p.in) + p.in_elem_offset;
+    const S *in = reinterpret_cast<const S *>(p.in) + p.in_elem_offset;
     const size_t rowlen = (size_t)p.nthread * p.nelem;
     const uint32_t pc = kq * 16u;
     size_t idx = (size_t)set * p.spf * rowlen;
@@ -1021,9 +1020,10 @@ BB_HD void enc_quad_emit(const QuantConsts<T> &c, const EncQuadItem<T> &it) {
 }
 
 // RUN / SCALAR: item = output word index over all units of the launch.
-template <typename T, int BPS, int QUANT, bool VEC>
-BB_HD void enc_word(const EncGeom &p, const QuantConsts<T> &c,
+template <typename S, int BPS, int QUANT, bool VEC>
+BB_HD void enc_word(const EncGeom &p, const QuantConsts<arith_t<S>> &c,
                     uint32_t item) {
+    using T = arith_t<S>;
     constexpr int CPW = 32 / BPS;
     // item = (set, k, slot), slot fastest: neighbouring lanes read the slots
     // of the same rows, i.e. neighbouring bytes of the input.
@@ -1033,13 +1033,13 @@ BB_HD void enc_word(const EncGeom &p, const QuantConsts<T> &c,
     const uint32_t unit = set * p.nthread + slot;
     long long off = p.unit_offset[unit];
     if (off < 0) return;
-    const T *in = reinterpret_cast<const T *>(p.in) + p.in_elem_offset;
+    const S *in = reinterpret_cast<const S *>(p.in) + p.in_elem_offset;
     const size_t rowlen = (size_t)p.nthread * p.nelem;
     const size_t set_base = (size_t)set * p.spf * rowlen;
     uint32_t w = 0u;
     if (VEC) {
         EncWordItem<T, BPS> it;
-        enc_word_fetch<T, BPS>(p, item, it);
+        enc_word_fetch<S, BPS>(p, item, it);
         enc_word_emit<T, BPS, QUANT>(c, it);
         return;
     } else {
@@ -1047,7 +1047,7 @@ BB_HD void enc_word(const EncGeom &p, const QuantConsts<T> &c,
             uint32_t pc = k * CPW + i;
             uint32_t t = pc / p.nelem, e = pc % p.nelem;
             size_t idx = set_base + ((size_t)t * p.nthread + slot) * p.nelem + e;
-            w |= quantise<T, BPS, QUANT>(in[idx], c) << (i * BPS);
+            w |= quantise<T, BPS, QUANT>(widen(in[idx]), c) << (i * BPS);
         }
     }
     store_u32(p.dst + off + 4ull * k, w);

@@ -201,6 +201,82 @@ BB_HD void store1(OT *p, float v) {
 template <typename OT, typename Geom>
 BB_HD OT *out_as(const Geom &p) { return static_cast<OT *>(p.out); }
 
+// -------------------------------------------------- encoder input element types
+// An encoder reads its input as the storage type S (float, double, F16, BF16)
+// and quantises in the arithmetic type arith_t<S>: double for double, float
+// for the rest.  A 16-bit value is widened to float32 once, as it is loaded;
+// widening is exact, so it encodes to the bits its float32 value would.
+template <typename S> struct Arith { using type = S; };
+template <> struct Arith<F16> { using type = float; };
+template <> struct Arith<BF16> { using type = float; };
+template <typename S> using arith_t = typename Arith<S>::type;
+
+// Host widening of a half bit pattern (the CPU emulation): exact for every
+// value, NaN keeps its sign and payload.
+inline uint32_t f16_to_f32_bits(uint32_t h) {
+    const uint32_t sign = (h & 0x8000u) << 16;
+    uint32_t e = (h >> 10) & 0x1fu, m = h & 0x3ffu;
+    if (e == 0x1fu) return sign | 0x7f800000u | (m << 13);  // inf / NaN
+    if (e == 0) {
+        if (m == 0) return sign;                              // +-0
+        e = 1;                                                // subnormal
+        while (!(m & 0x400u)) { m <<= 1; --e; }
+        m &= 0x3ffu;
+    }
+    return sign | ((e + 112u) << 23) | (m << 13);
+}
+
+// The two 16-bit values of S in one word (`lo` from the low half) -> float32.
+// bfloat16 is the high half of a float32: a shift and a mask.  Half takes one
+// cvt.f32.f16 each; a NaN's sign is then put back from the input, since only
+// the sign of a NaN can reach a code (the Mark 5B 1-bit quantiser).
+template <typename S>
+BB_HD void widen_half2(uint32_t u, float &lo, float &hi) {
+    if (S::kBrain) {
+        lo = uint_as_float(u << 16);
+        hi = uint_as_float(u & 0xffff0000u);
+        return;
+    }
+#if defined(__CUDA_ARCH__)
+    asm("{.reg .b16 l, h;\n\tmov.b32 {l, h}, %2;\n\t"
+        "cvt.f32.f16 %0, l;\n\tcvt.f32.f16 %1, h;}"
+        : "=f"(lo), "=f"(hi) : "r"(u));
+    lo = uint_as_float(float_as_uint(lo) | ((u << 16) & 0x80000000u));
+    hi = uint_as_float(float_as_uint(hi) | (u & 0x80000000u));
+#else
+    lo = uint_as_float(f16_to_f32_bits(u & 0xffffu));
+    hi = uint_as_float(f16_to_f32_bits(u >> 16));
+#endif
+}
+
+// One input value in the arithmetic type.
+BB_HD float widen(float x) { return x; }
+BB_HD double widen(double x) { return x; }
+template <typename S>
+BB_HD float widen(S x) {
+    float lo, hi;
+    widen_half2<S>(x.bits, lo, hi);
+    return lo;
+}
+
+// Four consecutive input values from one vector load: 16 bytes for float32,
+// two 16-byte loads for float64, 8 bytes for the 16-bit types.
+BB_HD void load4(const float *p, float v[4]) {
+    const F4 r = *reinterpret_cast<const F4 *>(p);
+    v[0] = r.x; v[1] = r.y; v[2] = r.z; v[3] = r.w;
+}
+BB_HD void load4(const double *p, double v[4]) {
+    const D2 a = reinterpret_cast<const D2 *>(p)[0];
+    const D2 b = reinterpret_cast<const D2 *>(p)[1];
+    v[0] = a.x; v[1] = a.y; v[2] = b.x; v[3] = b.y;
+}
+template <typename S>
+BB_HD void load4(const S *p, float v[4]) {
+    const H4 h = *reinterpret_cast<const H4 *>(p);
+    widen_half2<S>(h.lo, v[0], v[1]);
+    widen_half2<S>(h.hi, v[2], v[3]);
+}
+
 BB_HD double add_rn(double a, double b) {
 #if defined(__CUDA_ARCH__)
     return __dadd_rn(a, b);

@@ -25,18 +25,18 @@ __global__ void __launch_bounds__(kF8Threads) k_int8_decode_t64(const I8Geom p) 
 
 // Min-blocks hint of 4: lets ptxas keep eight float4 loads in flight (64
 // registers) instead of serialising them to stay within 32.
-template <typename T>
+template <typename S>
 __global__ void __launch_bounds__(kF8Threads, 4) k_int8_encode_t64(const I8Geom p) {
     __shared__ __align__(16) uint32_t tile[kF8SmemWords];
-    f8_enc_load<T>(p, tile, blockIdx.x, threadIdx.x);
+    f8_enc_load<S>(p, tile, blockIdx.x, threadIdx.x);
     __syncthreads();
     f8_enc_store(p, tile, blockIdx.x, threadIdx.x);
 }
 
-template <typename T>
+template <typename S>
 __global__ void __launch_bounds__(kI8Threads) k_int8_encode_t(const I8Geom p) {
     __shared__ __align__(16) uint8_t tile[kI8SmemBytes];
-    i8_enc_load<T>(p, tile, blockIdx.x, threadIdx.x);
+    i8_enc_load<S>(p, tile, blockIdx.x, threadIdx.x);
     __syncthreads();
     i8_enc_store(p, tile, blockIdx.x, threadIdx.x);
 }
@@ -52,13 +52,13 @@ __global__ void __launch_bounds__(kTFThreads) k_int8_decode_timefirst(
         tf_decode<OT>(p, blockIdx.y, item0 + u * kTFThreads);
 }
 
-template <typename T>
+template <typename S>
 __global__ void __launch_bounds__(kTFThreads) k_int8_encode_timefirst(
     const TFGeom p) {
     const uint32_t item0 = blockIdx.x * (kTFThreads * kTFUnroll) + threadIdx.x;
 #pragma unroll
     for (int u = 0; u < kTFUnroll; ++u)
-        tf_encode<T>(p, blockIdx.y, item0 + u * kTFThreads);
+        tf_encode<S>(p, blockIdx.y, item0 + u * kTFThreads);
 }
 
 static int fill_geom(I8Geom &g, int64_t nunit, int64_t nrow, int64_t ncol,
@@ -100,6 +100,15 @@ static void launch_int8_decode_t(const I8Geom &g, uint64_t nblocks, bool fast,
 template <typename OT>
 static void launch_int8_decode_tf(const TFGeom &g, dim3 grid, cudaStream_t s) {
     k_int8_decode_timefirst<OT><<<grid, kTFThreads, 0, s>>>(g);
+}
+
+template <typename S>
+static void launch_int8_encode_t(const I8Geom &g, uint64_t nblocks, bool fast,
+                                 cudaStream_t s) {
+    if (fast)
+        k_int8_encode_t64<S><<<(unsigned)nblocks, kF8Threads, 0, s>>>(g);
+    else
+        k_int8_encode_t<S><<<(unsigned)nblocks, kI8Threads, 0, s>>>(g);
 }
 
 // Alignment the int8 decoders require of `out`: float32 keeps its 8 / 4
@@ -161,15 +170,19 @@ extern "C" int bb_decode_int8_transposed(
                                            out_col0, BB_F32, out, stream);
 }
 
-extern "C" int bb_encode_int8_transposed(
+extern "C" int bb_encode_int8_transposed_typed(
     const void *in, int32_t in_dtype, void *dst, const int64_t *unit_offset,
     int64_t nunit, int64_t nrow, int64_t ncol, int32_t item_nbytes,
     void *stream) {
     if (!in || !dst || !unit_offset)
         return set_error(BB_ERR_ARGUMENT, "null pointer argument");
+    const int in_align = in_vec_align(in_dtype);
+    if (in_align == 0)
+        return set_error(BB_ERR_ARGUMENT,
+                         "in_dtype must be BB_F32, BB_F64, BB_F16 or BB_BF16");
     I8Geom g;
     uint64_t nblocks;
-    const bool fast = nrow % 2 == 0 && aligned(in, 16);
+    const bool fast = nrow % 2 == 0 && aligned(in, in_align);
     int rc = fill_geom(g, nunit, nrow, ncol, item_nbytes, nblocks, fast);
     if (rc != BB_OK) return rc;
     if (nblocks == 0) return BB_OK;
@@ -178,19 +191,24 @@ extern "C" int bb_encode_int8_transposed(
     g.col_begin = g.col_end = g.out_col0 = nullptr;
     g.out = nullptr;
     g.in = in;
-    if (in_dtype != BB_F32 && in_dtype != BB_F64)
-        return set_error(BB_ERR_ARGUMENT, "in_dtype must be BB_F32 or BB_F64");
     cudaStream_t s = as_stream(stream);
-    if (fast && in_dtype == BB_F32)
-        k_int8_encode_t64<float><<<(unsigned)nblocks, kF8Threads, 0, s>>>(g);
-    else if (fast)
-        k_int8_encode_t64<double><<<(unsigned)nblocks, kF8Threads, 0, s>>>(g);
-    else if (in_dtype == BB_F32)
-        k_int8_encode_t<float><<<(unsigned)nblocks, kI8Threads, 0, s>>>(g);
-    else
-        k_int8_encode_t<double><<<(unsigned)nblocks, kI8Threads, 0, s>>>(g);
+    if (in_dtype == BB_F32) launch_int8_encode_t<float>(g, nblocks, fast, s);
+    else if (in_dtype == BB_F64) launch_int8_encode_t<double>(g, nblocks, fast, s);
+    else if (in_dtype == BB_F16) launch_int8_encode_t<F16>(g, nblocks, fast, s);
+    else launch_int8_encode_t<BF16>(g, nblocks, fast, s);
     BB_CHECK_LAUNCH("bb_encode_int8_transposed launch");
     return BB_OK;
+}
+
+extern "C" int bb_encode_int8_transposed(
+    const void *in, int32_t in_dtype, void *dst, const int64_t *unit_offset,
+    int64_t nunit, int64_t nrow, int64_t ncol, int32_t item_nbytes,
+    void *stream) {
+    if (in_dtype != BB_F32 && in_dtype != BB_F64)
+        return set_error(BB_ERR_ARGUMENT, "in_dtype must be BB_F32 or BB_F64");
+    return bb_encode_int8_transposed_typed(in, in_dtype, dst, unit_offset,
+                                           nunit, nrow, ncol, item_nbytes,
+                                           stream);
 }
 
 extern "C" int bb_decode_int8_timefirst_typed(
@@ -240,17 +258,19 @@ extern "C" int bb_decode_int8_timefirst(
                                           t_end, out_t0, BB_F32, out, stream);
 }
 
-extern "C" int bb_encode_int8_timefirst(
+extern "C" int bb_encode_int8_timefirst_typed(
     const void *in, int32_t in_dtype, void *dst, const int64_t *unit_offset,
     int64_t nunit, int64_t nsample, int32_t nchan, int32_t npol,
     int32_t item_nbytes, void *stream) {
     if (!in || !dst || !unit_offset)
         return set_error(BB_ERR_ARGUMENT, "null pointer argument");
-    if (in_dtype != BB_F32 && in_dtype != BB_F64)
-        return set_error(BB_ERR_ARGUMENT, "in_dtype must be BB_F32 or BB_F64");
+    const int in_align = in_vec_align(in_dtype);
+    if (in_align == 0)
+        return set_error(BB_ERR_ARGUMENT,
+                         "in_dtype must be BB_F32, BB_F64, BB_F16 or BB_BF16");
     TFGeom g;
     if (const char *msg = tf_fill_geom(g, nunit, nsample, nchan, npol,
-                                       item_nbytes, aligned(in, 16)))
+                                       item_nbytes, aligned(in, in_align)))
         return set_error(BB_ERR_ARGUMENT, "%s", msg);
     if (nunit == 0) return BB_OK;
     g.src = (const uint8_t *)dst;
@@ -263,8 +283,23 @@ extern "C" int bb_encode_int8_timefirst(
     cudaStream_t s = as_stream(stream);
     if (in_dtype == BB_F32)
         k_int8_encode_timefirst<float><<<grid, kTFThreads, 0, s>>>(g);
-    else
+    else if (in_dtype == BB_F64)
         k_int8_encode_timefirst<double><<<grid, kTFThreads, 0, s>>>(g);
+    else if (in_dtype == BB_F16)
+        k_int8_encode_timefirst<F16><<<grid, kTFThreads, 0, s>>>(g);
+    else
+        k_int8_encode_timefirst<BF16><<<grid, kTFThreads, 0, s>>>(g);
     BB_CHECK_LAUNCH("bb_encode_int8_timefirst launch");
     return BB_OK;
+}
+
+extern "C" int bb_encode_int8_timefirst(
+    const void *in, int32_t in_dtype, void *dst, const int64_t *unit_offset,
+    int64_t nunit, int64_t nsample, int32_t nchan, int32_t npol,
+    int32_t item_nbytes, void *stream) {
+    if (in_dtype != BB_F32 && in_dtype != BB_F64)
+        return set_error(BB_ERR_ARGUMENT, "in_dtype must be BB_F32 or BB_F64");
+    return bb_encode_int8_timefirst_typed(in, in_dtype, dst, unit_offset,
+                                          nunit, nsample, nchan, npol,
+                                          item_nbytes, stream);
 }

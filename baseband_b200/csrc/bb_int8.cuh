@@ -30,7 +30,7 @@ struct I8Geom {
     const long long *unit_offset;    // [nunit]
     const long long *col_begin, *col_end, *out_col0;   // decode only
     void *out;                       // float32, F16 or BF16 elements
-    const void *in;                  // encode input (float or double)
+    const void *in;                  // encode input (float, double, F16, BF16)
     uint32_t nunit, nrow, ncol, ib;  // ib = item bytes (1 or 2)
     uint32_t tiles_r, tiles_c;       // tiles per unit
     uint32_t group;                  // fast path: column tiles per group
@@ -104,8 +104,9 @@ BB_HD void i8_dec_store(const I8Geom &p, const uint8_t *smem, uint32_t block,
     }
 }
 
-// Encode phase 1: float input (column-major items) -> int8 in the tile.
-template <typename T>
+// Encode phase 1: float input (column-major items) -> int8 in the tile.  The
+// encoders read storage type S and quantise in arith_t<S> (bb_common.cuh).
+template <typename S>
 BB_HD void i8_enc_load(const I8Geom &p, uint8_t *smem, uint32_t block,
                        uint32_t tid) {
     I8Tile t = i8_tile(p, block);
@@ -113,7 +114,8 @@ BB_HD void i8_enc_load(const I8Geom &p, uint8_t *smem, uint32_t block,
     const uint32_t tc = kI8RowBytes / p.ib;
     const uint32_t tr = p.nrow - t.r0 < (uint32_t)kI8Rows ? p.nrow - t.r0
                                                           : kI8Rows;
-    const T *in = reinterpret_cast<const T *>(p.in);
+    using T = arith_t<S>;
+    const S *in = reinterpret_cast<const S *>(p.in);
     const uint32_t total = tc * tr;
     for (uint32_t idx = tid; idx < total; idx += kI8Threads) {
         uint32_t c = tr == kI8Rows ? idx >> 5 : idx / tr;
@@ -123,7 +125,7 @@ BB_HD void i8_enc_load(const I8Geom &p, uint8_t *smem, uint32_t block,
         size_t o = ((size_t)t.unit * p.ncol + j) * p.nrow + t.r0 + r;
         uint8_t *s = smem + r * kI8Pitch + c * p.ib;
         for (uint32_t k = 0; k < p.ib; ++k)
-            s[k] = (uint8_t)quant_sint<T, 8>(in[o * p.ib + k]);
+            s[k] = (uint8_t)quant_sint<T, 8>(widen(in[o * p.ib + k]));
     }
 }
 
@@ -306,60 +308,49 @@ BB_HD void f8_dec_store(const I8Geom &p, const uint32_t *smem, uint32_t block,
 // rows 2l and 2l+1 of one output column as one float4 (a warp load is 512
 // contiguous bytes), quantises and writes two swizzled words; phase 2: a warp
 // writes 128 contiguous bytes of one packed row.
-template <typename T>
-BB_HD void f8_load4(const T *q, T v[4]) {
-    if (sizeof(T) == 4) {
-        F4 r = *reinterpret_cast<const F4 *>(q);
-        v[0] = (T)r.x; v[1] = (T)r.y; v[2] = (T)r.z; v[3] = (T)r.w;
-    } else {
-        D2 a = reinterpret_cast<const D2 *>(q)[0];
-        D2 b = reinterpret_cast<const D2 *>(q)[1];
-        v[0] = (T)a.x; v[1] = (T)a.y; v[2] = (T)b.x; v[3] = (T)b.y;
-    }
-}
-
-template <typename T>
+template <typename S>
 BB_HD void f8_enc_load(const I8Geom &p, uint32_t *smem, uint32_t block,
                        uint32_t tid) {
+    using T = arith_t<S>;
     const F8Tile t = f8_tile(p, block);
     if (p.unit_offset[t.unit] < 0) return;
     const uint32_t lane = tid & 31u, warp = tid >> 5;
     const uint32_t ra = 2u * lane;
     const bool rows_ok = t.r0 + ra < p.nrow;              // nrow is even
-    const T *in = reinterpret_cast<const T *>(p.in);
+    const S *in = reinterpret_cast<const S *>(p.in);
     const size_t row = (size_t)t.r0 + ra;
     const size_t col0 = (size_t)t.unit * p.ncol;
     constexpr int kIter = kF8Words / (kF8Threads / 32);    // 8
     if (sizeof(T) == 4 && p.ib == 2 && t.r0 + kF8Rows <= p.nrow
         && ((size_t)t.w0 + kF8Words) * 2 <= p.ncol) {
-        // Interior complex float32 tile (CTA-uniform test): the eight float4
-        // loads of four word columns are issued back to back before the
-        // first is quantised (4 KiB per warp in flight), as in the decode.
-        const float *fin = reinterpret_cast<const float *>(p.in);
-        const size_t colstride = 2 * (size_t)p.nrow;       // floats per column
+        // Interior complex tile with float arithmetic (float32 or 16-bit
+        // input; CTA-uniform test): the eight four-value loads of four word
+        // columns are issued back to back before the first is quantised
+        // (4 KiB per warp in flight for float32), as in the decode.
+        const size_t colstride = 2 * (size_t)p.nrow;       // values per column
         constexpr int kBatch = 4;
 #pragma unroll
         for (int i0 = 0; i0 < kIter; i0 += kBatch) {
-            F4 v[kBatch][2];
+            T v[kBatch][2][4];
 #pragma unroll
             for (int i = 0; i < kBatch; ++i) {
                 const uint32_t wc = warp + (i0 + i) * (kF8Threads / 32);
-                const float *q = fin
+                const S *q = in
                     + 2 * ((col0 + ((size_t)t.w0 + wc) * 2) * p.nrow + row);
-                v[i][0] = *reinterpret_cast<const F4 *>(q);
-                v[i][1] = *reinterpret_cast<const F4 *>(q + colstride);
+                load4(q, v[i][0]);
+                load4(q + colstride, v[i][1]);
             }
 #pragma unroll
             for (int i = 0; i < kBatch; ++i) {
                 const uint32_t wc = warp + (i0 + i) * (kF8Threads / 32);
-                const uint32_t a = quant_sint<float, 8>(v[i][0].x)
-                    | (quant_sint<float, 8>(v[i][0].y) << 8)
-                    | (quant_sint<float, 8>(v[i][1].x) << 16)
-                    | (quant_sint<float, 8>(v[i][1].y) << 24);
-                const uint32_t b = quant_sint<float, 8>(v[i][0].z)
-                    | (quant_sint<float, 8>(v[i][0].w) << 8)
-                    | (quant_sint<float, 8>(v[i][1].z) << 16)
-                    | (quant_sint<float, 8>(v[i][1].w) << 24);
+                const uint32_t a = quant_sint<T, 8>(v[i][0][0])
+                    | (quant_sint<T, 8>(v[i][0][1]) << 8)
+                    | (quant_sint<T, 8>(v[i][1][0]) << 16)
+                    | (quant_sint<T, 8>(v[i][1][1]) << 24);
+                const uint32_t b = quant_sint<T, 8>(v[i][0][2])
+                    | (quant_sint<T, 8>(v[i][0][3]) << 8)
+                    | (quant_sint<T, 8>(v[i][1][2]) << 16)
+                    | (quant_sint<T, 8>(v[i][1][3]) << 24);
                 smem[f8_swz(ra, wc)] = a;
                 smem[f8_swz(ra + 1, wc)] = b;
             }
@@ -377,7 +368,7 @@ BB_HD void f8_enc_load(const I8Geom &p, uint32_t *smem, uint32_t block,
                 for (int k = 0; k < 2; ++k) {
                     if (j + k >= p.ncol) continue;
                     T v[4];
-                    f8_load4(in + 2 * ((col0 + j + k) * p.nrow + row), v);
+                    load4(in + 2 * ((col0 + j + k) * p.nrow + row), v);
                     a |= (quant_sint<T, 8>(v[0])
                           | (quant_sint<T, 8>(v[1]) << 8)) << (16 * k);
                     b |= (quant_sint<T, 8>(v[2])
@@ -388,9 +379,9 @@ BB_HD void f8_enc_load(const I8Geom &p, uint32_t *smem, uint32_t block,
 #pragma unroll
                 for (int k = 0; k < 4; ++k) {
                     if (j + k >= p.ncol) continue;
-                    const T *q = in + (col0 + j + k) * p.nrow + row;
-                    a |= quant_sint<T, 8>(q[0]) << (8 * k);
-                    b |= quant_sint<T, 8>(q[1]) << (8 * k);
+                    const S *q = in + (col0 + j + k) * p.nrow + row;
+                    a |= quant_sint<T, 8>(widen(q[0])) << (8 * k);
+                    b |= quant_sint<T, 8>(widen(q[1])) << (8 * k);
                 }
             }
         }
@@ -562,17 +553,18 @@ BB_HD void tf_decode(const TFGeom &p, uint32_t unit, uint32_t item) {
            (float)s[(((size_t)t * p.nchan + chan) * p.npol + pol) * p.ib + k]);
 }
 
-template <typename T, int NPOL>
+template <typename S, int NPOL>
 BB_HD void tf_encode_group(const TFGeom &p, uint32_t unit, uint32_t item,
                            long long off) {
+    using T = arith_t<S>;
     uint32_t t, cg;
     p.div_sample_items.divmod(item, t, cg);
-    const T *q = reinterpret_cast<const T *>(p.in)
+    const S *q = reinterpret_cast<const S *>(p.in)
         + (((size_t)unit * p.nsample + t) * p.sample_floats + 4 * cg);
     T v[NPOL][4];
 #pragma unroll
     for (int pol = 0; pol < NPOL; ++pol)
-        f8_load4(q + (size_t)pol * p.row_floats, v[pol]);
+        load4(q + (size_t)pol * p.row_floats, v[pol]);
     uint32_t w[NPOL];
 #pragma unroll
     for (int i = 0; i < NPOL; ++i) w[i] = 0u;
@@ -593,26 +585,26 @@ BB_HD void tf_encode_group(const TFGeom &p, uint32_t unit, uint32_t item,
                          w);
 }
 
-template <typename T>
+template <typename S>
 BB_HD void tf_encode(const TFGeom &p, uint32_t unit, uint32_t item) {
     if (item >= p.items_per_unit) return;
     const long long off = p.unit_offset[unit];
     if (off < 0) return;
     if (p.vec == 4) {
-        if (p.npol == 2) tf_encode_group<T, 2>(p, unit, item, off);
-        else if (p.npol == 4) tf_encode_group<T, 4>(p, unit, item, off);
-        else tf_encode_group<T, 1>(p, unit, item, off);
+        if (p.npol == 2) tf_encode_group<S, 2>(p, unit, item, off);
+        else if (p.npol == 4) tf_encode_group<S, 4>(p, unit, item, off);
+        else tf_encode_group<S, 1>(p, unit, item, off);
         return;
     }
     uint32_t t, r, pol, f;
     p.div_sample_items.divmod(item, t, r);
     p.div_row_floats.divmod(r, pol, f);
     const uint32_t chan = p.ib == 2 ? f >> 1 : f, k = p.ib == 2 ? (f & 1u) : 0u;
-    const T *q = reinterpret_cast<const T *>(p.in)
+    const S *q = reinterpret_cast<const S *>(p.in)
         + (((size_t)unit * p.nsample + t) * p.sample_floats + r);
     const_cast<uint8_t *>(p.src)[off + (((size_t)t * p.nchan + chan) * p.npol
                                         + pol) * p.ib + k] =
-        (uint8_t)quant_sint<T, 8>(q[0]);
+        (uint8_t)quant_sint<arith_t<S>, 8>(widen(q[0]));
 }
 
 // Host-side validation / geometry shared with the CPU emulation.

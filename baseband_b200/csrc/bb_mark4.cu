@@ -118,25 +118,25 @@ __global__ void __launch_bounds__(kM4Block) k_mark4_decode(const M4Geom p) {
     }
 }
 
-template <typename T, int MODE>
+template <typename S, int MODE>
 __global__ void __launch_bounds__(kM4Block)
-k_mark4_encode(const M4Geom p, const QuantConsts<T> c) {
+k_mark4_encode(const M4Geom p, const QuantConsts<arith_t<S>> c) {
     constexpr int U = kM4UnrollEncFast;
     const uint32_t item0 = blockIdx.x * (kM4Block * U) + threadIdx.x;
 #pragma unroll 1
     for (int u = 0; u < U; ++u) {
         const uint32_t item = item0 + u * kM4Block;
         if (item >= p.nitems) break;
-        if (MODE == M4_FAST) m4_enc_fast<T>(p, c, item);
-        else m4_enc_generic<T>(p, c, item);
+        if (MODE == M4_FAST) m4_enc_fast<S>(p, c, item);
+        else m4_enc_generic<S>(p, c, item);
     }
 }
 
 // HALF encode, one kernel per track-word size: the bit masks of a thread are
 // built once (they only depend on the layout and the parity of the item).
-template <typename T, int W>
+template <typename S, int W>
 __global__ void __launch_bounds__(kM4Block)
-k_mark4_encode_half(const M4Geom p, const QuantConsts<T> c) {
+k_mark4_encode_half(const M4Geom p, const QuantConsts<arith_t<S>> c) {
     constexpr int U = kM4UnrollHalf;
     const uint32_t item0 = blockIdx.x * (kM4Block * U) + threadIdx.x;
     // kM4Block is even: every item of this thread has the parity of item0
@@ -145,7 +145,7 @@ k_mark4_encode_half(const M4Geom p, const QuantConsts<T> c) {
     for (int u = 0; u < U; ++u) {
         const uint32_t item = item0 + u * kM4Block;
         if (item >= p.nitems) break;
-        m4_enc_half_w<T, W>(p, mk, c, item);
+        m4_enc_half_w<S, W>(p, mk, c, item);
     }
 }
 
@@ -170,22 +170,23 @@ static int run_decode(const std::vector<M4Launch> &launches, cudaStream_t s) {
     return BB_OK;
 }
 
-template <typename T>
+template <typename S>
 static int run_encode(const std::vector<M4Launch> &launches, cudaStream_t s) {
+    using T = arith_t<S>;
     static const QuantConsts<T> consts = make_quant_consts<T>();
     for (const M4Launch &l : launches) {
         unsigned grid = m4_grid(l.g.nitems, l.mode == M4_HALF
                                 ? kM4UnrollHalf : kM4UnrollEncFast);
         if (l.mode == M4_FAST)
-            k_mark4_encode<T, M4_FAST><<<grid, kM4Block, 0, s>>>(l.g, consts);
+            k_mark4_encode<S, M4_FAST><<<grid, kM4Block, 0, s>>>(l.g, consts);
         else if (l.mode == M4_HALF && l.g.wordbytes == 8)
-            k_mark4_encode_half<T, 8><<<grid, kM4Block, 0, s>>>(l.g, consts);
+            k_mark4_encode_half<S, 8><<<grid, kM4Block, 0, s>>>(l.g, consts);
         else if (l.mode == M4_HALF && l.g.wordbytes == 4)
-            k_mark4_encode_half<T, 4><<<grid, kM4Block, 0, s>>>(l.g, consts);
+            k_mark4_encode_half<S, 4><<<grid, kM4Block, 0, s>>>(l.g, consts);
         else if (l.mode == M4_HALF)
-            k_mark4_encode_half<T, 2><<<grid, kM4Block, 0, s>>>(l.g, consts);
+            k_mark4_encode_half<S, 2><<<grid, kM4Block, 0, s>>>(l.g, consts);
         else
-            k_mark4_encode<T, M4_GENERIC_SCALAR>
+            k_mark4_encode<S, M4_GENERIC_SCALAR>
                 <<<grid, kM4Block, 0, s>>>(l.g, consts);
         BB_CHECK_LAUNCH("bb_mark4_encode launch");
     }
@@ -234,25 +235,41 @@ extern "C" int bb_mark4_decode(
                                  nsample, BB_F32, out, stream);
 }
 
-extern "C" int bb_mark4_encode(
+extern "C" int bb_mark4_encode_typed(
     const void *in, int32_t in_dtype, void *dst, const int64_t *unit_offset,
     int64_t nframe, int32_t nchan, int32_t fanout, int32_t ft, void *stream) {
     if (!in || !dst || !unit_offset)
         return set_error(BB_ERR_ARGUMENT, "null pointer argument");
-    if (!aligned(in, 16) || !aligned(dst, 8))
+    const int in_align = in_vec_align(in_dtype);
+    if (in_align == 0)
+        return set_error(BB_ERR_ARGUMENT,
+                         "in_dtype must be BB_F32, BB_F64, BB_F16 or BB_BF16");
+    if (!aligned(in, in_align) || !aligned(dst, 8))
         return set_error(BB_ERR_ALIGNMENT,
-                         "in must be 16-byte and dst 8-byte aligned");
+                         "in must be %d-byte and dst 8-byte aligned",
+                         in_align);
     std::vector<M4Launch> launches;
     std::string err;
     if (!plan_m4_frames(true, dst, unit_offset, nframe, nchan, fanout, ft,
                         nullptr, 0.f, 0, nframe * 20000ll * fanout, nullptr, in,
-                        launches, err))
+                        launches, err, in_align))
         return set_error(err.rfind("no Mark 4 codec", 0) == 0
                          ? BB_ERR_UNSUPPORTED : BB_ERR_ARGUMENT, "%s",
                          err.c_str());
-    if (in_dtype == BB_F32) return run_encode<float>(launches, as_stream(stream));
-    if (in_dtype == BB_F64) return run_encode<double>(launches, as_stream(stream));
-    return set_error(BB_ERR_ARGUMENT, "in_dtype must be BB_F32 or BB_F64");
+    cudaStream_t s = as_stream(stream);
+    if (in_dtype == BB_F32) return run_encode<float>(launches, s);
+    if (in_dtype == BB_F64) return run_encode<double>(launches, s);
+    if (in_dtype == BB_F16) return run_encode<F16>(launches, s);
+    return run_encode<BF16>(launches, s);
+}
+
+extern "C" int bb_mark4_encode(
+    const void *in, int32_t in_dtype, void *dst, const int64_t *unit_offset,
+    int64_t nframe, int32_t nchan, int32_t fanout, int32_t ft, void *stream) {
+    if (in_dtype != BB_F32 && in_dtype != BB_F64)
+        return set_error(BB_ERR_ARGUMENT, "in_dtype must be BB_F32 or BB_F64");
+    return bb_mark4_encode_typed(in, in_dtype, dst, unit_offset, nframe, nchan,
+                                 fanout, ft, stream);
 }
 
 extern "C" int bb_mark4_decode_words(

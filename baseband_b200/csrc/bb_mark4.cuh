@@ -296,10 +296,12 @@ BB_HD void m4s_emit_fast(const M4Geom &p, const float *lut, OT *chunk_out,
 }
 
 // ------------------------------------------------------------------ encode
-// FAST encode: item = (frame, step, half); header steps are skipped.
-template <typename T>
-BB_HD void m4_enc_fast(const M4Geom &p, const QuantConsts<T> &c,
+// FAST encode: item = (frame, step, half); header steps are skipped.  The
+// encoders read storage type S and quantise in arith_t<S> (bb_common.cuh).
+template <typename S>
+BB_HD void m4_enc_fast(const M4Geom &p, const QuantConsts<arith_t<S>> &c,
                        uint32_t item) {
+    using T = arith_t<S>;
     const uint32_t nhalf = p.wordbytes >> 2;
     const uint32_t h = item & (nhalf - 1u);
     const uint32_t fs = nhalf == 2 ? item >> 1 : item;
@@ -307,20 +309,13 @@ BB_HD void m4_enc_fast(const M4Geom &p, const QuantConsts<T> &c,
     p.div_steps.divmod(fs, frame, step);
     const long long off = p.unit_offset ? p.unit_offset[frame] : 0;
     if (off < 0 || step < p.header_steps) return;
-    const T *src = reinterpret_cast<const T *>(p.in) + p.in_elem_offset
+    const S *src = reinterpret_cast<const S *>(p.in) + p.in_elem_offset
         + (((size_t)frame * p.steps + step) * 4) * p.nchan + 4 * h;
     uint32_t bytes[4] = {0u, 0u, 0u, 0u};       // per channel j of this half
 #pragma unroll
     for (int f = 0; f < 4; ++f) {
         T v[4];
-        if (sizeof(T) == 4) {
-            F4 r = *reinterpret_cast<const F4 *>(src + (size_t)f * p.nchan);
-            v[0] = (T)r.x; v[1] = (T)r.y; v[2] = (T)r.z; v[3] = (T)r.w;
-        } else {
-            const D2 *q = reinterpret_cast<const D2 *>(src + (size_t)f * p.nchan);
-            D2 a = q[0], b = q[1];
-            v[0] = (T)a.x; v[1] = (T)a.y; v[2] = (T)b.x; v[3] = (T)b.y;
-        }
+        load4(src + (size_t)f * p.nchan, v);
 #pragma unroll
         for (int j = 0; j < 4; ++j)             // raw code = sign | mag << 1
             bytes[j] |= quantise<T, 2, QUANT_MARK5B>(v[j], c) << (2 * f);
@@ -334,19 +329,20 @@ BB_HD void m4_enc_fast(const M4Geom &p, const QuantConsts<T> &c,
 }
 
 // GENERIC encode: item = (frame, step) -> one whole track word.
-template <typename T>
-BB_HD void m4_enc_generic(const M4Geom &p, const QuantConsts<T> &c,
+template <typename S>
+BB_HD void m4_enc_generic(const M4Geom &p, const QuantConsts<arith_t<S>> &c,
                           uint32_t item) {
+    using T = arith_t<S>;
     uint32_t frame, step;
     p.div_steps.divmod(item, frame, step);
     const long long off = p.unit_offset ? p.unit_offset[frame] : 0;
     if (off < 0 || step < p.header_steps) return;
-    const T *src = reinterpret_cast<const T *>(p.in) + p.in_elem_offset
+    const S *src = reinterpret_cast<const S *>(p.in) + p.in_elem_offset
         + (((size_t)frame * p.steps + step) * p.fanout) * p.nchan;
     unsigned long long w = 0ull;
     const uint32_t nval = p.fanout * p.nchan;
     for (uint32_t i = 0; i < nval; ++i) {
-        uint32_t q = quantise<T, 2, QUANT_OFFSET>(src[i], c);   // 2*s + m
+        uint32_t q = quantise<T, 2, QUANT_OFFSET>(widen(src[i]), c);   // 2*s + m
         uint32_t pp = p.pos[i];
         w |= (unsigned long long)(q >> 1) << (pp & 0xffu);
         w |= (unsigned long long)(q & 1u) << (pp >> 8);
@@ -393,9 +389,10 @@ BB_HD M4HalfMasks m4_half_masks(const M4Geom &p, const uint16_t *pos,
     return mk;
 }
 
-template <typename T, int W>
+template <typename S, int W>
 BB_HD void m4_enc_half_w(const M4Geom &p, const M4HalfMasks &mk,
-                         const QuantConsts<T> &c, uint32_t item) {
+                         const QuantConsts<arith_t<S>> &c, uint32_t item) {
+    using T = arith_t<S>;
     if (item >= p.total32) return;
     uint32_t frame, i32;
     p.div_frame32.divmod(item, frame, i32);
@@ -404,23 +401,13 @@ BB_HD void m4_enc_half_w(const M4Geom &p, const M4HalfMasks &mk,
     if (off < 0 || step < p.header_steps) return;
     // first track word of this value, counted over the launch
     const size_t word0 = (size_t)frame * p.steps + step;
-    const T *in = reinterpret_cast<const T *>(p.in) + p.in_elem_offset;
+    const S *in = reinterpret_cast<const S *>(p.in) + p.in_elem_offset;
     T v[4][4];
 #pragma unroll
     for (int m = 0; m < 4; ++m) {
         // m-th float4 of this value: (word, position in word)
         const uint32_t wsel = W == 2 ? (m >> 1) : 0u;
-        const T *q = in + ((word0 + wsel) * W + mk.pps[m]) * 4;
-        if (sizeof(T) == 4) {
-            F4 r = *reinterpret_cast<const F4 *>(q);
-            v[m][0] = (T)r.x; v[m][1] = (T)r.y; v[m][2] = (T)r.z;
-            v[m][3] = (T)r.w;
-        } else {
-            D2 a = reinterpret_cast<const D2 *>(q)[0];
-            D2 b = reinterpret_cast<const D2 *>(q)[1];
-            v[m][0] = (T)a.x; v[m][1] = (T)a.y; v[m][2] = (T)b.x;
-            v[m][3] = (T)b.y;
-        }
+        load4(in + ((word0 + wsel) * W + mk.pps[m]) * 4, v[m]);
     }
     uint32_t out = 0u;
 #pragma unroll
@@ -441,15 +428,15 @@ BB_HD void m4_enc_half_w(const M4Geom &p, const M4HalfMasks &mk,
 }
 
 // Per-item form (masks rebuilt for every value): the CPU emulation.
-template <typename T>
+template <typename S>
 BB_HD void m4_enc_half(const M4Geom &p, const uint16_t *pos,
-                       const QuantConsts<T> &c, uint32_t item) {
+                       const QuantConsts<arith_t<S>> &c, uint32_t item) {
     if (p.wordbytes == 8)
-        m4_enc_half_w<T, 8>(p, m4_half_masks<8>(p, pos, item & 1u), c, item);
+        m4_enc_half_w<S, 8>(p, m4_half_masks<8>(p, pos, item & 1u), c, item);
     else if (p.wordbytes == 4)
-        m4_enc_half_w<T, 4>(p, m4_half_masks<4>(p, pos, 0u), c, item);
+        m4_enc_half_w<S, 4>(p, m4_half_masks<4>(p, pos, 0u), c, item);
     else
-        m4_enc_half_w<T, 2>(p, m4_half_masks<2>(p, pos, 0u), c, item);
+        m4_enc_half_w<S, 2>(p, m4_half_masks<2>(p, pos, 0u), c, item);
 }
 
 }  // namespace bb

@@ -141,13 +141,16 @@ inline void m4_warp_geom(M4Geom &g, uint32_t nframe) {
     }
 }
 
-// Frames API.  steps = 20000, header_steps = 160.
+// Frames API.  steps = 20000, header_steps = 160.  in_align: the bytes of one
+// four-value input load (16 for float32 / float64, 8 for the 16-bit types),
+// so that every input type gets the same decomposition.
 inline bool plan_m4_frames(bool encode, const void *src_or_dst,
                            const int64_t *unit_offset, int64_t nframe,
                            int nchan, int fanout, int ft, const float *levels,
                            float fill, int64_t sample_start, int64_t nsample,
                            void *out, const void *in,
-                           std::vector<M4Launch> &launches, std::string &err) {
+                           std::vector<M4Launch> &launches, std::string &err,
+                           uintptr_t in_align = 16) {
     M4Geom base;
     if (!m4_base_geom(nchan, fanout, ft, levels, base, err)) return false;
     const uint32_t steps = 20000, hsteps = 160;
@@ -166,7 +169,7 @@ inline bool plan_m4_frames(bool encode, const void *src_or_dst,
         per_frame = (uint64_t)steps * (base.wordbytes / 4);
     } else if (encode && m4_warp_ok(base)
                && ((uintptr_t)src_or_dst & 3u) == 0
-               && ((uintptr_t)in & 15u) == 0) {
+               && ((uintptr_t)in & (in_align - 1)) == 0) {
         mode = M4_HALF;                        // one item per 32-bit value
         per_frame = (uint64_t)steps * base.wordbytes / 4;
     } else if (encode) {

@@ -37,6 +37,14 @@ inline int out_elem_nbytes(int32_t out_dtype) {
         : (out_dtype == BB_F16 || out_dtype == BB_BF16) ? 2 : 0;
 }
 
+// Alignment an encoder requires of its input (one vector load of four
+// values: 16 bytes for float32 and float64, 8 for the 16-bit types), 0 if an
+// encoder cannot read the type.
+inline int in_vec_align(int32_t in_dtype) {
+    return (in_dtype == BB_F32 || in_dtype == BB_F64) ? 16
+        : (in_dtype == BB_F16 || in_dtype == BB_BF16) ? 8 : 0;
+}
+
 #define BB_CHECK_LAUNCH(what)                                            \
     do {                                                                 \
         cudaError_t e__ = cudaGetLastError();                            \

@@ -106,6 +106,28 @@ def _typed(lib, name, out):
     return fn, (code,)
 
 
+# Element types the encoders can read (bb_dtype codes).
+IN_DTYPES = {torch.float32: F32, torch.float64: F64, torch.float16: F16,
+             torch.bfloat16: BF16}
+
+
+def _typed_encoder(lib, name, data):
+    """The encode entry point for ``data``'s element type and its bb_dtype
+    code: ``(fn, code)``.  float32 / float64 use the plain function, float16
+    / bfloat16 its ``_typed`` variant, which takes the same arguments."""
+    code = IN_DTYPES.get(data.dtype)
+    if code is None:
+        raise TypeError('data must be float32, float64, float16 or bfloat16, '
+                        'not {}'.format(data.dtype))
+    if code in (F32, F64):
+        return getattr(lib, name), code
+    try:
+        return getattr(lib, name + '_typed'), code
+    except AttributeError:
+        raise ImportError('libbaseband_b200.so has no {}_typed: rebuild it '
+                          'for float16 / bfloat16 input'.format(name))
+
+
 def _levels_arg(levels):
     if levels is None:
         return None, None
@@ -160,16 +182,17 @@ def decode_bitfield(src, unit_offset, nset, nthread, payload_nbytes, bps,
 
 def encode_bitfield(data, dst, unit_offset, nset, nthread, payload_nbytes,
                     bps, nelem, quantiser=QUANT_OFFSET_BINARY):
-    """bb_encode_bitfield: quantise+pack ``data`` (float32/float64, logical
-    shape (nset*spf, nthread, nelem)) into ``dst`` (uint8) at the unit
-    offsets."""
+    """bb_encode_bitfield: quantise+pack ``data`` (float32, float64, float16
+    or bfloat16, logical shape (nset*spf, nthread, nelem)) into ``dst``
+    (uint8) at the unit offsets.  A 16-bit value encodes as its float32
+    value does."""
     lib = _lib.load()
     _require_cuda(data, dst, unit_offset)
-    code = _float_code(data)
+    fn, code = _typed_encoder(lib, 'bb_encode_bitfield', data)
     if data.numel() == 0:
         return dst                      # nothing to encode
     with _on(dst.device):
-        rc = lib.bb_encode_bitfield(
+        rc = fn(
             _dev(data, 'data'), code, _dev(dst, 'dst', torch.uint8),
             _dev(unit_offset, 'unit_offset', torch.int64), nset, nthread,
             payload_nbytes, bps, nelem, quantiser, _stream_ptr(dst.device))
@@ -205,12 +228,14 @@ def mark4_decode(src, unit_offset, nframe, nchan, fanout, ft=False,
 
 
 def mark4_encode(data, dst, unit_offset, nframe, nchan, fanout, ft=False):
+    """bb_mark4_encode of ``data`` (float32, float64, float16 or
+    bfloat16)."""
     lib = _lib.load()
-    code = _float_code(data)
+    fn, code = _typed_encoder(lib, 'bb_mark4_encode', data)
     if data.numel() == 0:
         return dst                      # nothing to encode
     with _on(dst.device):
-        rc = lib.bb_mark4_encode(
+        rc = fn(
             _dev(data, 'data'), code, _dev(dst, 'dst', torch.uint8),
             _dev(unit_offset, 'unit_offset', torch.int64), nframe, nchan,
             fanout, int(bool(ft)), _stream_ptr(dst.device))
@@ -272,12 +297,14 @@ def decode_int8_transposed(src, unit_offset, nunit, nrow, ncol, item_nbytes,
 
 def encode_int8_transposed(data, dst, unit_offset, nunit, nrow, ncol,
                            item_nbytes):
+    """bb_encode_int8_transposed of ``data`` (float32, float64, float16 or
+    bfloat16)."""
     lib = _lib.load()
-    code = _float_code(data)
+    fn, code = _typed_encoder(lib, 'bb_encode_int8_transposed', data)
     if data.numel() == 0:
         return dst                      # nothing to encode
     with _on(dst.device):
-        rc = lib.bb_encode_int8_transposed(
+        rc = fn(
             _dev(data, 'data'), code, _dev(dst, 'dst', torch.uint8),
             _dev(unit_offset, 'unit_offset', torch.int64), nunit, nrow, ncol,
             item_nbytes, _stream_ptr(dst.device))
@@ -309,12 +336,14 @@ def decode_int8_timefirst(src, unit_offset, nunit, nsample, nchan, npol,
 
 def encode_int8_timefirst(data, dst, unit_offset, nunit, nsample, nchan, npol,
                           item_nbytes):
+    """bb_encode_int8_timefirst of ``data`` (float32, float64, float16 or
+    bfloat16)."""
     lib = _lib.load()
-    code = _float_code(data)
+    fn, code = _typed_encoder(lib, 'bb_encode_int8_timefirst', data)
     if data.numel() == 0:
         return dst                      # nothing to encode
     with _on(dst.device):
-        rc = lib.bb_encode_int8_timefirst(
+        rc = fn(
             _dev(data, 'data'), code, _dev(dst, 'dst', torch.uint8),
             _dev(unit_offset, 'unit_offset', torch.int64), nunit, nsample,
             nchan, npol, item_nbytes, _stream_ptr(dst.device))

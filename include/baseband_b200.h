@@ -66,10 +66,13 @@ typedef enum bb_quantiser {
                                    (gsb/payload.py:45-53, guppi/payload.py:17) */
 } bb_quantiser;
 
-/* Element types.  Encoders take BB_F32 / BB_F64 input; decoders write BB_F32
- * or, through the `_typed` entry points, BB_F16 (IEEE half) / BB_BF16
- * (bfloat16).  A 16-bit result is the float32 result rounded elementwise to
- * nearest even (overflow to +-inf), as torch's `.to(dtype)` converts it. */
+/* Element types.  Encoders take BB_F32 / BB_F64 input or, through the
+ * `_typed` entry points, BB_F16 (IEEE half) / BB_BF16 (bfloat16); a 16-bit
+ * input value encodes to exactly the bits of its float32 value (widening is
+ * exact).  Decoders write BB_F32 or, through the `_typed` entry points,
+ * BB_F16 / BB_BF16.  A 16-bit result is the float32 result rounded
+ * elementwise to nearest even (overflow to +-inf), as torch's `.to(dtype)`
+ * converts it. */
 typedef enum bb_dtype {
     BB_F32 = 0, BB_F64 = 1, BB_F16 = 2, BB_BF16 = 3
 } bb_dtype;
@@ -149,6 +152,16 @@ int bb_encode_bitfield(const void *in, int32_t in_dtype, void *dst,
                        const int64_t *unit_offset, int64_t nset,
                        int32_t nthread, int64_t payload_nbytes, int32_t bps,
                        int32_t nelem, int32_t quantiser, void *stream);
+/* The same with 16-bit input as well: `in_dtype` BB_F32 / BB_F64 (in 16-byte
+ * aligned) or BB_F16 / BB_BF16 (in 8-byte aligned).  Each value is widened
+ * to float32 as it is loaded and quantised as float32 input is; the work
+ * decomposition is the same for every input type.  The plain function
+ * refuses BB_F16 / BB_BF16. */
+int bb_encode_bitfield_typed(const void *in, int32_t in_dtype, void *dst,
+                             const int64_t *unit_offset, int64_t nset,
+                             int32_t nthread, int64_t payload_nbytes,
+                             int32_t bps, int32_t nelem, int32_t quantiser,
+                             void *stream);
 
 /* ------------------------------------------------------------------ Mark 4
  * Replaces `reorder32/64/64_Ft` + the five `decode_*`/`encode_*` functions
@@ -178,6 +191,12 @@ int bb_mark4_decode_typed(const void *src, const int64_t *unit_offset,
 int bb_mark4_encode(const void *in, int32_t in_dtype, void *dst,
                     const int64_t *unit_offset, int64_t nframe, int32_t nchan,
                     int32_t fanout, int32_t ft, void *stream);
+/* 16-bit input as bb_encode_bitfield_typed (BB_F16 / BB_BF16: in 8-byte
+ * aligned). */
+int bb_mark4_encode_typed(const void *in, int32_t in_dtype, void *dst,
+                          const int64_t *unit_offset, int64_t nframe,
+                          int32_t nchan, int32_t fanout, int32_t ft,
+                          void *stream);
 /* Payload-only variants (Mark4Payload.data / .fromdata): nword track words,
  * no header region.  words/out are device pointers. */
 int bb_mark4_decode_words(const void *words, int64_t nword, int32_t nchan,
@@ -219,6 +238,13 @@ int bb_encode_int8_transposed(const void *in, int32_t in_dtype, void *dst,
                               const int64_t *unit_offset, int64_t nunit,
                               int64_t nrow, int64_t ncol, int32_t item_nbytes,
                               void *stream);
+/* 16-bit input as bb_encode_bitfield_typed.  Like the plain function it
+ * takes any element-aligned `in`; the fast tile path needs 16-byte (BB_F32,
+ * BB_F64) or 8-byte (BB_F16, BB_BF16) alignment. */
+int bb_encode_int8_transposed_typed(const void *in, int32_t in_dtype,
+                                    void *dst, const int64_t *unit_offset,
+                                    int64_t nunit, int64_t nrow, int64_t ncol,
+                                    int32_t item_nbytes, void *stream);
 
 /* Time-first GUPPI payloads (PKTFMT other than '1SFA';
  * baseband/guppi/payload.py:97-102 decode, :131-134 encode): unit u at
@@ -245,6 +271,13 @@ int bb_encode_int8_timefirst(const void *in, int32_t in_dtype, void *dst,
                              const int64_t *unit_offset, int64_t nunit,
                              int64_t nsample, int32_t nchan, int32_t npol,
                              int32_t item_nbytes, void *stream);
+/* 16-bit input as bb_encode_int8_transposed_typed (vector path: in 16-byte
+ * aligned for BB_F32 / BB_F64, 8-byte for BB_F16 / BB_BF16). */
+int bb_encode_int8_timefirst_typed(const void *in, int32_t in_dtype,
+                                   void *dst, const int64_t *unit_offset,
+                                   int64_t nunit, int64_t nsample,
+                                   int32_t nchan, int32_t npol,
+                                   int32_t item_nbytes, void *stream);
 
 /* ------------------------------------------------------- header batches
  * VDIF: extract the bit-fields of baseband/vdif/header.py:529-542, :557-559
