@@ -134,6 +134,9 @@ SIGNATURES = {
     'bb_int8_moments': (c_int, [
         _pv, _pi64, c_int64, c_int32, c_int64, c_int32, c_int64, c_int64,
         _pv, c_int64, c_void_p]),
+    'bb_byte_counts': (c_int, [
+        _pv, _pi64, c_int64, c_int32, c_int64, c_int32, c_int64, c_int64,
+        _pv, c_int64, c_void_p]),
     'bb_probe_fill': (c_int, [_pv, c_int64, c_int32, c_void_p]),
     'bb_probe_copy': (c_int, [_pv, _pv, c_int64, c_void_p]),
     'bb_probe_expand': (c_int, [_pv, c_int64, _pv, c_int32, c_void_p]),

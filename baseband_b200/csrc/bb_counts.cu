@@ -743,6 +743,198 @@ k_int8_moments(const CountGeom p, int words_per_sample) {
     }
 }
 
+// 8-bit payloads of any encoding: a 256-bin histogram of the stored byte per
+// (bin, thread, element); what a byte means is left to the host's level
+// table.  A CTA counts one window of elements (a `ww`-word stretch of every
+// sample: all of it up to 64 elements, 64 elements beyond) over every
+// split-th segment of its (bin, thread), in shared-memory counters laid out
+// [byte][element in window][replica]: `nrep` copies, lane l writing copy
+// l % nrep, so that nwin_elem * nrep = 64 (32 for one element) and the
+// table is 64 KiB whatever the geometry.  On the 16-byte path every lane of
+// a warp owns a different (element, replica) slot at every step -- a quad's
+// 16 bytes are taken in an order rotated per lane -- and since the slot
+// stride is the whole row of a byte value, the bank is the slot's: no two
+// lanes of a warp hit the same bank, however narrow the data (same-address
+// atomics would otherwise serialise on Gaussian noise that spans a handful
+// of codes).  Units that are not 16-byte aligned take single words, where
+// lanes 16 apart can share a slot (slower, still exact).  A work item is a
+// segment of 128 16-byte quads of one unit, taken by one warp: four loads
+// per lane in flight, the next item's unit offset fetched ahead.  The
+// segments of a bin are dealt out to its CTAs one by one, so a single large
+// unit (a DADA chunk piece) is spread over the GPU too.  Counters are 32
+// bit and read out once, at the end: the launcher gives no CTA more than
+// kByteMaxItems segments (2 GiB), so none can wrap.
+struct ByteGeom {
+    const uint8_t *src;
+    const long long *unit_offset;     // [nset][nthread], < 0: invalid frame
+    unsigned long long *counts;       // [nbin][nthread][nelem][256]
+    long long nset, set_origin, sets_per_bin, bin_first;
+    int nthread, nelem, split;
+    uint32_t nwin;                    // element windows (grid.x = split * nwin)
+    uint32_t lg_p, lg_ww;             // log2 words per sample, per window
+    uint32_t ne;                      // elements per window
+    uint32_t nrep;                    // replicas (lane l -> l % nrep)
+    uint32_t nq;                      // window words per unit
+    uint32_t nseg;                    // work items per unit
+};
+
+constexpr int kByteBlock = 256;
+constexpr int kByteCounters = 256 * 64;
+constexpr uint32_t kByteSegQuads = 128;          // 4 quads per lane
+constexpr int64_t kByteMaxItems = 1ll << 20;     // x 2 KiB = 2 GiB per CTA
+
+// 16 bytes rotated down by `rot` bytes: byte k of the result is byte
+// (k + rot) & 15 of v
+__device__ __forceinline__ void rotate16(const uint4 &v, uint32_t rot,
+                                         uint32_t (&o)[4]) {
+    uint32_t a0 = v.x, a1 = v.y, a2 = v.z, a3 = v.w;
+    if (rot & 4u) { const uint32_t t = a0; a0 = a1; a1 = a2; a2 = a3; a3 = t; }
+    if (rot & 8u) {
+        uint32_t t = a0; a0 = a2; a2 = t;
+        t = a1; a1 = a3; a3 = t;
+    }
+    const uint32_t sh = (rot & 3u) * 8u;
+    o[0] = __funnelshift_r(a0, a1, sh);
+    o[1] = __funnelshift_r(a1, a2, sh);
+    o[2] = __funnelshift_r(a2, a3, sh);
+    o[3] = __funnelshift_r(a3, a0, sh);
+}
+
+__global__ void __launch_bounds__(kByteBlock, 3)
+k_byte_counts(const ByteGeom p) {
+    extern __shared__ uint32_t hist[];          // [256][ne][nrep]
+    const long long bin = p.bin_first + blockIdx.z;
+    long long lo = bin * p.sets_per_bin - p.set_origin;
+    long long hi = lo + p.sets_per_bin;
+    if (lo < 0) lo = 0;
+    if (hi > p.nset) hi = p.nset;
+    if (lo >= hi) return;
+    const int t = blockIdx.y;
+    const uint32_t win = blockIdx.x % p.nwin;
+    const long long sx = blockIdx.x / p.nwin;         // this CTA's share
+    const uint32_t ww = 1u << p.lg_ww, w0 = win * ww;
+    const uint32_t row = p.ne * p.nrep;               // counters per byte value
+    const uint32_t lane = threadIdx.x & 31u, warp = threadIdx.x >> 5;
+    const uint32_t r = lane % p.nrep;
+    for (uint32_t i = threadIdx.x; i < 256u * row; i += kByteBlock) hist[i] = 0u;
+    // slot (element * nrep + replica) of every step: a lane's quads all
+    // start at window word (4 lane) mod ww, i.e. element (16 lane) mod ne,
+    // its single words at window word lane mod ww
+    const uint32_t rot = p.nrep == 1u
+        ? ((lane >> 2) << 1 | (lane >> 1 & 1u)) & 15u : (lane / p.nrep) & 15u;
+    uint32_t colq[16], colw[4];
+#pragma unroll
+    for (int k = 0; k < 16; ++k)
+        colq[k] = ((16u * lane + ((k + rot) & 15u)) % p.ne) * p.nrep + r;
+#pragma unroll
+    for (int b = 0; b < 4; ++b)
+        colw[b] = ((4u * lane + b) % p.ne) * p.nrep + r;
+    __syncthreads();
+
+    auto flush = [&]() {
+        // consecutive threads read consecutive counters (no bank conflict);
+        // the nrep replicas of a slot sit in adjacent lanes
+        unsigned long long *out = p.counts
+            + ((size_t)(bin * p.nthread + t) * p.nelem + (size_t)win * p.ne)
+                * 256u;
+        for (uint32_t i = threadIdx.x; i < 256u * row; i += kByteBlock) {
+            uint32_t n = hist[i];
+            hist[i] = 0u;
+            for (uint32_t o = p.nrep >> 1; o >= 1u; o >>= 1)
+                n += __shfl_xor_sync(0xffffffffu, n, o);
+            if (lane % p.nrep == 0u && n) {
+                const uint32_t v = i / row, e = (i % row) / p.nrep;
+                atomicAdd(out + (size_t)e * 256u + v, (unsigned long long)n);
+            }
+        }
+    };
+
+    // window word q of a unit -> word index in the payload
+    auto word_at = [&](uint32_t q) {
+        return ((q >> p.lg_ww) << p.lg_p) + w0 + (q & (ww - 1u));
+    };
+    auto count_word = [&](uint32_t v) {
+#pragma unroll
+        for (int b = 0; b < 4; ++b)
+            atomicAdd(&hist[((v >> (8 * b)) & 0xffu) * row + colw[b]], 1u);
+    };
+    // segments j = sx + split * item of the bin's (hi - lo) * nseg; the
+    // launcher keeps nitem <= kByteMaxItems
+    const long long jn = (hi - lo) * p.nseg;
+    const uint32_t nitem = sx >= jn ? 0u
+        : (uint32_t)((jn - sx + p.split - 1) / p.split);
+    const long long *uo = p.unit_offset + t;
+    // a warp's items are split * 8 segments apart: (unit k, segment g) of
+    // the next one by an add with carry, no division per item
+    const long long step = (long long)p.split * (kByteBlock / 32);
+    const long long dk = step / p.nseg;
+    const uint32_t dg = (uint32_t)(step - dk * p.nseg);
+    const long long j0 = sx + (long long)p.split * warp;
+    long long k = j0 / p.nseg;
+    uint32_t g = (uint32_t)(j0 - k * p.nseg);
+    uint32_t item = warp;
+    long long off = item < nitem ? uo[(lo + k) * p.nthread] : -1;
+    const uint32_t nquad = p.nq / 4u;
+    while (item < nitem) {
+        const uint32_t next = item + kByteBlock / 32;
+        uint32_t g_next = g + dg;
+        long long k_next = k + dk;
+        if (g_next >= p.nseg) {
+            g_next -= p.nseg;
+            ++k_next;
+        }
+        const long long off_next =
+            next < nitem ? uo[(lo + k_next) * p.nthread] : -1;
+        if (off >= 0) {                              // < 0: invalid frame
+            const uint8_t *base = p.src + off;
+            const uint32_t *w = reinterpret_cast<const uint32_t *>(base);
+            const bool last = g + 1u == p.nseg;
+            const uint32_t q0 = g * kByteSegQuads * 4u;
+            uint32_t q1 = last ? p.nq : q0 + kByteSegQuads * 4u;
+            uint32_t qs = q0;                        // words left to do singly
+            if ((reinterpret_cast<uintptr_t>(base) & 15u) == 0) {
+                // four window words in a row are adjacent in memory: the
+                // window is either a whole sample or a multiple of 4 words
+                const uint4 *q = reinterpret_cast<const uint4 *>(base);
+                const uint32_t i0 = g * kByteSegQuads + lane;
+                uint4 v[kByteSegQuads / 32];
+#pragma unroll
+                for (int u = 0; u < kByteSegQuads / 32; ++u)
+                    if (i0 + 32u * u < nquad)
+                        v[u] = q[word_at(4u * (i0 + 32u * u)) >> 2];
+#pragma unroll
+                for (int u = 0; u < kByteSegQuads / 32; ++u)
+                    if (i0 + 32u * u < nquad) {
+                        uint32_t o[4];
+                        rotate16(v[u], rot, o);
+#pragma unroll
+                        for (int k = 0; k < 16; ++k)
+                            atomicAdd(&hist[((o[k >> 2] >> (8 * (k & 3)))
+                                             & 0xffu) * row + colq[k]], 1u);
+                    }
+                qs = last ? nquad * 4u : q1;         // the 0-3 tail words
+            }
+            // unaligned units (and the tail): single words, 16 per lane in
+            // flight; a lane's words stay at window word lane mod ww
+            for (uint32_t i0 = qs + lane; i0 < q1; i0 += 16u * 32u) {
+                uint32_t v[16];
+#pragma unroll
+                for (int u = 0; u < 16; ++u)
+                    if (i0 + 32u * u < q1) v[u] = w[word_at(i0 + 32u * u)];
+#pragma unroll
+                for (int u = 0; u < 16; ++u)
+                    if (i0 + 32u * u < q1) count_word(v[u]);
+            }
+        }
+        item = next;
+        g = g_next;
+        k = k_next;
+        off = off_next;
+    }
+    __syncthreads();
+    flush();
+}
+
 template <int BPS, int NE>
 static void launch_reg(const CountGeom &g, dim3 grid, cudaStream_t s) {
     k_state_counts_reg<BPS, NE><<<grid, kCountBlock, 0, s>>>(g);
@@ -776,6 +968,30 @@ using namespace bb;
 static int count_depth(bool vert = false, int bps = 2) {
     const char *e = getenv(vert ? "BB_TUNE_VERT_DEPTH" : "BB_TUNE_COUNT_DEPTH");
     return (e && *e && atoi(e) > 0) ? atoi(e) : !vert ? 24 : bps == 4 ? 8 : 16;
+}
+
+// The integration bins a call touches, and how many CTAs each (bin, grid
+// row) gets: enough to fill the GPU `want` CTAs deep, at most `most` (one
+// per set, or per work item, of a bin).
+struct BinPlan {
+    int64_t b0, nb, per_bin;
+
+    int64_t split_for(int64_t want, int64_t rows, int64_t most) const {
+        int64_t split = (want + nb * rows - 1) / (nb * rows);
+        if (split > most) split = most;
+        if (split < 1) split = 1;
+        if (split > 65535) split = 65535;
+        return split;
+    }
+};
+
+static bool plan_bins(int64_t nset, int64_t set_origin, int64_t sets_per_bin,
+                      int64_t nbin, BinPlan &bp) {
+    bp.b0 = set_origin / sets_per_bin;
+    const int64_t b1 = (set_origin + nset - 1) / sets_per_bin;    // inclusive
+    bp.nb = b1 - bp.b0 + 1;
+    bp.per_bin = sets_per_bin < nset ? sets_per_bin : nset;
+    return b1 < nbin;
 }
 
 extern "C" int bb_state_counts(
@@ -925,9 +1141,8 @@ extern "C" int bb_int8_moments(
         return set_error(BB_ERR_UNSUPPORTED,
                          "too many elements per sample for moments");
     if (nset == 0) return BB_OK;
-    const int64_t b0 = set_origin / sets_per_bin;
-    const int64_t b1 = (set_origin + nset - 1) / sets_per_bin;
-    if (b1 >= nbin)
+    BinPlan bp;
+    if (!plan_bins(nset, set_origin, sets_per_bin, nbin, bp))
         return set_error(BB_ERR_ARGUMENT, "sets run past the last bin");
     CountGeom g;
     g.src = (const uint8_t *)src;
@@ -939,17 +1154,12 @@ extern "C" int bb_int8_moments(
     g.nthread = nthread;
     g.nelem = nelem;
     g.nword = (uint32_t)(payload_nbytes / 4);
-    const int64_t nb = b1 - b0 + 1;
-    const int64_t per_bin = sets_per_bin < nset ? sets_per_bin : nset;
-    const int64_t want = (int64_t)count_depth() * sm_count();
-    int64_t split = (want + nb * nthread - 1) / (nb * nthread);
-    if (split > per_bin) split = per_bin;
-    if (split < 1) split = 1;
-    if (split > 65535) split = 65535;
+    const int64_t split = bp.split_for((int64_t)count_depth() * sm_count(),
+                                       nthread, bp.per_bin);
     g.split = (int)split;
-    for (int64_t z0 = 0; z0 < nb; z0 += 65535) {
-        const int64_t nz = nb - z0 < 65535 ? nb - z0 : 65535;
-        g.bin_first = b0 + z0;
+    for (int64_t z0 = 0; z0 < bp.nb; z0 += 65535) {
+        const int64_t nz = bp.nb - z0 < 65535 ? bp.nb - z0 : 65535;
+        g.bin_first = bp.b0 + z0;
         dim3 grid((unsigned)split, (unsigned)nthread, (unsigned)nz);
         const char *e_u = getenv("BB_TUNE_MOM_U");
         const int u = (e_u && *e_u) ? atoi(e_u) : 4;
@@ -960,6 +1170,81 @@ extern "C" int bb_int8_moments(
         else
             k_int8_moments<4><<<grid, kCountBlock, 0, as_stream(stream)>>>(g, P);
         BB_CHECK_LAUNCH("bb_int8_moments");
+    }
+    return BB_OK;
+}
+
+extern "C" int bb_byte_counts(
+    const void *src, const int64_t *unit_offset, int64_t nset, int32_t nthread,
+    int64_t payload_nbytes, int32_t nelem, int64_t set_origin,
+    int64_t sets_per_bin, uint64_t *counts, int64_t nbin, void *stream) {
+    if (!src || !unit_offset || !counts)
+        return set_error(BB_ERR_ARGUMENT, "null pointer");
+    if (nset < 0 || nthread < 1 || nthread > 65535 || nelem < 1
+        || (nelem & (nelem - 1)) || payload_nbytes <= 0 || (payload_nbytes & 3)
+        || payload_nbytes % nelem || set_origin < 0 || sets_per_bin < 1
+        || nbin < 1)
+        return set_error(BB_ERR_ARGUMENT, "bad geometry (nelem must be a "
+                         "power of two, payload whole samples and words)");
+    if (!aligned(src, 4))
+        return set_error(BB_ERR_ALIGNMENT, "src must be 4-byte aligned");
+    if (payload_nbytes / 4 > 0x7fffffff)
+        return set_error(BB_ERR_ARGUMENT, "payload too large");
+    if (nset == 0) return BB_OK;
+    BinPlan bp;
+    if (!plan_bins(nset, set_origin, sets_per_bin, nbin, bp))
+        return set_error(BB_ERR_ARGUMENT, "sets run past the last bin");
+    // the element window and the number of counter replicas follow from
+    // nelem alone: windows of at most 16 words (64 elements) of a sample,
+    // and as many replicas as fit 64 KiB of counters (32 at most: one per
+    // lane)
+    const uint32_t P = nelem >= 4 ? (uint32_t)nelem / 4u : 1u;
+    const uint32_t ww = P < 16u ? P : 16u;
+    ByteGeom g;
+    g.src = (const uint8_t *)src;
+    g.unit_offset = (const long long *)unit_offset;
+    g.counts = (unsigned long long *)counts;
+    g.nset = nset;
+    g.set_origin = set_origin;
+    g.sets_per_bin = sets_per_bin;
+    g.nthread = nthread;
+    g.nelem = nelem;
+    g.lg_p = (uint32_t)__builtin_ctz(P);
+    g.lg_ww = (uint32_t)__builtin_ctz(ww);
+    g.nwin = P / ww;
+    g.ne = nelem >= 4 ? 4u * ww : (uint32_t)nelem;
+    g.nrep = 64u / g.ne < 32u ? 64u / g.ne : 32u;
+    g.nq = (uint32_t)(payload_nbytes / 4) / P * ww;
+    g.nseg = (g.nq + kByteSegQuads * 4u - 1u) / (kByteSegQuads * 4u);
+    // three CTAs fit an SM (64 KiB of counters each): two waves, so that the
+    // zeroing and read-out of the counters stays small against the payload
+    const int64_t items = bp.per_bin * (int64_t)g.nseg;     // per bin
+    int64_t split = bp.split_for(6ll * sm_count(), (int64_t)nthread * g.nwin,
+                                 items);
+    // no CTA reads more than kByteMaxItems segments: its 32-bit counters
+    // cannot wrap
+    const int64_t need = (items + kByteMaxItems - 1) / kByteMaxItems;
+    if (split < need) split = need;
+    if (split * g.nwin > 0x7fffffffll || split > 65535)
+        return set_error(BB_ERR_UNSUPPORTED,
+                         "too many sets or elements for one call");
+    g.split = (int)split;
+    const size_t smem = (size_t)256 * g.ne * g.nrep * sizeof(uint32_t);
+    static bool attr_set = false;
+    if (!attr_set) {
+        const int rc = check_cuda(cudaFuncSetAttribute(
+            k_byte_counts, cudaFuncAttributeMaxDynamicSharedMemorySize,
+            kByteCounters * (int)sizeof(uint32_t)), "bb_byte_counts (smem)");
+        if (rc != BB_OK) return rc;
+        attr_set = true;
+    }
+    cudaStream_t s = as_stream(stream);
+    for (int64_t z0 = 0; z0 < bp.nb; z0 += 65535) {
+        const int64_t nz = bp.nb - z0 < 65535 ? bp.nb - z0 : 65535;
+        g.bin_first = bp.b0 + z0;
+        dim3 grid((unsigned)(split * g.nwin), (unsigned)nthread, (unsigned)nz);
+        k_byte_counts<<<grid, kByteBlock, smem, s>>>(g);
+        BB_CHECK_LAUNCH("bb_byte_counts");
     }
     return BB_OK;
 }

@@ -161,7 +161,7 @@ class DADAStreamReader(_DADAStreamBase, StreamReaderBase):
                       h0.complex_data, self._mkbf, sample_start - s0,
                       nsample, out)
 
-    # -- packed consumers (tasks.moments) -----------------------------------
+    # -- packed consumers (tasks.moments, tasks.state_counts) --------------
     def _for_each_packed_chunk(self, frame0, nframe, fn):
         """The base loop works on whole frames; DADA frames can be far larger
         than a chunk, so the pieces of `_chunks` (never spanning frames) go
@@ -223,11 +223,12 @@ class DADAStreamReader(_DADAStreamBase, StreamReaderBase):
         uo = torch.zeros(1, dtype=torch.int64).to(raw.device)
         return uo, 1, raw.numel(), 8, h0['NPOL'] * h0['NCHAN'] * ib
 
-    def _moments_view(self, m):
-        """(nbin, 1, npol * nchan * parts, 3) -> (nbin, npol, nchan, parts)."""
+    def _unit_table_view(self, m):
+        """(nbin, 1, npol * nchan * parts, k) -> (nbin, npol, nchan, parts,
+        k), for `tasks.moments` and the 8-bit `tasks.state_counts`."""
         h0 = self.header0
         ib = 2 if h0.complex_data else 1
-        m = m.reshape(m.shape[0], h0['NPOL'], h0['NCHAN'], ib, 3)
+        m = m.reshape(m.shape[0], h0['NPOL'], h0['NCHAN'], ib, m.shape[-1])
         return m if ib == 2 else m[..., 0, :]
 
     @property

@@ -194,8 +194,7 @@ class GSBStreamReader(_GSBStreamBase, StreamReaderBase):
     def _packed_units(self, raw, frame0, nframe):
         """Unit table of a chunk (the raw files' pieces sit one after the
         other in ``raw``, `_read_raw`): a frame is ``npart`` sets of ``npol``
-        units (`tasks.state_counts` for the 4-bit modes, `tasks.moments` for
-        8 bit)."""
+        units (`tasks.state_counts`; also `tasks.moments` for 8 bit)."""
         files = self._files()
         npol, npart = len(files), len(files[0])
         pn = self._payload_nbytes
@@ -212,17 +211,19 @@ class GSBStreamReader(_GSBStreamBase, StreamReaderBase):
     @property
     def _levels(self):
         """Value of every 4-bit code (two's complement nibbles,
-        gsb/payload.py:19-42), for `tasks.state_levels`; 8-bit streams are
-        summarised by their moments instead."""
+        gsb/payload.py:19-42), for `tasks.state_levels`; 8-bit streams use
+        the int8 value of every byte."""
         if self._bps != 4:
             return None
         code = np.arange(16)
         return np.where(code < 8, code, code - 16).astype(np.float32)
 
-    def _moments_view(self, m):
-        """(nbin, npol, nchan * parts, 3) -> (nbin,) + sample shape + parts."""
+    def _unit_table_view(self, m):
+        """(nbin, npol, nchan * parts, k) -> (nbin,) + sample shape + parts
+        + (k,), for `tasks.moments` and the 8-bit `tasks.state_counts`."""
         ib = 2 if self._complex_data else 1
-        m = m.reshape((m.shape[0],) + tuple(self._sample_shape) + (ib, 3))
+        m = m.reshape((m.shape[0],) + tuple(self._sample_shape)
+                      + (ib, m.shape[-1]))
         return m if ib == 2 else m[..., 0, :]
 
 

@@ -124,10 +124,10 @@ class GUPPIStreamReader(_GUPPIStreamBase, StreamReaderBase):
 
     def _packed_units(self, raw, frame0, nframe):
         """Units for consumers that work on the packed int8 samples
-        (`tasks.moments`): the non-overlap part of every frame.  Channels
-        first: one unit per channel row (`thread` = channel, elements = pol x
-        (re, im)); time first: one unit per frame (elements = chan x pol x
-        (re, im))."""
+        (`tasks.moments`, `tasks.state_counts`): the non-overlap part of
+        every frame.  Channels first: one unit per channel row (`thread` =
+        channel, elements = pol x (re, im)); time first: one unit per frame
+        (elements = chan x pol x (re, im))."""
         import torch
         h0 = self.header0
         if h0.bps != 8:

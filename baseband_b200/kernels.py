@@ -668,6 +668,30 @@ def state_counts(src, unit_offset, nset, nthread, payload_nbytes, bps, nelem,
     return counts
 
 
+def byte_counts(src, unit_offset, nset, nthread, payload_nbytes, nelem,
+                counts, set_origin=0, sets_per_bin=None):
+    """bb_byte_counts: add the counts of every stored byte value of ``nset``
+    sets of 8-bit units to ``counts`` (int64 CUDA tensor (nbin, nthread,
+    nelem, 256))."""
+    lib = _lib.load()
+    _require_cuda(src, unit_offset, counts)
+    nbin = counts.shape[0]
+    if tuple(counts.shape[1:]) != (nthread, nelem, 256):
+        raise ValueError('counts must have shape (nbin, nthread, nelem, 256)')
+    if sets_per_bin is None:
+        sets_per_bin = max(1, set_origin + nset)
+    with _on(src.device):
+        rc = lib.bb_byte_counts(
+            _dev(src, 'src', torch.uint8),
+            _dev(unit_offset, 'unit_offset', torch.int64), nset, nthread,
+            payload_nbytes, nelem, int(set_origin), int(sets_per_bin),
+            _dev(counts, 'counts', torch.int64), nbin,
+            _stream_ptr(src.device))
+    _lib.check(rc, lib)
+    _count()
+    return counts
+
+
 def mark4_state_counts(src, unit_offset, nframe, nchan, fanout, ft, counts,
                        set_origin=0, sets_per_bin=None):
     """bb_mark4_state_counts: add the (sign, magnitude) state counts of

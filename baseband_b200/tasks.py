@@ -22,8 +22,9 @@ pipeline (file / pinned host -> H2D -> header scan), and return a few numbers.
     count, sum and sum of squares for 8-bit two's-complement streams (GUPPI),
     which `integrated_power` uses for those.
 
-`state_counts` takes any reader with packed bit-field payloads of 1, 2 or 4
-bits (VDIF, Mark 5B).
+`state_counts` takes any reader with packed payloads: bit fields of 1, 2 or
+4 bits (VDIF, Mark 5B, Mark 4, 4-bit GSB) and 8-bit samples (VDIF, GUPPI,
+DADA, GSB phased), whose 256 states are counted by the stored byte.
 """
 import numpy as np
 import torch
@@ -59,8 +60,18 @@ def _units(fh, raw, f0, nf):
     return units if len(units) == 6 else tuple(units) + (1,)
 
 
+def _int8(fh):
+    """Whether ``fh`` holds 8-bit two's-complement samples (GUPPI, DADA,
+    GSB phased): 8 bits and no level table of its own."""
+    return (fh.bps == 8 and getattr(fh, '_codec', None) is None
+            and getattr(fh, '_levels', None) is None)
+
+
 def state_levels(fh):
-    """float32 level of every code of ``fh``'s payloads (the decode table)."""
+    """float32 level of every code of ``fh``'s payloads (the decode table;
+    for 8-bit two's-complement data the int8 value of every byte)."""
+    if _int8(fh):
+        return np.arange(256, dtype=np.uint8).view(np.int8).astype(np.float32)
     codec = getattr(fh, '_codec', None)
     lv = codec[1] if codec is not None else getattr(fh, '_levels', None)
     if lv is None:
@@ -68,21 +79,56 @@ def state_levels(fh):
     return np.asarray(lv, np.float32)
 
 
+def _sample_view(fh, table):
+    """Per-unit table ``(nbin, nthread, nelem, k)`` of an 8-bit
+    two's-complement reader -> ``(nbin,) + sample shape [+ (2,) for complex
+    data] + (k,)`` (numpy array or torch tensor)."""
+    nbin = table.shape[0]
+    view = getattr(fh, '_unit_table_view', None)
+    if view is not None:                           # GSB: (pol, chan, parts)
+        m = view(table)
+        if getattr(fh, 'squeeze', False):
+            keep = tuple(d for d in m.shape[1:1 + len(fh._unsliced_shape)]
+                         if d > 1)
+            m = m.reshape((nbin,) + keep
+                          + tuple(m.shape[1 + len(fh._unsliced_shape):]))
+        return m
+    h0 = fh.header0
+    ib = 2 if fh.complex_data else 1
+    # (thread = channel, elem = (pol, part)) or (elem = (chan, pol, part))
+    m = table.reshape(nbin, h0.nchan, h0.npol, ib, table.shape[-1])
+    m = m.swapaxes(1, 2)                           # -> (nbin, npol, nchan, ..)
+    if ib == 1:
+        m = m[:, :, :, 0]
+    if getattr(fh, 'squeeze', False):
+        m = m.reshape((nbin,) + tuple(d for d in m.shape[1:3] if d > 1)
+                      + tuple(m.shape[3:]))
+    return m
+
+
 def state_counts(fh, samples_per_bin=None, count=None, device_output=False):
     """Occurrences of every code in the next ``count`` samples of ``fh``.
 
     Returns an int64 array ``(nbin,) + sample shape [+ (2,) for complex
-    data] + (2**bps,)``; for VDIF the sample shape is ``(nthread, nchan)``
+    data] + (2**bps,)``; 8-bit data are counted by the stored byte (index =
+    byte value, levels from `state_levels`).  For VDIF the sample shape is
+    ``(nthread, nchan)``
     with the threads the reader decodes (its thread subset; unit dimensions
     dropped if the reader squeezes), for Mark 5B and Mark 4 ``(nchan,)``
     (Mark 4: codes indexed ``2 * sign + magnitude`` like its level table,
     counted from the track words; the header steps that open every frame are
-    not samples and are left out).  Bin ``b`` covers samples ``[b, b + 1) *
+    not samples and are left out); for GUPPI, DADA and GSB phased the
+    sample shape `moments` returns, and by default the whole frames only, as
+    there (GUPPI's overlap samples are left out).  Bin ``b`` covers samples
+    ``[b, b + 1) *
     samples_per_bin`` from the current sample pointer (default: one bin);
     frames marked invalid are skipped.  The sample pointer advances by
     ``count``.  The packed frames go host -> HBM once; nothing else moves but
     the counts (``device_output=True`` leaves even those on the GPU).
     """
+    int8 = _int8(fh)
+    if int8:
+        count = _whole_frames(fh, count)
     frame0, nframe, frames_per_bin = _frame_range(fh, count, samples_per_bin)
     nbin = -(-nframe // frames_per_bin)
     state = {}
@@ -103,10 +149,16 @@ def state_counts(fh, samples_per_bin=None, count=None, device_output=False):
             state['geom'] = (nthread, nelem, bps)
             state['counts'] = kernels.zeros(
                 (nbin, nthread, nelem, 1 << bps), torch.int64, raw.device)
-        kernels.state_counts(raw, uo, nf * per, nthread, payload_nbytes, bps,
-                             nelem, state['counts'],
-                             set_origin=(f0 - frame0) * per,
-                             sets_per_bin=frames_per_bin * per)
+        if bps == 8:
+            kernels.byte_counts(raw, uo, nf * per, nthread, payload_nbytes,
+                                nelem, state['counts'],
+                                set_origin=(f0 - frame0) * per,
+                                sets_per_bin=frames_per_bin * per)
+        else:
+            kernels.state_counts(raw, uo, nf * per, nthread, payload_nbytes,
+                                 bps, nelem, state['counts'],
+                                 set_origin=(f0 - frame0) * per,
+                                 sets_per_bin=frames_per_bin * per)
 
     fh._for_each_packed_chunk(frame0, nframe, consume)
     check = getattr(fh, '_new_inconsistencies', None)
@@ -115,6 +167,10 @@ def state_counts(fh, samples_per_bin=None, count=None, device_output=False):
                       'it once (which indexes it) before counting states.')
     fh.seek(fh.tell() + nframe * fh.samples_per_frame)
     counts = state['counts']
+    if int8:
+        counts = _sample_view(fh, counts if device_output
+                              else counts.cpu().numpy())
+        return counts
     nthread, nelem, bps = state['geom']
     shape = tuple(fh._unsliced_shape)
     if getattr(fh, '_decode_ids', None) is not None and len(shape) == 2:
@@ -157,27 +213,7 @@ def moments(fh, samples_per_bin=None, count=None):
 
     fh._for_each_packed_chunk(frame0, nframe, consume)
     fh.seek(fh.tell() + nframe * fh.samples_per_frame)
-    m = state['m'].cpu().numpy()
-    nthread, nelem = state['geom']
-    view = getattr(fh, '_moments_view', None)
-    if view is not None:                           # GSB: (pol, chan, parts)
-        m = view(m)
-        if getattr(fh, 'squeeze', False):
-            keep = tuple(d for d in m.shape[1:1 + len(fh._unsliced_shape)]
-                         if d > 1)
-            m = m.reshape((nbin,) + keep
-                          + m.shape[1 + len(fh._unsliced_shape):])
-        return m[..., 0], m[..., 1], m[..., 2]
-    h0 = fh.header0
-    ib = 2 if fh.complex_data else 1
-    # (thread = channel, elem = (pol, part)) or (elem = (chan, pol, part))
-    m = m.reshape(nbin, h0.nchan, h0.npol, ib, 3)
-    m = m.transpose(0, 2, 1, 3, 4)                 # -> (nbin, npol, nchan, ..)
-    if ib == 1:
-        m = m[:, :, :, 0]
-    if getattr(fh, 'squeeze', False):
-        m = m.reshape((nbin,) + tuple(d for d in m.shape[1:3] if d > 1)
-                      + m.shape[3:])
+    m = _sample_view(fh, state['m'].cpu().numpy())
     return m[..., 0], m[..., 1], m[..., 2]
 
 
@@ -197,8 +233,7 @@ def integrated_power(fh, samples_per_bin=None, count=None, average=True):
     ``sum_c counts[c] * level[c]**2``; for complex data re**2 + im**2).
     With ``average`` the mean over the valid samples of the bin (NaN for a
     bin without valid samples), else the sum."""
-    if fh.bps == 8 and getattr(fh, '_codec', None) is None \
-            and getattr(fh, '_levels', None) is None:
+    if _int8(fh):
         # 8-bit two's complement: from the moments
         n, _, sq = moments(fh, samples_per_bin, count)
         total = sq.astype(np.float64)

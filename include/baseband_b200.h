@@ -515,6 +515,23 @@ int bb_int8_moments(const void *src, const int64_t *unit_offset, int64_t nset,
                     int64_t set_origin, int64_t sets_per_bin,
                     int64_t *moments, int64_t nbin, void *stream);
 
+/* bb_byte_counts: the state counts of 8-bit payloads of any encoding,
+ *   counts[bin][thread][elem][byte] += number of samples whose stored byte
+ *   is `byte`
+ * (uint64, nbin x nthread x nelem x 256, caller-zeroed).  The index is the
+ * byte as stored, so the kernel does not know the encoding: offset binary
+ * (VDIF) and two's complement (GUPPI, DADA, GSB) alike; the level of a code
+ * is the host's business.  Bins, invalid units (offset < 0) and
+ * accumulation as in bb_state_counts; elem = byte index within a sample
+ * (nelem a power of two, any size up to the payload).  src 4-byte aligned,
+ * payload_nbytes a multiple of 4 and of nelem (checked); unit offsets
+ * multiples of 4 (not checked: device data).  Exact integers, identical for
+ * any launch shape. */
+int bb_byte_counts(const void *src, const int64_t *unit_offset, int64_t nset,
+                   int32_t nthread, int64_t payload_nbytes, int32_t nelem,
+                   int64_t set_origin, int64_t sets_per_bin,
+                   uint64_t *counts, int64_t nbin, void *stream);
+
 /* bb_mark4_state_counts: the same for Mark 4 track words.  Frames are the
  * units: unit_offset[i] is the offset of frame i's payload (past the 160
  * header steps, as bb_mark4_scan writes it; < 0: invalid frame, left out);
