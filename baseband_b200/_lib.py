@@ -46,6 +46,10 @@ SIGNATURES = {
     'bb_decode_bitfield_typed': (c_int, [
         _pv, _pi64, c_int64, c_int32, c_int64, c_int32, c_int32, c_int32,
         c_int32, _pf, c_float, c_int64, c_int64, c_int32, _pv, c_void_p]),
+    'bb_decode_select_bitfield': (c_int, [
+        _pv, _pi64, c_int64, c_int32, c_int64, c_int32, c_int32, c_int32,
+        c_int32, _pf, c_float, c_int64, c_int64, _pv, c_int32, c_int32, _pv,
+        c_void_p]),
     'bb_encode_bitfield': (c_int, [
         _pv, c_int32, _pv, _pi64, c_int64, c_int32, c_int64, c_int32,
         c_int32, c_int32, c_void_p]),
@@ -92,6 +96,9 @@ SIGNATURES = {
     'bb_encode_int8_timefirst_typed': (c_int, [
         _pv, c_int32, _pv, _pi64, c_int64, c_int64, c_int32, c_int32,
         c_int32, c_void_p]),
+    'bb_decode_select_int8': (c_int, [
+        _pv, _pi64, c_int64, c_int64, c_int64, c_int64, c_int64, _pv,
+        c_int32, _pi64, _pi64, _pi64, c_int32, _pv, c_void_p]),
     'bb_vdif_scan': (c_int, [
         _pv, _pi64, c_int64, c_int64, c_int32, c_int32, c_int32, _pv, _pv,
         _pi64, _pv, c_int64, c_int32, c_int32, c_int32, c_void_p]),
@@ -153,7 +160,9 @@ OPTIONAL = ('bb_decode_bitfield_typed', 'bb_mark4_decode_typed',
             'bb_decode_int8_transposed_typed',
             'bb_decode_int8_timefirst_typed', 'bb_encode_bitfield_typed',
             'bb_mark4_encode_typed', 'bb_encode_int8_transposed_typed',
-            'bb_encode_int8_timefirst_typed')
+            'bb_encode_int8_timefirst_typed',
+            # the selective decoders of subset reads (`kernels.decode_select_*`)
+            'bb_decode_select_bitfield', 'bb_decode_select_int8')
 
 
 def bind(cdll, required=EXPORTS):

@@ -376,6 +376,7 @@ class _Stage:
         self.free = None          # event: kernels no longer read ``raw``
         self.host = None          # pinned staging of the decoded output
         self.pending = None       # (host view, destination) still to copy
+        self.full = None          # whole decoded rows of a gathered subset
 
     def host_out(self, like):
         """Pinned staging tensor shaped and typed like the device tensor
@@ -395,6 +396,14 @@ class _Stage:
         self.done.synchronize()
         _device._threaded_copy(dst.reshape(-1).view(np.uint8),
                                src.numpy().reshape(-1).view(np.uint8))
+
+    def scratch(self, nfloat, dev, dtype):
+        """Device buffer of ``nfloat`` elements for the whole decoded rows
+        of a chunk that a reader decodes before gathering its subset."""
+        if (self.full is None or self.full.numel() < nfloat
+                or self.full.dtype != dtype or self.full.device != dev):
+            self.full = torch.empty(nfloat, dtype=dtype, device=dev)
+        return self.full[:nfloat]
 
     def buffers(self, nbytes, nfloat, dev, need_dec, dtype=torch.float32):
         if self.pin is None or self.pin.numel() < nbytes:
@@ -913,29 +922,118 @@ class StreamReaderBase(StreamBase):
     def _decode_chunk(self, raw, frame0, nframe, sample_start, nsample, out):
         """Decode ``nsample`` samples starting ``sample_start`` samples into
         the first frame of ``raw`` (device bytes of ``nframe`` frames) into
-        the float32, float16 or bfloat16 device tensor ``out`` (flat,
-        unsliced sample layout)."""
+        the float32, float16 or bfloat16 device tensor ``out`` (flat): rows
+        of the components ``self._sel`` of the decoded row, or of the whole
+        decoded row (`_decoded_shape`) if that is None or the reader does
+        not decode selections (`_decodes_selection`)."""
         raise NotImplementedError
+
+    # -- subsets ---------------------------------------------------------
+    # A subset (with squeeze) is resolved once into ``_sel``: the component
+    # of the decoded row behind each output component, in output order,
+    # found by running `_select` -- the squeeze and subset indexing the
+    # reader applies to decoded samples -- on an array of component indices,
+    # so the indexing semantics are torch's own.  The kernels then decode
+    # exactly those components.  From ``_gather_fraction`` of the row on
+    # (Mark 4: always) a reader decodes whole rows chunk by chunk into a
+    # stage's scratch and gathers each chunk instead.
+    _gather_fraction = None
+
+    @property
+    def _decodes_selection(self):
+        f = self._gather_fraction
+        return f is None or self._sel.size < f * self._row_floats
+
+    @property
+    def _decoded_shape(self):
+        """Sample shape of a decoded row (complex: without the (re, im)
+        axis)."""
+        return tuple(self._unsliced_shape)
+
+    def _select(self, data):
+        """Decoded samples (n,) + `_decoded_shape` -> the reader's samples."""
+        return self._squeeze_and_subset(data)
+
+    @property
+    def _sel(self):
+        """int32 array of decoded-row components per output component, or
+        None where the output row is the decoded row."""
+        if '_sel_cache' not in self.__dict__:
+            shape = self._decoded_shape
+            n = int(np.prod(shape, dtype=np.int64))
+            picked = self._select(torch.arange(n).view((1,) + shape))
+            sel = picked.reshape(-1).numpy()
+            if self._complex_data:
+                sel = np.stack([2 * sel, 2 * sel + 1], -1).reshape(-1)
+            if sel.size == self._row_floats and np.array_equal(
+                    sel, np.arange(sel.size)):
+                self._sel_cache = None
+            else:
+                self._sel_cache = sel.astype(np.int32)
+                self._sel_shape = tuple(picked.shape[1:])
+        return self._sel_cache
+
+    def _table_on(self, name, dev, make):
+        """The array ``make()`` as a tensor on ``dev``, made once per reader
+        (tables derived from `_sel`)."""
+        cache = self.__dict__.setdefault('_sel_dev', {})
+        key = (name, str(dev))
+        if key not in cache:
+            cache[key] = torch.from_numpy(make()).to(dev)
+        return cache[key]
+
+    def _sel_on(self, dev, dtype=torch.int32):
+        """`_sel` as a tensor on ``dev``."""
+        return self._table_on(str(dtype), dev, lambda: self._sel.astype(
+            np.int64 if dtype == torch.int64 else np.int32))
+
+    def _decode_bitfield(self, *args, out):
+        """`kernels.decode_bitfield` (src, unit_offset, ..., nsample) into
+        ``out``, or its selective form when the reader has a subset."""
+        from .. import kernels
+        if self._sel is None:
+            return kernels.decode_bitfield(*args, out=out)
+        return kernels.decode_select_bitfield(
+            *args, self._sel_on(out.device), out)
+
+    def _decode_rows(self, st, raw, f0, nf, s0, ns, out):
+        """`_decode_chunk` into ``out``, ``ns`` rows of `_floats_per_sample`;
+        a reader that cannot select decodes whole rows into the stage's
+        scratch and gathers the subset from there."""
+        if self._sel is None or self._decodes_selection:
+            self._decode_chunk(raw, f0, nf, s0, ns, out)
+            return
+        full = st.scratch(ns * self._row_floats, out.device, out.dtype)
+        self._decode_chunk(raw, f0, nf, s0, ns, full)
+        torch.index_select(full.view(ns, -1), 1,
+                           self._sel_on(out.device, torch.int64),
+                           out=out.view(ns, -1))
 
     # -- helpers ---------------------------------------------------------
     @property
-    def _floats_per_sample(self):
+    def _row_floats(self):
+        """Components of a decoded row."""
         n = 2 if self._complex_data else 1
-        for dim in self._unsliced_shape:
+        for dim in self._decoded_shape:
             n *= dim
         return n
 
+    @property
+    def _floats_per_sample(self):
+        """Components of an output row: the selected ones."""
+        sel = self._sel
+        return self._row_floats if sel is None else sel.size
+
     def _finish(self, flat, nsample):
-        """Decoded device buffer -> (nsample, *sample_shape) tensor."""
-        shape = tuple(self._unsliced_shape)
-        if self._complex_data:
-            data = self._complex_view(
-                flat[:nsample * self._floats_per_sample].view(
-                    (nsample,) + shape + (2,)))
-        else:
-            data = flat[:nsample * self._floats_per_sample].view(
-                (nsample,) + shape)
-        return self._squeeze_and_subset(data)
+        """Output rows on the device -> (nsample, *sample_shape) tensor."""
+        n = nsample * self._floats_per_sample
+        pair = (2,) if self._complex_data else ()
+        if self._sel is not None:
+            return self._complex_view(flat[:n].view(
+                (nsample,) + self._sel_shape + pair)) if pair else \
+                flat[:n].view((nsample,) + self._sel_shape)
+        data = flat[:n].view((nsample,) + self._decoded_shape + pair)
+        return self._select(self._complex_view(data) if pair else data)
 
     def _squeeze_and_subset(self, data):
         if self._squeeze:
@@ -1058,7 +1156,9 @@ class StreamReaderBase(StreamBase):
         dev = out.device if out is not None else self.device
         fps = self._floats_per_sample
         dec = self._read_decode_dtype(out)
-        direct = (out is not None and not self._subset and out.is_contiguous()
+        # the decoders write output rows, subsets included: straight into a
+        # contiguous ``out`` of the type they write
+        direct = (out is not None and out.is_contiguous()
                   and out.dtype == self._result_dtype(dec))
         if direct:
             flat = (torch.view_as_real(out) if out.is_complex()
@@ -1095,11 +1195,13 @@ class StreamReaderBase(StreamBase):
                     ahead.wait()
                 raise
         ss.caller_after(1)
+        if direct:
+            return out
         result = self._finish(flat, count)
-        if out is not None and not direct:
+        if out is not None:
             out.copy_(result)
             return out
-        return out if direct else result
+        return result
 
     def _queue_chunk(self, ss, st, raw, pin, flat, fps, dev, f0, nf, s0, ns,
                      row):
@@ -1113,13 +1215,16 @@ class StreamReaderBase(StreamBase):
         with ss.use(1):
             ss.wait_event(1, st.done)
             piece = flat[row * fps:(row + ns) * fps]
-            # the kernels store 4 elements at a time (16 / 8 bytes)
-            if piece.data_ptr() % (4 * piece.element_size()):
+            # the kernels that decode whole rows store 4 elements at a time
+            # (16 / 8 bytes); the selective ones and the gather take any
+            # element alignment
+            if (self._sel is None
+                    and piece.data_ptr() % (4 * piece.element_size())):
                 tmp = torch.empty(ns * fps, dtype=piece.dtype, device=dev)
                 self._decode_chunk(raw, f0, nf, s0, ns, tmp)
                 piece.copy_(tmp)
             else:
-                self._decode_chunk(raw, f0, nf, s0, ns, piece)
+                self._decode_rows(st, raw, f0, nf, s0, ns, piece)
             if self._on_device is not None:
                 self._on_device(self._finish(piece, ns))
             st.free = ss.event(1)
@@ -1169,7 +1274,8 @@ class StreamReaderBase(StreamBase):
                     self._upload(raw, pin, f0, nf)
                 with ss.use(1):
                     ss.wait(1, 0)
-                    self._decode_chunk(raw, f0, nf, s0, ns, st.dec[:ns * fps])
+                    self._decode_rows(st, raw, f0, nf, s0, ns,
+                                      st.dec[:ns * fps])
                     piece = self._finish(st.dec, ns)
                     if self._on_device is not None:
                         self._on_device(piece)
@@ -1214,6 +1320,7 @@ class StreamReaderBase(StreamBase):
         state['_stages'] = None
         state['_streams'] = None
         state['_small_cache'] = None
+        state.pop('_sel_dev', None)
         state.pop('_slots_dev', None)
         state.pop('_bad_dev', None)
         state.pop('_bad_seen', None)
@@ -1259,6 +1366,14 @@ def _decode_dtype_arg(dtype):
         raise ValueError("dtype must be None, 'float32', 'float16' or "
                          "'bfloat16' (or the torch dtype), not {!r}"
                          .format(dtype)) from None
+
+
+def _int32(offsets):
+    """Byte offsets -> the int32 table of `kernels.decode_select_int8`."""
+    offsets = np.asarray(offsets, np.int64)
+    if offsets.size and offsets.max() > np.iinfo(np.int32).max:
+        raise ValueError('payload too large for a selective decode')
+    return offsets.astype(np.int32)
 
 
 def _torch_index(subset, dev):

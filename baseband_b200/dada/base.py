@@ -8,8 +8,9 @@ one launch of the int8 kernel.
 """
 import numpy as np
 
+from .. import kernels
 from ..base.opener import make_opener
-from ..base.stream import (StreamReaderBase, StreamWriterBase,
+from ..base.stream import (StreamReaderBase, StreamWriterBase, _int32,
                            read_file_into)
 from ..base.utils import lcm
 from ..vdif.base import _FileBase
@@ -157,9 +158,41 @@ class DADAStreamReader(_DADAStreamBase, StreamReaderBase):
         if h0.bps != 8:
             raise KeyError(h0.bps)
         s0, b0, b1 = self._piece(sample_start, nsample)
-        decode_device(raw, 0, raw.numel(), h0['NPOL'], h0['NCHAN'],
-                      h0.complex_data, self._mkbf, sample_start - s0,
-                      nsample, out)
+        start = sample_start - s0
+        if self._sel is None or not self._decodes_selection:
+            decode_device(raw, 0, raw.numel(), h0['NPOL'], h0['NCHAN'],
+                          h0.complex_data, self._mkbf, start, nsample, out)
+        elif not self._mkbf:
+            uo = self._table_on('uo', raw.device,
+                                lambda: np.zeros(1, np.int64))
+            self._decode_bitfield(
+                raw, uo, 1, 1, raw.numel(), 8, self._row_floats,
+                h0.complex_data, kernels.CODEC_SINT, None, 0., start, nsample,
+                out=out)
+        else:
+            # one unit: the piece, heaps of (pol, chan, HEAP, re/im)
+            import torch
+            window = torch.tensor([0, start, start + nsample, 0],
+                                  dtype=torch.int64).to(raw.device)
+            kernels.decode_select_int8(
+                raw, window[0:1], 1, nsample, HEAP,
+                self._row_floats * HEAP, 2 if h0.complex_data else 1,
+                self._table_on('off', raw.device, self._mkbf_off),
+                window[1:2], window[2:3], window[3:4], out)
+
+    @property
+    def _gather_fraction(self):
+        # near-full subsets of MKBF heaps: decoding whole rows with the
+        # transposing decoder and gathering is as fast (as for GUPPI)
+        return 7 / 8 if self._mkbf else None
+
+    def _mkbf_off(self):
+        """Byte offset in a heap of every selected component at its first
+        sample: decoded rows are (pol, chan, re/im), heaps (pol, chan, HEAP,
+        re/im)."""
+        ib = 2 if self.header0.complex_data else 1
+        comp, part = np.divmod(self._sel.astype(np.int64), ib)
+        return _int32(comp * HEAP * ib + part)
 
     # -- packed consumers (tasks.moments, tasks.state_counts) --------------
     def _for_each_packed_chunk(self, frame0, nframe, fn):

@@ -186,10 +186,10 @@ class GSBStreamReader(_GSBStreamBase, StreamReaderBase):
     def _decode_chunk(self, raw, frame0, nframe, sample_start, nsample, out):
         uo, npol, pn, bps, nelem, npart = self._packed_units(raw, frame0,
                                                              nframe)
-        kernels.decode_bitfield(
+        self._decode_bitfield(
             raw, uo, nframe * npart, npol, pn, bps, nelem, self._complex_data,
             kernels.CODEC_SINT, None, self._fill_value, sample_start, nsample,
-            out)
+            out=out)
 
     def _packed_units(self, raw, frame0, nframe):
         """Unit table of a chunk (the raw files' pieces sit one after the

@@ -11,7 +11,7 @@ out_col0`` tables of one ``bb_decode_int8_transposed`` launch per chunk.
 import numpy as np
 
 from ..base.opener import make_opener
-from ..base.stream import StreamReaderBase, StreamWriterBase
+from ..base.stream import StreamReaderBase, StreamWriterBase, _int32
 from ..vdif.base import _FileBase
 from .frame import GUPPIFrame
 from .header import GUPPIHeader
@@ -74,6 +74,9 @@ class _GUPPIStreamBase:
 class GUPPIStreamReader(_GUPPIStreamBase, StreamReaderBase):
     """GUPPI stream reader (GPU decode).  ``samples_per_frame`` excludes the
     overlap."""
+    # Near-full subsets: the transposing decoder of whole rows plus a gather
+    # is as fast as the selective decoder (DESIGN.md section 4).
+    _gather_fraction = 7 / 8
 
     def __init__(self, fh_raw, squeeze=True, subset=(), verify=True,
                  device=None, chunk_nbytes=None, dtype=None):
@@ -158,9 +161,39 @@ class GUPPIStreamReader(_GUPPIStreamBase, StreamReaderBase):
         end[-1] -= (end - begin).sum() - nsample
         if h0.bps != 8:
             raise KeyError(h0.bps)
-        decode_device(raw, offsets, self._full_spf, h0.npol, h0.nchan,
-                      h0.complex_data, h0.channels_first, begin, end,
-                      out=out)
+        if self._sel is None or not self._decodes_selection:
+            decode_device(raw, offsets, self._full_spf, h0.npol, h0.nchan,
+                          h0.complex_data, h0.channels_first, begin, end,
+                          out=out)
+            return
+        import torch
+        from .. import kernels
+        first = np.concatenate([[0], np.cumsum(end - begin)[:-1]])
+        tables = torch.from_numpy(np.stack(
+            [offsets.astype(np.int64), begin, end, first])).to(raw.device)
+        kernels.decode_select_int8(
+            raw, tables[0], nframe, self._full_spf, self._full_spf, 0,
+            self._t_stride, self._table_on('off', raw.device, self._sel_off),
+            tables[1], tables[2], tables[3], out)
+
+    @property
+    def _t_stride(self):
+        """Bytes from one sample of a component to the next in a payload."""
+        h0 = self.header0
+        ib = 2 if h0.complex_data else 1
+        return h0.npol * ib * (1 if h0.channels_first else h0.nchan)
+
+    def _sel_off(self):
+        """Byte offset in a payload of every selected component at time 0:
+        channels first [chan][time][pol][re/im], else [time][chan][pol]
+        [re/im]; decoded rows are (pol, chan, re/im)."""
+        h0 = self.header0
+        ib = 2 if h0.complex_data else 1
+        pol, rest = np.divmod(self._sel.astype(np.int64), h0.nchan * ib)
+        chan, part = np.divmod(rest, ib)
+        chan_stride = (self._full_spf * h0.npol * ib if h0.channels_first
+                       else h0.npol * ib)
+        return _int32(chan * chan_stride + pol * ib + part)
 
     @property
     def stop_time(self):

@@ -180,6 +180,73 @@ def decode_bitfield(src, unit_offset, nset, nthread, payload_nbytes, bps,
     return out
 
 
+def _select_entry(lib, name, out):
+    """A selective decode entry point and the bb_dtype code of ``out``."""
+    code = OUT_DTYPES.get(out.dtype)
+    if code is None:
+        raise TypeError('out must be float32, float16 or bfloat16, not {}'
+                        .format(out.dtype))
+    try:
+        return getattr(lib, name), code
+    except AttributeError:
+        raise ImportError('libbaseband_b200.so has no {}: rebuild it for '
+                          'subset reads'.format(name))
+
+
+def decode_select_bitfield(src, unit_offset, nset, nthread, payload_nbytes,
+                           bps, nelem, complex_data, codec, levels, fill_value,
+                           sample_start, nsample, sel, out):
+    """bb_decode_select_bitfield: only the components ``sel`` (int32 CUDA
+    tensor of indices into the decoded row of `decode_bitfield`) of every
+    row, ``out`` (float32, float16 or bfloat16) = (nsample, len(sel))."""
+    lib = _lib.load()
+    _require_cuda(src, unit_offset, sel, out)
+    nsel = sel.numel()
+    if out.numel() != nsample * nsel:
+        raise ValueError('out has the wrong number of elements')
+    if out.numel() == 0:
+        return out
+    fn, code = _select_entry(lib, 'bb_decode_select_bitfield', out)
+    keep, lv = _levels_arg(levels)
+    with _on(src.device):
+        rc = fn(
+            _dev(src, 'src', torch.uint8),
+            _dev(unit_offset, 'unit_offset', torch.int64), nset, nthread,
+            payload_nbytes, bps, nelem, int(bool(complex_data)), codec, lv,
+            float(fill_value), sample_start, nsample,
+            _dev(sel, 'sel', torch.int32), nsel, code, _dev(out, 'out'),
+            _stream_ptr(src.device))
+    _lib.check(rc, lib)
+    _count()
+    return out
+
+
+def decode_select_int8(src, unit_offset, nunit, nsample, heap, heap_stride,
+                       t_stride, off, t_begin, t_end, out_t0, out):
+    """bb_decode_select_int8: component j of sample t of unit u is the int8
+    at ``unit_offset[u] + (t // heap) * heap_stride + (t % heap) * t_stride
+    + off[j]`` (``off``: int32 CUDA tensor); samples [t_begin[u], t_end[u])
+    go to rows out_t0[u] on of ``out`` (float32, float16 or bfloat16, rows
+    of len(off))."""
+    lib = _lib.load()
+    _require_cuda(src, unit_offset, off, t_begin, t_end, out_t0, out)
+    if out.numel() == 0:
+        return out
+    fn, code = _select_entry(lib, 'bb_decode_select_int8', out)
+    with _on(src.device):
+        rc = fn(
+            _dev(src, 'src', torch.uint8),
+            _dev(unit_offset, 'unit_offset', torch.int64), nunit, nsample,
+            heap, heap_stride, t_stride, _dev(off, 'off', torch.int32),
+            off.numel(), _dev(t_begin, 't_begin', torch.int64),
+            _dev(t_end, 't_end', torch.int64),
+            _dev(out_t0, 'out_t0', torch.int64), code, _dev(out, 'out'),
+            _stream_ptr(src.device))
+    _lib.check(rc, lib)
+    _count()
+    return out
+
+
 def encode_bitfield(data, dst, unit_offset, nset, nthread, payload_nbytes,
                     bps, nelem, quantiser=QUANT_OFFSET_BINARY):
     """bb_encode_bitfield: quantise+pack ``data`` (float32, float64, float16

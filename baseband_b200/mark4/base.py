@@ -128,6 +128,9 @@ class Mark4FileWriter(_FileBase):
 class Mark4StreamReader(StreamReaderBase):
     """Mark 4 stream reader (GPU decode)."""
     _sample_shape_maker = Mark4Payload._sample_shape_maker
+    # the decode is a layout-specific track reorder: a subset is gathered
+    # from whole decoded rows, chunk by chunk
+    _gather_fraction = 0.
 
     def __init__(self, fh_raw, sample_rate=None, ntrack=None, decade=None,
                  ref_time=None, squeeze=True, subset=(), fill_value=0.,

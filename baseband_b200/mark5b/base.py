@@ -167,10 +167,10 @@ class Mark5BStreamReader(_Mark5BStreamBase, StreamReaderBase):
     def _decode_chunk(self, raw, frame0, nframe, sample_start, nsample, out):
         uo, nthread, payload_nbytes, bps, nelem = self._packed_units(
             raw, frame0, nframe)
-        kernels.decode_bitfield(
+        self._decode_bitfield(
             raw, uo, nframe, nthread, payload_nbytes, bps, nelem, False,
             kernels.CODEC_LEVELS, self._levels, self._fill_value,
-            sample_start, nsample, out)
+            sample_start, nsample, out=out)
 
     def _packed_units(self, raw, frame0, nframe):
         if self._index is not None:

@@ -190,7 +190,8 @@ class VDIFStreamReader(_VDIFStreamBase, StreamReaderBase):
             device=device, chunk_nbytes=chunk_nbytes, dtype=dtype)
         # Split the subset into thread selection (done by the scan kernel's
         # slot table, so unwanted threads are never decoded) and the rest,
-        # applied after decoding (vdif/base.py:464-490).
+        # which `_select` applies to the decoded slots (vdif/base.py:464-490)
+        # -- on component indices, to find what the kernels decode.
         if self._subset and (nthread > 1 or not self._squeeze):
             picked = np.array(thread_ids)[self._subset[0]]
             self._thread_ids = np.atleast_1d(picked.squeeze()).tolist()
@@ -205,8 +206,8 @@ class VDIFStreamReader(_VDIFStreamBase, StreamReaderBase):
             self._post_subset = self._subset
             self._thread_ids = list(thread_ids)
         # A selection may name a thread more than once (subset [0, -1] on a
-        # one-thread file): each thread is decoded once and duplicates are
-        # expanded by a gather on the decoded samples.
+        # one-thread file): each thread has one slot and the duplicates are
+        # expanded in `_select`.
         self._decode_ids = list(dict.fromkeys(self._thread_ids))
         self._thread_expand = None
         if len(self._decode_ids) != len(self._thread_ids):
@@ -260,23 +261,15 @@ class VDIFStreamReader(_VDIFStreamBase, StreamReaderBase):
 
     # decoded layout: selected threads only
     @property
-    def _floats_per_sample(self):
-        return (len(self._decode_ids) * self._sample_shape[1]
-                * (2 if self._complex_data else 1))
+    def _decoded_shape(self):
+        return (len(self._decode_ids), self._sample_shape[1])
 
-    def _finish(self, flat, nsample):
-        nthread, nchan = len(self._decode_ids), self._sample_shape[1]
-        n = nsample * self._floats_per_sample
-        if self._complex_data:
-            data = self._complex_view(flat[:n].view(nsample, nthread,
-                                                    nchan, 2))
-        else:
-            data = flat[:n].view(nsample, nthread, nchan)
+    def _select(self, data):
         if self._thread_expand is not None:
             data = data[:, torch.as_tensor(self._thread_expand,
                                            device=data.device)]
         if self._squeeze:
-            data = data.reshape((nsample,) + tuple(
+            data = data.reshape(tuple(data.shape[:1]) + tuple(
                 d for d in data.shape[1:] if d > 1))
         if self._post_subset:
             from ..base.stream import _torch_index
@@ -287,10 +280,10 @@ class VDIFStreamReader(_VDIFStreamBase, StreamReaderBase):
     def _decode_chunk(self, raw, frame0, nframe, sample_start, nsample, out):
         uo, nthread, payload_nbytes, bps, nelem = self._packed_units(
             raw, frame0, nframe)
-        kernels.decode_bitfield(
+        self._decode_bitfield(
             raw, uo, nframe, nthread, payload_nbytes, bps, nelem,
             self._complex_data, self._codec[0], self._codec[1],
-            self._fill_value, sample_start, nsample, out)
+            self._fill_value, sample_start, nsample, out=out)
 
     def _packed_units(self, raw, frame0, nframe):
         h0 = self.header0

@@ -163,6 +163,24 @@ int bb_encode_bitfield_typed(const void *in, int32_t in_dtype, void *dst,
                              int32_t bps, int32_t nelem, int32_t quantiser,
                              void *stream);
 
+/* Selective decode (the `subset` of a stream reader): the arguments of
+ * bb_decode_bitfield_typed plus a device table `sel` of `nsel` component
+ * indices into the decoded row (slot * nelem + e, 0 <= sel[j] <
+ * nthread * nelem; repeats and any order allowed).  Writes only
+ *   out[r * nsel + j] = row r of bb_decode_bitfield's output [sel[j]]
+ * for 0 <= r < nsample, with the same values, fill included.  out needs only
+ * element alignment (4 bytes for BB_F32, 2 for BB_F16 / BB_BF16); an entry
+ * outside the row is written as NaN and reads nothing. */
+int bb_decode_select_bitfield(const void *src, const int64_t *unit_offset,
+                              int64_t nset, int32_t nthread,
+                              int64_t payload_nbytes, int32_t bps,
+                              int32_t nelem, int32_t complex_data,
+                              int32_t codec, const float *levels_host,
+                              float fill_value, int64_t sample_start,
+                              int64_t nsample, const int32_t *sel,
+                              int32_t nsel, int32_t out_dtype, void *out,
+                              void *stream);
+
 /* ------------------------------------------------------------------ Mark 4
  * Replaces `reorder32/64/64_Ft` + the five `decode_*`/`encode_*` functions
  * (baseband/mark4/payload.py:48-69, :122-300), keyed like
@@ -278,6 +296,25 @@ int bb_encode_int8_timefirst_typed(const void *in, int32_t in_dtype,
                                    int64_t nunit, int64_t nsample,
                                    int32_t nchan, int32_t npol,
                                    int32_t item_nbytes, void *stream);
+
+/* Selective int8 decode for layouts with an axis transpose (GUPPI
+ * channels-first and time-first, MKBF heaps): component j of sample t of unit
+ * u is the int8 at
+ *   src + unit_offset[u] + (t / heap) * heap_stride + (t % heap) * t_stride
+ *       + off[j]
+ * (off: device int32[nsel], byte offsets at t = 0); samples
+ * [t_begin[u], t_end[u]) go to output rows from out_t0[u] on (the window
+ * tables above, at most nsample samples per unit), out[row * nsel + j].  GUPPI:
+ * heap = nsample; MKBF: heap = 256 samples of (pol, chan, 256, re/im).
+ * out needs only element alignment; units with a negative offset are
+ * skipped. */
+int bb_decode_select_int8(const void *src, const int64_t *unit_offset,
+                          int64_t nunit, int64_t nsample, int64_t heap,
+                          int64_t heap_stride, int64_t t_stride,
+                          const int32_t *off, int32_t nsel,
+                          const int64_t *t_begin, const int64_t *t_end,
+                          const int64_t *out_t0, int32_t out_dtype, void *out,
+                          void *stream);
 
 /* ------------------------------------------------------- header batches
  * VDIF: extract the bit-fields of baseband/vdif/header.py:529-542, :557-559
